@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the hot path: HCQT feature extraction + patch-wise network inference / training (BASELINE.json).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference|reference-gpu] [--workload ...] [--precision ...]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference|reference-gpu] [--workload ...] [--precision ...] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 Default run (what the driver launches): the HEADLINE workload = BASELINE configs[0] at the north star's target size — HCQT + DRCNN
@@ -39,6 +39,7 @@ HCQT_KW = dict(fs=22050, fs_hcqt_target=50, bins_per_octave=36, num_octaves=6, n
 GFLOP_PREFILT_LAYER = 11.664      # one 40->40 15x15 layer per patch (SURVEY 8a row N3)
 DRAM_BYTES_PER_PATCH_LAYER = (951.8e6 + 938.2e6) / 646     # ncu, fused conv_tc_kernel, 75 rows per patch (profiles/README.md)
 REF_ROOT = '/root/reference'
+DUMP_BYTES = 64 << 20                   # --dump-outputs writes at most this much
 
 DRCNN_KW = dict(n_chan_input=6, n_chan_layers=[40, 40, 30, 10], n_prefilt_layers=5, residual=True, n_bins_in=216, n_bins_out=72)
 CNN_XS_KW = dict(n_chan_input=6, n_chan_layers=[20, 20, 10, 1], n_bins_in=216, n_bins_out=72)
@@ -377,8 +378,30 @@ def gather_outputs(ctx, act, gathered):
     return gathered
 
 
-def run_infer(ctx, name, precision, steps, warmup, preload, detail=False, e2e_first=False):
-    """HCQT + patch-wise inference of one clip per GPU per step.  DRCNN: streaming engine; U-Nets: batches of materialised patches."""
+def host_arrays(outputs):
+    """{name: tensor} -> {name: ndarray}: float64 and integer tensors as float64 (exact), other floating types as float32."""
+    import torch
+    return {k: (t.double() if t.dtype == torch.float64 or not t.is_floating_point() else t.float()).cpu().numpy() for k, t in outputs.items()}
+
+
+def write_outputs(path, arrays):
+    """Each array as path/<name>.npy.  An array larger than its share of DUMP_BYTES is replaced by a fixed, seeded sample of its rows
+    (along the first axis, in order), and the indices of those rows go to path/<name>_rows.npy."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    share = DUMP_BYTES // max(1, len(arrays))
+    for name, a in arrays.items():
+        if a.nbytes > share:
+            row_bytes = a.nbytes // a.shape[0] + 8          # + its float64 index
+            rows = np.sort(np.random.default_rng(0).choice(a.shape[0], max(1, share // row_bytes), replace=False))
+            np.save(os.path.join(path, name + '_rows.npy'), rows.astype(np.float64))
+            a = a[rows]
+        np.save(os.path.join(path, name + '.npy'), a)
+
+
+def run_infer(ctx, name, precision, steps, warmup, preload, detail=False, e2e_first=False, outputs=None):
+    """HCQT + patch-wise inference of one clip per GPU per step.  DRCNN: streaming engine; U-Nets: batches of materialised patches.
+    outputs: a dict that receives, as host arrays, what the last timed device-resident step returned."""
     import torch
     from multipitch_architectures_b200 import _lib
     from multipitch_architectures_b200.engine import CnnStreamEngine, predict_patchwise
@@ -396,18 +419,22 @@ def run_infer(ctx, name, precision, steps, warmup, preload, detail=False, e2e_fi
     gathered = torch.empty(ctx.world * n_frames, 72, dtype=torch.float32, device=dev) if ctx.world > 1 else None
 
     def predict(y):
+        """-> {name: tensor}: what a caller of the path receives for the clip y."""
         with torch.no_grad():
             if cnn:
-                return eng.predict_audio(y, plan)[0]
+                act, tuning = eng.predict_audio(y, plan)
+                return {'activations': act, 'tuning_index': tuning}
             hcqt, _ = plan.run_graph(y)
             out = predict_patchwise(model, hcqt, batch=args.infer_batch)
-            return out[0] if isinstance(out, tuple) else out
+            return dict(zip(('activations', 'polyphony'), out)) if isinstance(out, tuple) else {'activations': out}
+
+    last = [None]
 
     def step_resident(i):
-        return predict(clips_dev[i % 2])
+        last[0] = predict(clips_dev[i % 2])
 
     def step_e2e(i):
-        act = predict(clips_host[i % 2].to(dev, non_blocking=True))
+        act = predict(clips_host[i % 2].to(dev, non_blocking=True))['activations']
         g = gather_outputs(ctx, act, gathered)
         if ctx.rank == 0:
             out_host.view(-1, 72).copy_(g, non_blocking=True)        # rank 0 receives the whole job's activations
@@ -432,6 +459,8 @@ def run_infer(ctx, name, precision, steps, warmup, preload, detail=False, e2e_fi
     n0, g0 = _lib.launch_count(), plan.graph_launches
     ms = ctx.timed(step_resident, steps)
     launches = _lib.launch_count() - n0 + (plan.graph_launches - g0)      # host-side counter + the kernel nodes of the replayed HCQT graphs
+    if outputs is not None:                 # copied before the untimed steps below reuse the engine's buffers
+        outputs.update(host_arrays(last[0]))
     timers, share_timers = [], []
     if eng is not None and detail:
         timers, eng.timers, eng.timer_tags = eng.timers, [], None
@@ -492,8 +521,11 @@ def run_infer(ctx, name, precision, steps, warmup, preload, detail=False, e2e_fi
     return res
 
 
-def run_train(ctx, name, precision, steps, warmup, preload):
-    """One training step per call: forward + loss + backward (+ NCCL gradient all-reduce at N > 1) + fused AdamW."""
+def run_train(ctx, name, precision, steps, warmup, preload, outputs=None):
+    """One training step per call: forward + loss + backward (+ NCCL gradient all-reduce at N > 1) + fused AdamW.
+    outputs: a dict that receives, as host arrays, the loss of the last timed device-resident step and the parameters it left.  The weight
+    gradients are split-K sums finished with fp32 atomicAdd, whose order varies, and AdamW amplifies such last-bit differences, so two runs
+    of the same build agree on these to a tolerance only (the headline DRCNN inference outputs repeat bit for bit)."""
     import torch
     from multipitch_architectures_b200 import _lib
     from multipitch_architectures_b200.io import HostPrefetcher
@@ -510,9 +542,10 @@ def run_train(ctx, name, precision, steps, warmup, preload):
     xh, th = synth_patches(batch, ctx.rank).pin_memory(), synth_targets(batch, ctx.rank).pin_memory()
     xd, td = xh.to(dev), th.to(dev)
     loss_host = torch.empty(1).pin_memory()
+    last = [None]
 
     def resident(i):
-        step(xd, td)
+        last[0] = step(xd, td)
 
     # end to end: every step's batch travels from pinned host memory inside the timed region, double-buffered on a side stream
     # (io.HostPrefetcher: the copy of batch k+1 overlaps the step on batch k), and the loss is read back
@@ -537,6 +570,8 @@ def run_train(ctx, name, precision, steps, warmup, preload):
     ms = ctx.timed(resident, steps)
     # kernels launched inside the timed region: the host-side counter plus the kernel nodes of every CUDA-graph replay
     launches = _lib.launch_count() - n0 + (getattr(step, 'replays', 0) - r0) * getattr(step, 'launches_per_replay', 0)
+    if outputs is not None:                 # copied before the end-to-end steps below train on
+        outputs.update(host_arrays({'loss': last[0], 'parameters': step.flat_p}))
     comm = step.comm_events
     step.comm_events = None
     ms_e2e = ctx.timed(e2e, steps)
@@ -689,7 +724,14 @@ def main():
     ap.add_argument('--no-train-graph', action='store_true', help='training: launch every kernel eagerly instead of replaying the captured CUDA graph')
     ap.add_argument('--infer-batch', type=int, default=646, help='patches per forward of the U-Net inference workloads')
     ap.add_argument('--no-extras', action='store_true', help='headline only: skip the `workloads`, `other_modes` and `dropin_e2e` legs')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write what the last timed step of the headline workload returned (rank 0) as DIR/<name>.npy, float32 or float64, '
+                         'at most 64 MB in all; the inputs are seeded, so two builds can be compared output for output')
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error('--steps must be >= 1 and --warmup >= 0')
+    if args.dump_outputs and args.impl != 'b200':
+        ap.error('--dump-outputs writes the outputs of the b200 implementation only')
 
     rank = int(os.environ.get('RANK', 0))
     world = int(os.environ.get('WORLD_SIZE', 1))
@@ -712,6 +754,7 @@ def main():
     spec = WORKLOADS[headline]
     line = {}
     parity = None
+    outputs = {} if args.dump_outputs else None
     if spec['kind'] == 'infer':
         precision = args.precision
         if headline == 'infer_drcnn' and not (args.no_extras and precision != 'auto'):
@@ -723,11 +766,13 @@ def main():
                 parity['fp16']['meets_1e-3'] = bool(flag.item())
         if precision == 'auto':
             precision = 'fp16' if (parity is None or parity['fp16']['meets_1e-3']) else 'fp16x3'
-        r = run_infer(ctx, headline, precision, args.steps, args.warmup, args.preload, detail=True, e2e_first=args.e2e_first)
+        r = run_infer(ctx, headline, precision, args.steps, args.warmup, args.preload, detail=True, e2e_first=args.e2e_first, outputs=outputs)
         metric, unit = 'audio_seconds_per_second', 'audio-s/s'
     else:
-        r = run_train(ctx, headline, args.train_precision, args.steps, args.warmup, args.preload)
+        r = run_train(ctx, headline, args.train_precision, args.steps, args.warmup, args.preload, outputs=outputs)
         metric, unit = 'train_patches_per_second', 'patches/s'
+    if args.dump_outputs and rank == 0:
+        write_outputs(args.dump_outputs, outputs)
     line = {'metric': metric, 'value': r.pop('value'), 'unit': unit, 'n_gpus': world, 'steps': args.steps, 'warmup': args.warmup,
             'ms_per_step': r.pop('ms_per_step'), 'higher_is_better': True, 'scaling': 'weak', 'vs_baseline': None, 'dtype': r.pop('dtype'),
             'data': 'synthetic', 'config': workload_config(headline, args)}
