@@ -519,9 +519,9 @@ class PackJob(_ct.Structure):
 
 
 class PackPlan:
-    """The conv_tc_pack_dev calls of one training step, recorded during the first step of their owner (a fused train step whose
-    parameters are views of one flat buffer: stable pointers) and from then on re-packed by ONE launch at the start of every step
-    (mpa_conv_tc_pack_weights_multi); the individual calls then just hand out their persistent buffer."""
+    """The conv_tc_pack_dev calls of one fused training step (its parameters are views of one flat buffer: stable pointers), recorded
+    during its first step and from then on re-packed by ONE launch at the start of every step (mpa_conv_tc_pack_weights_multi); the
+    individual calls then just hand out their persistent buffer."""
 
     def __init__(self):
         self.index, self.jobs, self.table, self.fresh = {}, [], None, False
@@ -545,15 +545,12 @@ class PackPlan:
         self.table = torch.frombuffer(bytearray(host), dtype=torch.uint8).to(dev)
 
 
-_PACK_PLAN = None
-
-
-def conv_tc_pack_dev(w, Cin, Cout, ksize, fmt, transpose_flip=False, Cout_total=None, co0=0, J=0, split=0, C0=0):
+def conv_tc_pack_dev(w, Cin, Cout, ksize, fmt, transpose_flip=False, Cout_total=None, co0=0, J=0, split=0, C0=0, plan=None):
     """Device-side packing of conv_tc A-operand tiles from the fp32 weight tensor `w` (state_dict layout, on the GPU).
     transpose_flip: pack the data-gradient convolution of the forward weight `w` (see mpa_conv_tc_pack_weights_dev).
-    split = s, C0: the phase-split form of a KH x s / stride (1, s) convolution with C0 real input channels (mpa_conv_tc_pack_weights_split_dev)."""
+    split = s, C0: the phase-split form of a KH x s / stride (1, s) convolution with C0 real input channels (mpa_conv_tc_pack_weights_split_dev).
+    plan: the PackPlan of the calling train step (None: a fresh buffer packed by its own launch)."""
     KH, KW = ksize
-    plan = _PACK_PLAN
     Ct = Cout if Cout_total is None else Cout_total
     key = (w.data_ptr(), Cin, Cout, KH, KW, fmt, int(bool(transpose_flip)), Ct, co0, J, split, C0)
     if plan is not None and plan.fresh and key in plan.index:

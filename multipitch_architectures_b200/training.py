@@ -13,27 +13,94 @@ With `precision='bf16'` the convolutions run on the tensor cores (TcConv) and, f
 gradients stay in the 16-bit CP8 planes between the block convolutions (`_cp8_resident`: pool + dropout forward / backward and the bias
 gradients are train_cp8.cu kernels; bit-identical to crossing the nchw<->CP8 converters around the fp32 kernels).
 Dropout uses a Philox stream (seed, per-site offset); the reference's torch RNG stream cannot be reproduced, so parity
-tests run with p_dropout = 0 (SURVEY.md §7)."""
+tests run with p_dropout = 0 (SURVEY.md §7).
+
+`FusedTrainStep` is the fused step of both families (`TrainStep` here, `training_unet.UnetTrainStep`).  What a step keeps from one call to
+the next — pooled activation / gradient planes, the pack plan of its weights, the side stream of its weight gradients, the device-side step
+counter of a graph capture — lives in its `StepState`, which the step makes active around its forward and backward.  Calls made outside any
+step (the autograd bridge, direct TcConv calls) allocate fresh planes, pack without a plan, compute weight gradients inline and form dropout
+offsets on the host."""
+import contextlib
+
 import torch
 
 from . import _lib, ops
 from .libdl.nn_models import _exec
 from ._lib import call, stream_ptr
 
+SITES_PER_STEP = 64       # dropout sites reserved per step of the CNN path: offset = step * 64 + site
 
-# Device-resident step counter (int64[1]) while a training step is being captured into a CUDA graph: dropout offsets are then formed on
-# the device as step * 256 + site instead of being baked into the kernel arguments.
-_step_dev = None
-_step_mul = 256        # offset = step * _step_mul + site (256 sites per step in the U-Net tape, 64 in the CNN path)
+
+class StepState:
+    """What one fused training step keeps from call to call: the pooled CP8 / byte / phase-split buffers (keyed by tag and shape; the step
+    runs forward and backward atomically, so reusing the SAVED planes across its calls is safe), the PackPlan of its convolution weights,
+    the side stream of its weight gradients with the tensors they read (`keep`) and whether the main stream still has to wait for them
+    (`dirty`), and — while the step is captured into a CUDA graph — the device-side step counter (int64[1]) its dropout offsets are formed
+    from as counter * sites_per_step + site."""
+
+    def __init__(self, dev, sites_per_step):
+        self.pool, self.plan = {}, ops.PackPlan()
+        self.side, self.keep, self.dirty = torch.cuda.Stream(device=dev), [], False
+        self.step_dev, self.sites_per_step = None, sites_per_step
+
+    @contextlib.contextmanager
+    def active(self, refresh=True):
+        """Make this the active state.  refresh: the scope opens a step, whose packed operands are refreshed by one launch (from the second
+        step on); False: the second half of a step, whose operands the first half refreshed.  On the way out — a raising stage included —
+        the current stream waits for the weight gradients issued on the side stream, and their kept tensors are let go.  The plan is built
+        after the first scope that completes."""
+        global _active
+        prev, _active = _active, self
+        plan = self.plan
+        if refresh:
+            plan.fresh = False
+            plan.refresh()
+        else:
+            plan.fresh = plan.table is not None
+        try:
+            yield self
+        finally:
+            if self.dirty:
+                torch.cuda.current_stream().wait_stream(self.side)
+                self.dirty = False
+            self.keep.clear()
+            _active, plan.fresh = prev, False
+        plan.build()
+
+
+_active = None            # the StepState of the fused step being run; None = outside any step
+
+
+def _pooled(key, make):
+    """make() once per key for the active step; outside any step every call gets a fresh one — the autograd bridge may run a second forward
+    before the first backward (gradient accumulation, two losses, two same-shape models), and the planes are what the backward reads."""
+    if _active is None:
+        return make()
+    b = _active.pool.get(key)
+    if b is None:
+        b = _active.pool[key] = make()
+    return b
+
+
+def _pack(w, *args, **kw):
+    """ops.conv_tc_pack_dev under the pack plan of the active step (no plan outside a step)."""
+    return ops.conv_tc_pack_dev(w, *args, plan=_active.plan if _active is not None else None, **kw)
+
+
+def _step_args():
+    """(device step counter, sites per step) while a step is captured into a CUDA graph, else (None, 0): offsets formed on the host."""
+    if _active is None or _active.step_dev is None:
+        return None, ctypes_u64(0)
+    return _active.step_dev, ctypes_u64(_active.sites_per_step)
 
 
 def _dropout(x, p, seed, offset):
     if p <= 0.0:
         return x
     out = torch.empty_like(x)
-    if _step_dev is not None:
-        call('dropout_dev_f32', x, out, _lib.i64(x.numel()), float(p), ctypes_u64(seed), ctypes_u64(offset), _step_dev, ctypes_u64(_step_mul),
-             stream_ptr())
+    sd, sm = _step_args()
+    if sd is not None:
+        call('dropout_dev_f32', x, out, _lib.i64(x.numel()), float(p), ctypes_u64(seed), ctypes_u64(offset), sd, sm, stream_ptr())
         return out
     call('dropout_f32', x, out, _lib.i64(x.numel()), float(p), ctypes_u64(seed), ctypes_u64(offset), stream_ptr())
     return out
@@ -93,8 +160,6 @@ def _wgrad(conv, x, g, gw, gb):
          conv.padding[1], stream_ptr())
 
 
-WGRAD_SIDE = True          # test knob: False = weight gradients on the main stream, in front of the data gradient of their layer
-PACK_MULTI = True          # test knob: False = one weight-packing launch per convolution and direction
 ROWS_TC = True             # test knob: False = conv3 of the bf16 models on the fp32 strided-GEMM kernels (conv_rows.cu)
 
 
@@ -130,7 +195,7 @@ def _rows_tc_backward(conv, x, g, gw, gb, need_dx):
         gt = ops.strided_chunks(g, Cout, Mt, 256, fm, (Cout, 0, W), (W, Cout * W, 1))
         xt = ops.strided_chunks(x, K, Mt, 128, fm, (K, 0, W), (W, K * W, 1))
         ops.gemm_tc_ex(gt, xt, None, Cout, K, Mt, False, fm, y=gw.view(Cout, K))
-    TcConv.wgrad_async(g.device, wgrad, keep=(g, x))
+    TcConv.wgrad_async(wgrad, keep=(g, x))
     ops.channel_sum(g, out=gb)
     if not need_dx:
         return None
@@ -154,10 +219,6 @@ def _act_bwd(out, g, act, a=0.0):
 
 
 FUSE_POOL_DROPOUT = True      # test knob: False = separate pool / dropout (/ add) kernels; the results are identical
-
-
-def _step_args():
-    return _step_dev, ctypes_u64(_step_mul if _step_dev is not None else 0)
 
 
 def _pool_dropout(act_t, k, res, p, seed, offset):
@@ -197,7 +258,6 @@ class TcConv:
     mpa_conv_wgrad_tc, bias gradient = a channel reduction.  Activations and gradients cross the boundary through nchw<->CP8 converters
     (16-bit operands, fp32 accumulation; the optimiser state and every element-wise stage stay fp32)."""
     PF, PT = 8, 1
-    _pool = {}
 
     @staticmethod
     def eligible(model, conv, F):
@@ -205,104 +265,34 @@ class TcConv:
         return (getattr(model, 'precision', 'fp32') == 'bf16' and tuple(conv.stride) == (1, 1) and KH % 2 == 1 and KW % 2 == 1 and 3 <= KW <= 15 and KH >= 3
                 and tuple(conv.padding) == (KH // 2, KW // 2) and F + TcConv.PF + 15 < 272 and conv.bias is not None)
 
-    _scope = None           # owner of the pooled buffers (a TrainStep); None = allocate per call
-
-    @classmethod
-    def scope(cls, owner, refresh=True):
-        """Context manager: inside it `_buf` hands out buffers pooled under `owner` (a fused train step, which runs forward and backward
-        atomically, so reusing the SAVED activation planes across steps is safe).  Outside any scope — the autograd bridge, where a
-        second forward may run before the first backward (gradient accumulation, two losses, two same-shape models) — every call gets
-        fresh planes, because the planes are what the backward reads."""
-        import contextlib
-
-        @contextlib.contextmanager
-        def cm():
-            prev, cls._scope = cls._scope, id(owner)
-            plan = cls._plans.get(id(owner))
-            if plan is None:
-                plan = cls._plans[id(owner)] = ops.PackPlan()
-            prev_plan, ops._PACK_PLAN = ops._PACK_PLAN, plan
-            if refresh:
-                plan.fresh = False
-                if PACK_MULTI:
-                    plan.refresh()       # every packed operand of the step in one launch (from the second step on)
-            else:
-                plan.fresh = plan.table is not None and PACK_MULTI      # second half of a step: the operands were refreshed by the first
-            try:
-                yield
-                cls.join()
-                if PACK_MULTI:
-                    plan.build()
-            finally:
-                cls._scope, ops._PACK_PLAN = prev, prev_plan
-                plan.fresh = False
-        return cm()
-
-    _plans = {}
-
-    @classmethod
-    def release(cls, owner):
-        """Drop every pooled buffer of `owner`."""
-        for k in [k for k in cls._pool if k[0] == id(owner)]:
-            del cls._pool[k]
-        cls._plans.pop(id(owner), None)
-
     @classmethod
     def _buf(cls, tag, B, C, T, F, dev, fmt):
-        """CP8 scratch reused across the steps of one owner (zero gap columns are never written, so they stay zero)."""
+        """CP8 scratch pooled by the active step (zero gap columns are never written, so they stay zero)."""
         pitch = (F + cls.PF + 15) // 16 * 16
-        if cls._scope is None:
-            return ops.CP8(B, C, T, F, pitch, cls.PF, cls.PT, dev, fmt=fmt)
-        key = (cls._scope, tag, B, C, T, F, str(dev), fmt)
-        b = cls._pool.get(key)
-        if b is None:
-            b = ops.CP8(B, C, T, F, pitch, cls.PF, cls.PT, dev, fmt=fmt)
-            cls._pool[key] = b
-        return b
+        return _pooled(('cp8', tag, B, C, T, F, fmt), lambda: ops.CP8(B, C, T, F, pitch, cls.PF, cls.PT, dev, fmt=fmt))
 
-    # Weight gradients on a side stream: inside a fused train step (scope set) the weight gradient of a convolution is independent of
-    # everything that follows it in the backward (it reads the saved input planes and the dy planes of its own layer — pooled per layer,
-    # not reused within the step — and writes its own slice of the flat gradient buffer), so it is issued on a second stream and joined
-    # at the end of the backward: the small, latency-bound layers of the deep U-Net levels then run side by side with the data-gradient
-    # chain instead of in front of it.  Under CUDA-graph capture the fork / join become parallel branches of the graph.
-    _side_streams, _side_dirty = {}, False
-
-    _keep = []
-
-    @classmethod
-    def wgrad_async(cls, dev, fn, keep=()):
-        """keep: tensors allocated on the main stream that `fn` reads — held until the join, so that the allocator cannot hand their memory
-        to later main-stream work while the side stream still reads it."""
-        if not WGRAD_SIDE or cls._scope is None:
+    @staticmethod
+    def wgrad_async(fn, keep=()):
+        """Weight gradients on a side stream: inside a fused train step the weight gradient of a convolution is independent of everything
+        that follows it in the backward (it reads the saved input planes and the dy planes of its own layer — pooled per layer, not reused
+        within the step — and writes its own slice of the flat gradient buffer), so `fn` is issued on the step's second stream and joined
+        when the step's scope ends: the small, latency-bound layers of the deep U-Net levels then run side by side with the data-gradient
+        chain instead of in front of it.  Under CUDA-graph capture the fork / join become parallel branches of the graph.  keep: tensors
+        allocated on the main stream that `fn` reads — held until the join, so that the allocator cannot hand their memory to later
+        main-stream work while the side stream still reads it.  Outside any step: fn() inline."""
+        st = _active
+        if st is None:
             return fn()
-        cls._keep.extend(keep)
-        side = cls._side_streams.get(str(dev))
-        if side is None:
-            side = cls._side_streams[str(dev)] = torch.cuda.Stream(device=dev)
-        side.wait_stream(torch.cuda.current_stream())
-        with torch.cuda.stream(side):
+        st.keep.extend(keep)
+        st.side.wait_stream(torch.cuda.current_stream())
+        with torch.cuda.stream(st.side):
             fn()
-        cls._side_dirty = True
+        st.dirty = True
 
-    @classmethod
-    def join(cls):
-        """The current stream waits for the weight gradients issued so far."""
-        if cls._side_dirty:
-            for side in cls._side_streams.values():
-                torch.cuda.current_stream().wait_stream(side)
-            cls._side_dirty = False
-        cls._keep.clear()
-
-    @classmethod
-    def _raw(cls, tag, nbytes, zero, dev):
+    @staticmethod
+    def _raw(tag, nbytes, zero, dev):
         """Byte scratch pooled like `_buf` (zero: zero-filled when it is created; the users never dirty the parts that must stay zero)."""
-        if cls._scope is None:
-            return (torch.zeros if zero else torch.empty)(nbytes, dtype=torch.uint8, device=dev)
-        key = (cls._scope, tag, nbytes, str(dev), bool(zero))
-        b = cls._pool.get(key)
-        if b is None:
-            b = cls._pool[key] = (torch.zeros if zero else torch.empty)(nbytes, dtype=torch.uint8, device=dev)
-        return b
+        return _pooled(('raw', tag, nbytes, bool(zero)), lambda: (torch.zeros if zero else torch.empty)(nbytes, dtype=torch.uint8, device=dev))
 
     @staticmethod
     def _pad8(v, n):
@@ -340,7 +330,7 @@ class TcConv:
         for c0 in range(0, Cout, 128):
             c = min(128, Cout - c0)
             cp = (c + 7) // 8 * 8                        # whole chunks: the coalesced epilogue needs Cout % 8 == 0
-            wp = ops.conv_tc_pack_dev(conv.weight, Cin, cp, (KH, KW), fmt, False, Cout, c0)
+            wp = _pack(conv.weight, Cin, cp, (KH, KW), fmt, False, Cout, c0)
             ops.conv_tc(xc, wp, cls._pad8(conv.bias[c0:c0 + c], cp), cp, (KH, KW), act, a, out=yc.channels(c0, cp))
         return yc
 
@@ -362,7 +352,7 @@ class TcConv:
         B, Cout, T, F = gc.B, gc.C, gc.T, gc.F
         _, Cin, KH, KW = conv.weight.shape
         dev = gc.buf.device
-        cls.wgrad_async(dev, lambda: ops.conv_wgrad_tc(xc, gc, gw, (KH, KW)))
+        cls.wgrad_async(lambda: ops.conv_wgrad_tc(xc, gc, gw, (KH, KW)))
         if gb is not None:
             ops.channel_sum_cp8(gc, out=gb)
         if not need_dx:
@@ -372,7 +362,7 @@ class TcConv:
         for c0 in range(0, Cin, 128):
             c = min(128, Cin - c0)
             cp = (c + 7) // 8 * 8
-            wp = ops.conv_tc_pack_dev(conv.weight, Cout, cp, (KH, KW), fmt, True, Cin, c0)
+            wp = _pack(conv.weight, Cout, cp, (KH, KW), fmt, True, Cin, c0)
             ops.conv_tc(gc, wp, zb[:cp], cp, (KH, KW), ops.ACT_NONE, 0.0, out=gxc.channels(c0, cp))
         return gxc
 
@@ -398,7 +388,7 @@ def _tc_s3_forward(tag, conv, x, act, a):
     for c0 in range(0, Cout, 128):
         c = min(128, Cout - c0)
         cp = (c + 7) // 8 * 8
-        wp = ops.conv_tc_pack_dev(conv.weight, Cin, cp, (3, 3), fmt, False, Cout, c0)
+        wp = _pack(conv.weight, Cin, cp, (3, 3), fmt, False, Cout, c0)
         ops.conv_tc(xc, wp, TcConv._pad8(conv.bias[c0:c0 + c], cp), cp, (3, 3), act, a, subsample=(3, 1), out=yc.channels(c0, cp))
     return ops.cp8_to_nchw(yc), xc
 
@@ -409,14 +399,14 @@ def _tc_s3_backward(tag, conv, xc, g, gw, gb, keep_cp8=False):
     Cin, F = conv.weight.shape[1], xc.F
     gc = TcConv._buf(tag + ':g3', B, Cout, T, F, g.device, fmt)
     call('nchw_to_cp8_strided', g, gc.ptr(), B, Cout, T, Fo, F, 3, 1, gc.pitch, gc.pf, gc.pt, fmt, gc.ncs, stream_ptr())
-    TcConv.wgrad_async(g.device, lambda: ops.conv_wgrad_tc(xc, gc, gw, (3, 3)))
+    TcConv.wgrad_async(lambda: ops.conv_wgrad_tc(xc, gc, gw, (3, 3)))
     ops.channel_sum(g, out=gb)
     gxc = TcConv._buf(tag + ':gx', B, Cin, T, F, g.device, fmt)
     zb = TcConv._zero_bias(g.device)
     for c0 in range(0, Cin, 128):
         c = min(128, Cin - c0)
         cp = (c + 7) // 8 * 8
-        wp = ops.conv_tc_pack_dev(conv.weight, Cout, cp, (3, 3), fmt, True, Cin, c0)
+        wp = _pack(conv.weight, Cout, cp, (3, 3), fmt, True, Cin, c0)
         ops.conv_tc(gc, wp, zb[:cp], cp, (3, 3), ops.ACT_NONE, 0.0, out=gxc.channels(c0, cp))
     return gxc if keep_cp8 else ops.cp8_to_nchw(gxc)
 
@@ -436,13 +426,7 @@ def _s3_split_eligible(model, conv, F):
 
 def _split_buf(tag, B, C, T, F, s, dev, fmt):
     """Phase-split planes (ops.split_cp8) pooled like TcConv._buf."""
-    if TcConv._scope is None:
-        return ops.split_cp8(B, C, T, F, s, dev, fmt)
-    key = (TcConv._scope, tag, 'split', B, C, T, F, s, str(dev), fmt)
-    b = TcConv._pool.get(key)
-    if b is None:
-        b = TcConv._pool[key] = ops.split_cp8(B, C, T, F, s, dev, fmt)
-    return b
+    return _pooled(('split', tag, B, C, T, F, s, fmt), lambda: ops.split_cp8(B, C, T, F, s, dev, fmt))
 
 
 def _tc_s3_forward_split(tag, conv, xs, act, a):
@@ -455,7 +439,7 @@ def _tc_s3_forward_split(tag, conv, xs, act, a):
     for c0 in range(0, Cout, 128):
         c = min(128, Cout - c0)
         cp = (c + 7) // 8 * 8
-        wp = ops.conv_tc_pack_dev(conv.weight, 3 * C0p, cp, (3, 1), fmt, False, Cout, c0, J=J, split=3, C0=C0)
+        wp = _pack(conv.weight, 3 * C0p, cp, (3, 1), fmt, False, Cout, c0, J=J, split=3, C0=C0)
         ops.conv_tc(xs, wp, TcConv._pad8(conv.bias[c0:c0 + c], cp), cp, (3, 1), act, a, subsample=(1, 0), out=yc.channels(c0, cp), J=J)
     return ops.cp8_to_nchw(yc), xs
 
@@ -474,7 +458,7 @@ def _tc_s3_backward_split(tag, conv, xs, g, gw, gb):
     zb = TcConv._zero_bias(dev)
     for c0 in range(0, 3 * C0p, 128):
         cp = min(128, 3 * C0p - c0)
-        wp = ops.conv_tc_pack_dev(conv.weight, Cout, cp, (3, 1), fmt, True, 3 * C0p, c0, split=3, C0=C0)
+        wp = _pack(conv.weight, Cout, cp, (3, 1), fmt, True, 3 * C0p, c0, split=3, C0=C0)
         ops.conv_tc(gc, wp, zb[:cp], cp, (3, 1), ops.ACT_NONE, 0.0, out=gxs.channels(c0, cp))
     return gxs
 
@@ -535,12 +519,12 @@ def cnn_train_forward(model, x, seed=0, step=0):
     a, p = model.a_lrelu, (model.p_dropout if model.training else 0.0)
     blocks = _exec.cnn_blocks(model)
     residual = getattr(model, 'residual', False)
-    site = [step * 64]
+    site = [step * SITES_PER_STEP]
 
     def drop(t):
         site[0] += 1
         return _dropout(t, p, seed, site[0])
-    sv = {'x': x, 'blocks': [], 'p': p, 'seed': seed, 'site0': step * 64}
+    sv = {'x': x, 'blocks': [], 'p': p, 'seed': seed, 'site0': step * SITES_PER_STEP}
     if _cp8_resident(model, blocks, x.shape[3]) and x.shape[1] <= 8:
         return _cnn_train_forward_cp8(model, blocks, x, sv, site, drop)
     z = ops.layernorm_cf(x, model.layernorm.weight, model.layernorm.bias, model.layernorm.eps)
@@ -662,12 +646,16 @@ def cnn_forward_train(model, x):
     return CnnTrainFunction.apply(model, x, seed, model._train_calls, *[p for _, p in model.named_parameters()])
 
 
-class TrainStep:
-    """Fused training step on flat parameter / gradient / moment buffers (one all-reduce, one AdamW sweep)."""
+class FusedTrainStep:
+    """Fused training step on flat parameter / gradient / moment buffers: the subclass's forward, loss and backward, ONE gradient all-reduce
+    (NCCL, when a process group is active), fused AdamW.  A subclass supplies `_forward_backward` and `sites_per_step`; one whose parameters
+    start with an encoder trunk sets `n_trunk` and supplies `_trunk_backward` (UnetTrainStep)."""
+    sites_per_step = None
 
     def __init__(self, model, lr=1e-3, betas=(0.9, 0.999), eps=1e-8, weight_decay=0.01, seed=0x5EED, process_group=None, graph=False):
-        """graph=True: from the third step on, forward + loss + backward replay ONE captured CUDA graph (fixed input shape; dropout offsets
-        come from a device-side step counter, so a replayed step equals the eager step of the same number); all-reduce and AdamW stay eager."""
+        """graph=True: after two eager steps forward + loss + backward are captured ONCE into a CUDA graph and replayed (fixed input shape;
+        dropout offsets come from a device-side step counter, so a replayed step equals the eager step of the same number); the all-reduce
+        and AdamW stay eager."""
         self.model, self.lr, self.betas, self.eps, self.wd, self.seed = model, lr, betas, eps, weight_decay, seed
         self.group = process_group
         named = list(model.named_parameters())
@@ -686,63 +674,97 @@ class TrainStep:
                 self.grads[name] = self.flat_g[off:off + k].view_as(p)
                 off += k
         self.step_count = 0
-        self.use_graph, self._graph = bool(graph), None
+        self.use_graph, self._graph, self._graph2 = bool(graph), None, None
+        self.n_trunk, self.overlap_comm = 0, False     # no trunk split: one flat all-reduce after the backward
+        self.comm_events = None                        # bench.py: a list that receives CUDA events around the all-reduce
+        self._state = StepState(dev, self.sites_per_step)
 
-    def _forward_backward(self, x, target, tape_step):
-        with TcConv.scope(self):
-            y, sv = cnn_train_forward(self.model, x, self.seed, tape_step)
-            loss, g_y = ops.bce_fwd_bwd(y, target.contiguous())
-            cnn_train_backward(self.model, sv, g_y, self.grads)
-        return loss
+    def _forward_backward(self, x, target, tape_step, split):
+        """-> loss (the step state is active).  split: stop the backward at the trunk (its part follows in _trunk_backward)."""
+        raise NotImplementedError
 
     def release(self):
-        """Free the pooled activation planes of this step (and the captured graph that points into them)."""
-        self._graph = None
-        TcConv.release(self)
+        """Free the pooled activation planes and the pack plan of this step, and the captured graphs that point into them (dropping the
+        step frees them too)."""
+        self._graph = self._graph2 = None
+        self._state = StepState(self.flat_p.device, self.sites_per_step)
 
-    def _capture(self, x, target):
-        global _step_dev, _step_mul
+    def _capture(self, x, target, split):
         self._xs, self._ts = x.clone(), target.contiguous().clone()
-        self._step_dev = torch.zeros(1, dtype=torch.int64, device=x.device)
-        self._graph = torch.cuda.CUDAGraph()
+        self._graph, self._graph2 = torch.cuda.CUDAGraph(), None
+        self._counter = self._state.step_dev = torch.zeros(1, dtype=torch.int64, device=x.device)    # read by the graph's dropout kernels
         n0 = _lib.launch_count()
-        with torch.cuda.graph(self._graph):
-            self._step_dev += 1
-            _step_dev, _step_mul = self._step_dev, 64
-            try:
-                self._loss = self._forward_backward(self._xs, self._ts, 0)
-            finally:
-                _step_dev, _step_mul = None, 256
-        self.launches_per_replay = _lib.launch_count() - n0
+        try:
+            with torch.cuda.graph(self._graph):
+                self._counter += 1
+                with self._state.active():
+                    self._loss = self._forward_backward(self._xs, self._ts, 0, split)
+            if split:                                  # the trunk's backward as a second graph (same memory pool): the all-reduce of the
+                self._graph2 = torch.cuda.CUDAGraph()  # finished gradients is issued between the two replays
+                with torch.cuda.graph(self._graph2, pool=self._graph.pool()), self._state.active(refresh=False):
+                    self._trunk_backward()
+        finally:
+            self._state.step_dev = None
+        self.launches_per_replay = _lib.launch_count() - n0      # libmpa kernels inside the graph(s) (the host counter does not see replays)
         self.replays = 0
-        self._step_dev.fill_(self.step_count - 1)
+        self._counter.fill_(self.step_count - 1)
 
     def __call__(self, x, target):
         import torch.distributed as dist
         self.step_count += 1
         with torch.no_grad():
-            if self.use_graph and self.step_count > 2:
+            multi = self.group is not None or (dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1)
+            split = bool(multi and self.overlap_comm and self.n_trunk > 0)
+            graphed = self.use_graph and self.step_count > 2
+            if graphed:
                 if self._graph is None:
-                    self._capture(x, target)
+                    self._capture(x, target, split)
                 self._xs.copy_(x)
                 self._ts.copy_(target)
                 self._graph.replay()
                 self.replays += 1
                 loss = self._loss
             else:
-                loss = self._forward_backward(x, target, self.step_count)
+                with self._state.active():
+                    loss = self._forward_backward(x, target, self.step_count, split)
             scale = 1.0
-            if self.group is not None or (dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1):
-                ev = getattr(self, 'comm_events', None)
-                if ev is not None:                    # bench.py: CUDA events around the collective (time of the all-reduce per step)
+            if multi:
+                ev = self.comm_events
+                if split:
+                    w_a = dist.all_reduce(self.flat_g[self.n_trunk:], group=self.group, async_op=True)    # NCCL's stream waits for the work so far
+                    if graphed:
+                        self._graph2.replay()
+                    else:
+                        with self._state.active(refresh=False):
+                            self._trunk_backward()
+                if ev is not None:                    # CUDA events around the part of the collective the step waits for
                     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
                     e0.record()
-                dist.all_reduce(self.flat_g, group=self.group)
+                if split:
+                    w_b = dist.all_reduce(self.flat_g[:self.n_trunk], group=self.group, async_op=True)
+                    w_a.wait()
+                    w_b.wait()
+                else:
+                    dist.all_reduce(self.flat_g, group=self.group)
                 if ev is not None:
                     e1.record()
                     ev.append((e0, e1))
                 scale = 1.0 / dist.get_world_size(self.group)
             call('adamw_f32', self.flat_p, self.flat_g, self.m, self.v, _lib.i64(self.flat_p.numel()), float(self.lr), float(self.betas[0]),
                  float(self.betas[1]), float(self.eps), float(self.wd), self.step_count, float(scale), stream_ptr())
-        _exec.invalidate_caches(self.model)   # packed operands derived from the old parameter values are stale
+        # the raw-pointer AdamW leaves data_ptr / _version unchanged: every ParamCache of the module tree (model, encoder layers, BLSTM
+        # layers) is stale now
+        _exec.invalidate_caches(self.model)
+        return loss
+
+
+class TrainStep(FusedTrainStep):
+    """Fused training step of the CNN family.  Its backward is one piece: n_trunk stays 0 (its parameter names begin with `layernorm.`
+    like a U-Net trunk's, but the CNN tape cannot stop half-way)."""
+    sites_per_step = SITES_PER_STEP
+
+    def _forward_backward(self, x, target, tape_step, split):
+        y, sv = cnn_train_forward(self.model, x, self.seed, tape_step)
+        loss, g_y = ops.bce_fwd_bwd(y, target.contiguous())
+        cnn_train_backward(self.model, sv, g_y, self.grads)
         return loss

@@ -19,8 +19,11 @@ import torch
 from . import _lib, ops
 from ._lib import call, stream_ptr
 from .libdl.nn_models import _exec
-from .training import (TcConv, ctypes_u64, _s3_split_eligible, _split_buf, _tc_s3_backward_split, _tc_s3_forward_split, _rows_tc_backward, _rows_tc_eligible, _rows_tc_forward, _act_bwd, _add, _conv_fwd, _dgrad, _dropout, _pool_bwd, _tc_s3_backward, _tc_s3_eligible, _tc_s3_forward,
-                       _wgrad)
+from .training import (FusedTrainStep, TcConv, ctypes_u64, _s3_split_eligible, _split_buf, _step_args, _tc_s3_backward_split, _tc_s3_forward_split,
+                       _rows_tc_backward, _rows_tc_eligible, _rows_tc_forward, _act_bwd, _add, _conv_fwd, _dgrad, _dropout, _pool_bwd, _tc_s3_backward,
+                       _tc_s3_eligible, _tc_s3_forward, _wgrad)
+
+SITES_PER_STEP = 256      # dropout sites reserved per step of the U-Net tape: offset = step * 256 + site
 
 
 class Node:
@@ -36,7 +39,7 @@ class Node:
 
 class Tape:
     def __init__(self, grads, seed, step, model=None):
-        self.ops, self.grads, self.seed, self.site, self.model = [], grads, seed, step * 256, model
+        self.ops, self.grads, self.seed, self.site, self.model = [], grads, seed, step * SITES_PER_STEP, model
         self.trunk_mark = 0
 
     def push(self, fn):
@@ -301,8 +304,7 @@ class Tape:
                 site_tok = self.site
             self.site += 1
             site_att = self.site
-        from . import training as T
-        sd, sm = T._step_dev, ctypes_u64(T._step_mul if T._step_dev is not None else 0)
+        sd, sm = _step_args()
         t, qkv, att, u1, h1 = f32(M, E), f32(M, 3 * E), f32(M, E), f32(M, E), f32(M, E)
         call('enc_attn_train_fwd_f32', x.d, pe, w_qkvT, at.in_proj_bias, w_projT, b_proj, layer.layernorm1.weight, layer.layernorm1.bias,
              float(layer.layernorm1.eps), t, qkv, att, u1, h1, B, E, S, H, float(p_drop), ctypes_u64(self.seed), ctypes_u64(site_tok),
@@ -311,7 +313,7 @@ class Tape:
 
         def bwd():
             g_p, g_qkv, g_x = f32(M, E), f32(M, 3 * E), f32(B, E, Th, Fw)
-            sd_b, sm_b = T._step_dev, ctypes_u64(T._step_mul if T._step_dev is not None else 0)
+            sd_b, sm_b = _step_args()
             call('enc_attn_train_bwd_f32', h1.g, u1, qkv, w_qkv, w_proj, layer.layernorm1.weight, float(layer.layernorm1.eps), g_p, g_qkv, g_x,
                  G[name + '.layernorm1.weight'], G[name + '.layernorm1.bias'], B, E, S, H, int(pe is not None), float(p_drop),
                  ctypes_u64(self.seed), ctypes_u64(site_tok), ctypes_u64(site_att), sd_b, sm_b, stream_ptr())
@@ -325,7 +327,7 @@ class Tape:
                 call('enc_fold_bwd_f32', dWf, dWp, dbp, *params, G[name + '.attn.in_proj_weight'], G[name + '.q_linear.weight'],
                      G[name + '.k_linear.weight'], G[name + '.v_linear.weight'], G[name + '.o_linear.weight'], G[name + '.attn.out_proj.weight'],
                      G[name + '.attn.out_proj.bias'], E, stream_ptr())
-            TcConv.wgrad_async(dev, weight_grads, keep=(g_p, g_qkv, att, t))
+            TcConv.wgrad_async(weight_grads, keep=(g_p, g_qkv, att, t))
         self.push(bwd)
         return h1
 
@@ -445,7 +447,7 @@ class Tape:
                 ops.gemm_tc_ex(ops.gemm_tc_chunks(g_m2, 256, fm, True), hid_tok, None, E, Dm, M, False, fm, y=G[name + '.mlp.2.weight'],
                                w_rows=rows_t)
                 colsum(g_m2, M, E, out=G[name + '.mlp.2.bias'])
-            TcConv.wgrad_async(dev, dw2, keep=(g_m2,))
+            TcConv.wgrad_async(dw2, keep=(g_m2,))
             # g_hid = (g_m2 W2) * [hid > 0] -> both operand layouts, bias gradient = its column sums
             ghid_tok = TcConv._raw(name + ':ghid_tok', KCt * rows_t * 16, True, dev)
             ghid_feat = TcConv._raw(name + ':ghid_feat', Np8 * Mp * 16, False, dev)
@@ -454,8 +456,8 @@ class Tape:
             ops.gemm_tc_ex(ops.gemm_tc_chunks(g_m2, 256, fm), ops.gemm_tc_chunks(W2, 128, fm, True), None, M, Dm, E, False, fm, y_tok=ghid_tok,
                            y_tok_rows=rows_t, y_tok_chunks=KCt, y_feat=ghid_feat, y_feat_rows=Mp, mask_tok=hid_tok, colsum=gb1)
             # dW1 [Dm, E] = g_hid^T h1;  g_h1 [M, E] = g_hid W1
-            TcConv.wgrad_async(dev, lambda: ops.gemm_tc_ex(ghid_tok, ops.gemm_tc_chunks(h1.d, 128, fm, True), None, Dm, E, M, False, fm,
-                                                           y=G[name + '.mlp.0.weight'], x_rows=rows_t), keep=(h1.d,))
+            TcConv.wgrad_async(lambda: ops.gemm_tc_ex(ghid_tok, ops.gemm_tc_chunks(h1.d, 128, fm, True), None, Dm, E, M, False, fm,
+                                                      y=G[name + '.mlp.0.weight'], x_rows=rows_t), keep=(h1.d,))
             h1.acc(ops.gemm_tc_ex(ghid_feat, ops.gemm_tc_chunks(W1, 128, fm, True), None, M, E, Dm, False, fm, y=f32(M, E)))
 
         def bwd_mlp():
@@ -682,40 +684,21 @@ def unet_forward_train(model, x):
     return UnetTrainFunction.apply(model, x, seed, model._train_calls, *[p for _, p in model.named_parameters()])
 
 
-class UnetTrainStep:
-    """Fused training step of a U-Net-family model on flat parameter / gradient / moment buffers:
-    forward, BCE (+ CE/25 for the PUnet), backward, ONE gradient all-reduce (NCCL, when a process group is active), fused AdamW."""
+class UnetTrainStep(FusedTrainStep):
+    """Fused training step of a U-Net-family model (FusedTrainStep): forward, BCE (+ CE/25 for the PUnet), backward, ONE gradient
+    all-reduce, fused AdamW.  graph=True replays ~3,500 kernel launches of the SAUnet:L (more host launch time than GPU time) from one graph."""
+    sites_per_step = SITES_PER_STEP
 
     def __init__(self, model, lr=1e-3, betas=(0.9, 0.999), eps=1e-8, weight_decay=0.01, seed=0x5EED, process_group=None, ce_scale=1.0 / 25.0,
                  graph=False, overlap_comm=True):
-        """graph=True: after two eager steps the forward + loss + backward sequence (~3,500 kernel launches for the SAUnet:L, more host
-        launch time than GPU time) is captured ONCE into a CUDA graph and replayed; the all-reduce and AdamW stay eager.  Inputs must keep
-        their shape.  The replayed step is the eager step of the same number (dropout offsets come from a device-side step counter)."""
-        self.model, self.lr, self.betas, self.eps, self.wd, self.seed = model, lr, betas, eps, weight_decay, seed
-        self.group, self.ce_scale = process_group, ce_scale
-        named = list(model.named_parameters())
-        dev = named[0][1].device
-        n = sum(p.numel() for _, p in named)
-        self.flat_p = torch.empty(n, dtype=torch.float32, device=dev)
-        self.flat_g = torch.zeros(n, dtype=torch.float32, device=dev)
-        self.m = torch.zeros(n, dtype=torch.float32, device=dev)
-        self.v = torch.zeros(n, dtype=torch.float32, device=dev)
-        self.grads, off = {}, 0
-        with torch.no_grad():
-            for name, p in named:
-                k = p.numel()
-                self.flat_p[off:off + k] = p.reshape(-1)
-                p.data = self.flat_p[off:off + k].view_as(p)
-                self.grads[name] = self.flat_g[off:off + k].view_as(p)
-                off += k
-        self.step_count = 0
-        self.use_graph, self._graph = bool(graph), None
+        super().__init__(model, lr, betas, eps, weight_decay, seed, process_group, graph)
+        self.ce_scale = ce_scale
         # Data-parallel runs overlap the gradient all-reduce with the backward: the parameters of the encoder trunk (layernorm, inc, down1-4)
         # are a PREFIX of the flat buffer; everything behind it (attention, decoder, head: ~3/4 of the SAUnet:L's bytes) is final once the
         # backward has reached the bottleneck, and is reduced on NCCL's stream while the trunk's backward still runs.
         self.overlap_comm = bool(overlap_comm)
-        self.n_trunk, seen_other = 0, False
-        for name, p in named:
+        seen_other = False
+        for name, p in model.named_parameters():
             trunk = name.startswith(('layernorm.', 'inc.', 'down'))
             if trunk and seen_other:
                 self.n_trunk = 0                       # not a prefix (unknown model layout): one flat all-reduce after the backward
@@ -726,97 +709,21 @@ class UnetTrainStep:
                 seen_other = True
         self._tape = None
 
-    def _forward_backward(self, x, target, tape_step, split=False):
-        """split: stop the backward at the bottleneck (the trunk's part follows in _trunk_backward)."""
-        with TcConv.scope(self):
-            y, n_pred, tape = unet_train_forward(self.model, x, self.grads, self.seed, tape_step)
-            target = target.contiguous()
-            loss, y.g = ops.bce_fwd_bwd(y.d, target)
-            if n_pred is not None:
-                B, K = n_pred.d.shape[0], n_pred.d.shape[1]
-                n_pred.g = torch.empty_like(n_pred.d)
-                call('ce_count_fwd_bwd_f32', n_pred.d, target, loss, n_pred.g, B, K, target.numel() // B, float(self.ce_scale), 1, stream_ptr())
-            if split:
-                tape.backward(lo=tape.trunk_mark)
-                self._tape = tape
-            else:
-                tape.backward()
+    def _forward_backward(self, x, target, tape_step, split):
+        y, n_pred, tape = unet_train_forward(self.model, x, self.grads, self.seed, tape_step)
+        target = target.contiguous()
+        loss, y.g = ops.bce_fwd_bwd(y.d, target)
+        if n_pred is not None:
+            B, K = n_pred.d.shape[0], n_pred.d.shape[1]
+            n_pred.g = torch.empty_like(n_pred.d)
+            call('ce_count_fwd_bwd_f32', n_pred.d, target, loss, n_pred.g, B, K, target.numel() // B, float(self.ce_scale), 1, stream_ptr())
+        if split:
+            tape.backward(lo=tape.trunk_mark)
+            self._tape = tape
+        else:
+            tape.backward()
         return loss
 
     def _trunk_backward(self):
-        with TcConv.scope(self, refresh=False):
-            tape, self._tape = self._tape, None
-            tape.backward()
-
-    def release(self):
-        """Free the pooled activation planes of this step (and the captured graph that points into them)."""
-        self._graph = self._graph2 = None
-        TcConv.release(self)
-
-    def _capture(self, x, target, split):
-        from . import training as T
-        self._xs, self._ts = x.clone(), target.contiguous().clone()
-        self._step_dev = torch.zeros(1, dtype=torch.int64, device=x.device)
-        self._graph = torch.cuda.CUDAGraph()
-        self._graph2 = None
-        n0 = _lib.launch_count()
-        T._step_dev, T._step_mul = self._step_dev, 256
-        try:
-            with torch.cuda.graph(self._graph):
-                self._step_dev += 1
-                self._loss = self._forward_backward(self._xs, self._ts, 0, split)
-            if split:                                  # the trunk's backward as a second graph (same memory pool): the all-reduce of the
-                self._graph2 = torch.cuda.CUDAGraph()  # finished gradients is issued between the two replays
-                with torch.cuda.graph(self._graph2, pool=self._graph.pool()):
-                    self._trunk_backward()
-        finally:
-            T._step_dev = None
-        self.launches_per_replay = _lib.launch_count() - n0      # libmpa kernels inside the graph(s) (the host counter does not see replays)
-        self.replays = 0
-        self._step_dev.fill_(self.step_count - 1)
-
-    def __call__(self, x, target):
-        import torch.distributed as dist
-        self.step_count += 1
-        with torch.no_grad():
-            multi = self.group is not None or (dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1)
-            split = bool(multi and self.overlap_comm and self.n_trunk > 0)
-            graphed = self.use_graph and self.step_count > 2
-            if graphed:
-                if self._graph is None:
-                    self._capture(x, target, split)
-                self._xs.copy_(x)
-                self._ts.copy_(target)
-                self._graph.replay()
-                self.replays += 1
-                loss = self._loss
-            else:
-                loss = self._forward_backward(x, target, self.step_count, split)
-            scale = 1.0
-            if multi:
-                ev = getattr(self, 'comm_events', None)
-                if split:
-                    w_a = dist.all_reduce(self.flat_g[self.n_trunk:], group=self.group, async_op=True)    # NCCL's stream waits for the work so far
-                    if graphed:
-                        self._graph2.replay()
-                    else:
-                        self._trunk_backward()
-                if ev is not None:                    # bench.py: CUDA events around the part of the collective the step waits for
-                    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-                    e0.record()
-                if split:
-                    w_b = dist.all_reduce(self.flat_g[:self.n_trunk], group=self.group, async_op=True)
-                    w_a.wait()
-                    w_b.wait()
-                else:
-                    dist.all_reduce(self.flat_g, group=self.group)
-                if ev is not None:
-                    e1.record()
-                    ev.append((e0, e1))
-                scale = 1.0 / dist.get_world_size(self.group)
-            call('adamw_f32', self.flat_p, self.flat_g, self.m, self.v, _lib.i64(self.flat_p.numel()), float(self.lr), float(self.betas[0]),
-                 float(self.betas[1]), float(self.eps), float(self.wd), self.step_count, float(scale), stream_ptr())
-        # the raw-pointer AdamW leaves data_ptr / _version unchanged: every ParamCache of the module tree (model, encoder layers, BLSTM
-        # layers) is stale now
-        _exec.invalidate_caches(self.model)
-        return loss
+        tape, self._tape = self._tape, None
+        tape.backward()
