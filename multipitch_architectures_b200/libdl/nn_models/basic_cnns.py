@@ -56,12 +56,12 @@ def _dispatch(model, x):
     """Autograd recording -> the training tape; train mode under no_grad -> the training forward with its tape discarded (dropout stays
     active exactly as in the reference, whose validation pass runs in train mode: exp126a...py:333-345); eval -> inference path."""
     if torch.is_grad_enabled() and (model.training or x.requires_grad):
-        from ...training import cnn_forward_train
-        return cnn_forward_train(model, x)
+        from ...training import cnn_train_forward, forward_train
+        return forward_train(cnn_train_forward, model, x)
     if model.training and model.p_dropout > 0:
         from ...training import cnn_train_forward
         model._train_calls = getattr(model, '_train_calls', 0) + 1
-        return cnn_train_forward(model, x, getattr(model, 'dropout_seed', 0x5EED), model._train_calls)[0]
+        return cnn_train_forward(model, x, {}, getattr(model, 'dropout_seed', 0x5EED), model._train_calls)[0].d
     return _exec.cnn_forward(model, x)
 
 

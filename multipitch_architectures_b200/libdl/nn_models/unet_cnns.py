@@ -221,9 +221,10 @@ class _UnetBase(_MpaModel):
             raise ValueError('U-Net models need at least 75 frames of context')
         if self.training:
             # train mode (BatchNorm batch statistics, dropout): the tape-driven training path, with or without autograd recording
-            from ...training_unet import unet_forward_train, unet_train_forward
+            from ...training import forward_train
+            from ...training_unet import unet_train_forward
             if torch.is_grad_enabled():
-                out = unet_forward_train(self, x)
+                out = forward_train(unet_train_forward, self, x)
                 return out if isinstance(out, tuple) else (out, None)
             self._train_calls = getattr(self, '_train_calls', 0) + 1
             y, n_pred, _ = unet_train_forward(self, x, {}, getattr(self, 'dropout_seed', 0x5EED), self._train_calls)

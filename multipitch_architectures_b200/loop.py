@@ -94,8 +94,8 @@ def _train_mode_loss(model, step, x, t):
         if isinstance(model, (basic_cnn_segm_sigmoid, deep_cnn_segm_sigmoid)):
             from .training import cnn_train_forward
             step.val_calls = getattr(step, 'val_calls', 0) + 1
-            y, _ = cnn_train_forward(model, x, step.seed ^ 0x5A5A, step.val_calls)
-            return ops.bce_fwd_bwd(y, t.contiguous())[0]
+            y = cnn_train_forward(model, x, {}, step.seed ^ 0x5A5A, step.val_calls)[0]
+            return ops.bce_fwd_bwd(y.d, t.contiguous())[0]
         out = model(x)
         y, n_pred = out if isinstance(out, tuple) else (out, None)
         t = t.contiguous()

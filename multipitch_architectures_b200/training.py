@@ -1,12 +1,13 @@
-"""Training path of the CNN family (basic_cnn_segm_sigmoid / deep_cnn_segm_sigmoid): forward with saved activations,
-hand-written backward, fused BCE and AdamW — all libmpa kernels (fp32).
+"""Training path of the CNN family (basic_cnn_segm_sigmoid / deep_cnn_segm_sigmoid), and what it shares with the U-Net family
+(training_unet.py): the reverse-mode `Tape` on which every stage of a train-mode forward records its own backward, the stages both
+families use, the autograd bridge and the fused step — all libmpa kernels (fp32).
 
 Reference loop being replaced (experiments/Exp1_SectionIV-B/exp126a_musicnet_cnn_basic.py:315-329):
     y_pred = model(X); loss = BCELoss(y_pred, y); optimizer.zero_grad(); loss.backward(); optimizer.step()
 
 Two ways in:
   * drop-in: `model.train(); y = model(x); loss = torch.nn.BCELoss()(y, t); loss.backward(); torch.optim.AdamW(...).step()`
-    — `model.forward` routes through `CnnTrainFunction` (a torch.autograd.Function whose backward is the code below);
+    — `model.forward` routes through `TrainFunction` (a torch.autograd.Function whose backward runs the tape);
   * fused: `TrainStep(model, lr=...)(x, t)` — BCE forward/backward kernel, backward, (optional) gradient all-reduce over
     NCCL on ONE flat buffer, fused AdamW; no torch operator touches an activation or a gradient.
 With `precision='bf16'` the convolutions run on the tensor cores (TcConv) and, for the models without the residual path, activations and
@@ -160,14 +161,11 @@ def _wgrad(conv, x, g, gw, gb):
          conv.padding[1], stream_ptr())
 
 
-ROWS_TC = True             # test knob: False = conv3 of the bf16 models on the fp32 strided-GEMM kernels (conv_rows.cu)
-
-
 def _rows_tc_eligible(model, conv, x):
     """The head's full-height 75x1 convolution of a bf16 model with more than 10 output channels: forward and both gradients as tcgen05
     GEMMs.  Thinner ones (CNN:XS 20 -> 10, DRCNN 30 -> 10) are HBM-bound matrix-vector products and stay on the conv_rows_thin_* kernels (the
     tensor-core form was measured at batch 256: 3.39 -> 3.48 ms per CNN:XS step — two operand-chunking passes over x outweigh the GEMMs)."""
-    return (ROWS_TC and model is not None and getattr(model, 'precision', 'fp32') == 'bf16' and _is_rows_conv(conv, x.shape[2])
+    return (getattr(model, 'precision', 'fp32') == 'bf16' and _is_rows_conv(conv, x.shape[2])
             and conv.weight.shape[0] > 10 and x.shape[3] % 8 == 0 and conv.bias is not None)
 
 
@@ -464,7 +462,9 @@ def _tc_s3_backward_split(tag, conv, xs, g, gw, gb):
 
 
 CP8_RESIDENT = True          # test knob: False = every block crosses nchw<->CP8 converters and pools in fp32 NCHW (identical results)
-LN_PIXEL = True          # LayerNorm -> CP8 and its parameter gradient on the pixel-per-thread kernels (False: row kernels)
+# LayerNorm -> CP8 and its parameter gradient on the pixel-per-thread kernels, which save (mean, rstd) of every row for the parameter gradient.
+# Test knob: False = the row kernels, whose fp32 sums run in the order of the fp32 NCHW path (bit-for-bit tape comparisons in the tests).
+LN_PIXEL = True
 
 
 def _cp8_resident(model, blocks, F):
@@ -474,183 +474,253 @@ def _cp8_resident(model, blocks, F):
             and _tc_s3_eligible(model, model.conv2[0], F))
 
 
-def _cnn_train_forward_cp8(model, blocks, x, sv, site, drop):
-    a, p, seed = model.a_lrelu, sv['p'], sv['seed']
-    fmt = ops.FMT_BF16
-    B, C0, T, F = x.shape
-    z = x           # (device of the buffers below)
-    ln = model.layernorm
-    # LayerNorm writes the first convolution's input planes directly (no fp32 copy of the normalised patch, no converter pass)
-    # pixel-per-thread LayerNorm kernels (train_cp8.cu): (mean, rstd) of every row saved for the parameter gradient.  LN_PIXEL = False keeps
-    # the row kernels, whose fp32 sums run in the order of the fp32 NCHW path (bit-for-bit tape comparisons in the tests)
-    sv['ln_stats'] = torch.empty(B * T, 2, dtype=torch.float32, device=x.device) if (F <= 256 and LN_PIXEL) else None
-    xc = ops.layernorm_cf_cp8(x, ln.weight, ln.bias, ln.eps, TcConv._buf(blocks[0][0] + ':x', B, C0, T, F, x.device, fmt), stats=sv['ln_stats'],
-                              pixel=LN_PIXEL)
-    sd, sm = _step_args()
-    split = 3 if _s3_split_eligible(model, model.conv2[0], F) else 0
-    for bi, (name, conv) in enumerate(blocks):
+class Node:
+    """An activation and its (lazily accumulated) gradient."""
+    __slots__ = ('d', 'g')
+
+    def __init__(self, d):
+        self.d, self.g = d, None
+
+    def acc(self, g):
+        self.g = g if self.g is None else _add(self.g, g)
+
+
+class Tape:
+    """Reverse-mode tape of a train-mode forward: each stage computes its output Node and records the closure of its own backward, which
+    reads the output's gradient and accumulates its input's.  A dropout stage takes its Philox offset (step * sites_per_step + site, sites
+    counted in forward order) once, in the forward, and its backward reuses it."""
+
+    def __init__(self, grads, seed, step, sites_per_step, model):
+        self.ops, self.grads, self.seed, self.site, self.model = [], grads, seed, step * sites_per_step, model
+        self.trunk_mark = 0
+
+    def push(self, fn):
+        self.ops.append(fn)
+
+    def backward(self, lo=0, hi=None):
+        """Run the recorded stages ops[lo:hi] in reverse (default: all).  `trunk_mark` = number of stages of the encoder trunk: running
+        [trunk_mark, end) first and [0, trunk_mark) second splits the backward where the gradients of everything but the trunk are final."""
+        hi = len(self.ops) if hi is None else hi
+        for fn in reversed(self.ops[lo:hi]):
+            fn()
+        del self.ops[lo:hi]
+
+    def _take_site(self):
+        self.site += 1
+        return self.site
+
+    # ---------------------------------------------------------------------------------------------- stages
+    def dropout(self, x, p):
+        if p <= 0.0:
+            return x
+        off = self._take_site()
+        out = Node(_dropout(x.d, p, self.seed, off))
+        self.push(lambda: x.acc(_dropout(out.g, p, self.seed, off)))
+        return out
+
+    def conv(self, name, conv, x, act=ops.ACT_NONE, a=0.0, need_dx=True, rows_tc=True):
+        """Conv2d (+ bias, + fused pointwise activation); stride-1 'same' convolutions of a bf16 model run on the tensor cores, and so do
+        full-height ones with more than 10 output channels unless rows_tc is False (_rows_tc_eligible)."""
+        if TcConv.eligible(self.model, conv, x.d.shape[3]) and x.d.shape[2] >= 2:
+            y, xc = TcConv.forward(name, conv, x.d, act, a)
+            out = Node(y)
+
+            def bwd_tc():
+                g = out.g if act == ops.ACT_NONE else _act_bwd(out.d, out.g, act, a)
+                gx = TcConv.backward(name, conv, xc, g, self.grads[name + '.weight'], self.grads[name + '.bias'], need_dx)
+                if need_dx:
+                    x.acc(gx)
+            self.push(bwd_tc)
+            return out
+        if rows_tc and _rows_tc_eligible(self.model, conv, x.d):
+            out = Node(_rows_tc_forward(conv, x.d, act, a))
+
+            def bwd_rows():
+                g = out.g if act == ops.ACT_NONE else _act_bwd(out.d, out.g, act, a)
+                gx = _rows_tc_backward(conv, x.d, g, self.grads[name + '.weight'], self.grads[name + '.bias'], need_dx)
+                if need_dx:
+                    x.acc(gx)
+            self.push(bwd_rows)
+            return out
+        out = Node(_conv_fwd(conv, x.d, act, a))
+
+        def bwd():
+            g = out.g if act == ops.ACT_NONE else _act_bwd(out.d, out.g, act, a)
+            _wgrad(conv, x.d, g, self.grads[name + '.weight'], self.grads[name + '.bias'])
+            if need_dx:
+                x.acc(_dgrad(conv, g, x.d.shape))
+        self.push(bwd)
+        return out
+
+    def layernorm_cf(self, ln, x):
+        """LayerNorm([C,F]) on the network input: only the affine parameters receive gradients."""
+        out = Node(ops.layernorm_cf(x, ln.weight, ln.bias, ln.eps))
+
+        def bwd():
+            B, C, T, F = x.shape
+            call('layernorm_cf_param_grad_f32', x, out.g, self.grads['layernorm.weight'], self.grads['layernorm.bias'], B, C, T, F,
+                 float(ln.eps), 0.0, stream_ptr())
+        self.push(bwd)
+        return out
+
+    def layernorm_cf_cp8(self, ln, x, dst):
+        """LayerNorm([C,F]) on the network input, written straight into the first convolution's planes (no fp32 copy of the normalised
+        input, no converter pass); the parameter gradients read the planes the first convolution's data gradient wrote."""
+        B, _, T, F = x.shape
+        stats = torch.empty(B * T, 2, dtype=torch.float32, device=x.device) if (F <= 256 and LN_PIXEL) else None
+        out = Node(ops.layernorm_cf_cp8(x, ln.weight, ln.bias, ln.eps, dst, stats=stats, pixel=LN_PIXEL))
+        self.push(lambda: ops.layernorm_cf_param_grad_cp8(x, out.g, self.grads['layernorm.weight'], self.grads['layernorm.bias'], ln.eps, stats=stats))
+        return out
+
+    # The fused pool + dropout stages below take their dropout site whatever p is: the CP8 kernels receive the offset even when p = 0.
+    def block(self, name, conv, x, p, a, residual):
+        """CNN block on fp32 NCHW: Conv2d (tensor cores behind the nchw<->CP8 converters when TcConv is eligible) -> LeakyReLU ->
+        MaxPool((3,1)) -> dropout (+ x when `residual`)."""
+        if TcConv.eligible(self.model, conv, x.d.shape[3]):
+            act, xc = TcConv.forward(name, conv, x.d, ops.ACT_LRELU, a)
+        else:
+            act, xc = _conv_fwd(conv, x.d, ops.ACT_LRELU, a), None
+        off = self._take_site()
+        out = Node(_pool_dropout(act, 3, x.d if residual else None, p, self.seed, off))
+
+        def bwd():
+            g = _pool_bwd_dropout(act, out.g, 3, ops.ACT_LRELU, a, p, self.seed, off)
+            gw, gb = self.grads[name + '.weight'], self.grads[name + '.bias']
+            if xc is not None:
+                x.acc(TcConv.backward(name, conv, xc, g, gw, gb, need_dx=True))
+            else:
+                _wgrad(conv, x.d, g, gw, gb)
+                x.acc(_dgrad(conv, g, x.d.shape))
+            if residual:
+                x.acc(out.g)
+        self.push(bwd)
+        return out
+
+    def block_cp8(self, name, conv, x, p, a, split=0):
+        """CNN block on the CP8 planes (_cp8_resident): Conv2d + LeakyReLU on the tensor cores -> MaxPool((3,1)) + dropout into the next
+        convolution's planes (split = 3: phase-split planes, the hand-over to the head's conv2, whose data gradient comes back in them); the
+        bias gradient is summed from the planes."""
+        xc = x.d
         yc = TcConv.forward_cp8(name, conv, xc, ops.ACT_LRELU, a)
-        site[0] += 1
-        sp = split if bi == len(blocks) - 1 else 0          # the last block hands over to conv2 in phase-split planes
-        zc = _split_buf(name + ':zs', B, (yc.C + 7) // 8 * 8, T, F, sp, z.device, fmt) if sp else TcConv._buf(name + ':z', B, yc.C, T, F, z.device, fmt)
-        call('pool3_dropout_split_cp8', yc.ptr(), zc.ptr(), B, yc.C, T, F, yc.pitch, yc.pf, yc.pt, fmt, float(p), ctypes_u64(seed),
-             ctypes_u64(site[0]), sd, sm, sp, zc.pitch if sp else 0, stream_ptr())
-        sv['blocks'].append((None, yc, xc))
-        xc = zc
-    sv['split'] = split
-    if split:
-        a2, x2c = _tc_s3_forward_split('conv2', model.conv2[0], xc, ops.ACT_LRELU, a)
-    else:
-        a2, x2c = _tc_s3_forward('conv2', model.conv2[0], xc, ops.ACT_LRELU, a)
-    site[0] += 1
-    d2 = _pool_dropout(a2, 13, None, p, seed, site[0])
-    a3 = _rows_tc_forward(model.conv3[0], d2, ops.ACT_LRELU, a) if _rows_tc_eligible(model, model.conv3[0], d2) else \
-        _conv_fwd(model.conv3[0], d2, ops.ACT_LRELU, a)
-    d3 = drop(a3)
-    a4 = _conv_fwd(model.conv4[0], d3, ops.ACT_LRELU, a)
-    d4 = drop(a4)
-    y = _conv_fwd(model.conv4[3], d4, ops.ACT_SIGMOID, 0.0)
-    sv.update(z_head=None, a2=a2, d2=d2, a3=a3, d3=d3, a4=a4, d4=d4, y=y, x2c=x2c, cp8=True)
-    return y, sv
-
-
-def cnn_train_forward(model, x, seed=0, step=0):
-    """-> (y_pred [B,1,T-74,72], saved).  Train mode: dropout active when model.p_dropout > 0."""
-    a, p = model.a_lrelu, (model.p_dropout if model.training else 0.0)
-    blocks = _exec.cnn_blocks(model)
-    residual = getattr(model, 'residual', False)
-    site = [step * SITES_PER_STEP]
-
-    def drop(t):
-        site[0] += 1
-        return _dropout(t, p, seed, site[0])
-    sv = {'x': x, 'blocks': [], 'p': p, 'seed': seed, 'site0': step * SITES_PER_STEP}
-    if _cp8_resident(model, blocks, x.shape[3]) and x.shape[1] <= 8:
-        return _cnn_train_forward_cp8(model, blocks, x, sv, site, drop)
-    z = ops.layernorm_cf(x, model.layernorm.weight, model.layernorm.bias, model.layernorm.eps)
-    for i, (name, conv) in enumerate(blocks):
-        if TcConv.eligible(model, conv, z.shape[3]):
-            act, xc = TcConv.forward(name, conv, z, ops.ACT_LRELU, a)
-        else:
-            act, xc = _conv_fwd(conv, z, ops.ACT_LRELU, a), None
-        site[0] += 1
-        sv['blocks'].append((z, act, xc))
-        z = _pool_dropout(act, 3, z if (residual and i > 0) else None, p, seed, site[0])
-    if _tc_s3_eligible(model, model.conv2[0], z.shape[3]):
-        a2, x2c = _tc_s3_forward('conv2', model.conv2[0], z, ops.ACT_LRELU, a)
-    else:
-        a2, x2c = _conv_fwd(model.conv2[0], z, ops.ACT_LRELU, a), None
-    site[0] += 1
-    d2 = _pool_dropout(a2, 13, None, p, seed, site[0])
-    a3 = _rows_tc_forward(model.conv3[0], d2, ops.ACT_LRELU, a) if _rows_tc_eligible(model, model.conv3[0], d2) else \
-        _conv_fwd(model.conv3[0], d2, ops.ACT_LRELU, a)
-    d3 = drop(a3)
-    a4 = _conv_fwd(model.conv4[0], d3, ops.ACT_LRELU, a)
-    d4 = drop(a4)
-    y = _conv_fwd(model.conv4[3], d4, ops.ACT_SIGMOID, 0.0)
-    sv.update(z_head=z, a2=a2, d2=d2, a3=a3, d3=d3, a4=a4, d4=d4, y=y, x2c=x2c)
-    return y, sv
-
-
-def cnn_train_backward(model, sv, g_y, grads):
-    """grads: dict parameter-name -> preallocated fp32 tensor (overwritten)."""
-    a, p, seed = model.a_lrelu, sv['p'], sv['seed']
-    blocks = _exec.cnn_blocks(model)
-    residual = getattr(model, 'residual', False)
-    n_sites = len(blocks) + 3
-    site = [sv['site0'] + n_sites + 1]
-
-    def drop_bwd(g):
-        site[0] -= 1
-        return _dropout(g, p, seed, site[0])
-    c43, c40, c3, c2 = model.conv4[3], model.conv4[0], model.conv3[0], model.conv2[0]
-    g = _act_bwd(sv['y'], g_y.contiguous(), ops.ACT_SIGMOID)
-    _wgrad(c43, sv['d4'], g, grads['conv4.3.weight'], grads['conv4.3.bias'])
-    g = drop_bwd(_dgrad(c43, g, sv['d4'].shape))
-    g = _act_bwd(sv['a4'], g, ops.ACT_LRELU, a)
-    _wgrad(c40, sv['d3'], g, grads['conv4.0.weight'], grads['conv4.0.bias'])
-    g = drop_bwd(_dgrad(c40, g, sv['d3'].shape))
-    g = _act_bwd(sv['a3'], g, ops.ACT_LRELU, a)
-    if _rows_tc_eligible(model, c3, sv['d2']):
-        g_d2 = _rows_tc_backward(c3, sv['d2'], g, grads['conv3.0.weight'], grads['conv3.0.bias'], True)
-    else:
-        _wgrad(c3, sv['d2'], g, grads['conv3.0.weight'], grads['conv3.0.bias'])
-        g_d2 = _dgrad(c3, g, sv['d2'].shape)
-    site[0] -= 1
-    g = _pool_bwd_dropout(sv['a2'], g_d2, 13, ops.ACT_LRELU, a, p, seed, site[0])
-    if sv.get('cp8'):
-        fmt = ops.FMT_BF16
-        split = sv.get('split', 0)
-        if split:
-            gzc = _tc_s3_backward_split('conv2', c2, sv['x2c'], g, grads['conv2.0.weight'], grads['conv2.0.bias'])
-        else:
-            gzc = _tc_s3_backward('conv2', c2, sv['x2c'], g, grads['conv2.0.weight'], grads['conv2.0.bias'], keep_cp8=True)
+        off = self._take_site()
+        B, C, T, F, fmt, dev = yc.B, yc.C, yc.T, yc.F, yc.fmt, yc.buf.device
+        zc = _split_buf(name + ':zs', B, (C + 7) // 8 * 8, T, F, split, dev, fmt) if split else TcConv._buf(name + ':z', B, C, T, F, dev, fmt)
         sd, sm = _step_args()
-        for i in range(len(blocks) - 1, -1, -1):
-            name, conv = blocks[i]
-            _, yc, xc = sv['blocks'][i]
-            site[0] -= 1
-            gc = TcConv._buf(name + ':g', yc.B, yc.C, yc.T, yc.F, yc.buf.device, fmt)
-            sp = split if i == len(blocks) - 1 else 0       # conv2's data gradient arrives in phase-split planes
-            call('pool3_bwd_dropout_split_cp8', yc.ptr(), gzc.ptr(), gc.ptr(), yc.B, yc.C, yc.T, yc.F, yc.pitch, yc.pf, yc.pt, fmt, ops.ACT_LRELU,
-                 float(a), float(p), ctypes_u64(seed), ctypes_u64(site[0]), sd, sm, sp, gzc.pitch if sp else 0, stream_ptr())
-            gzc = TcConv.backward_cp8(name, conv, xc, gc, grads[f'{name}.0.weight'], grads[f'{name}.0.bias'], need_dx=True)
-        ops.layernorm_cf_param_grad_cp8(sv['x'], gzc, grads['layernorm.weight'], grads['layernorm.bias'], model.layernorm.eps,
-                                        stats=sv.get('ln_stats'))
-        return grads
-    elif sv.get('x2c') is not None:
-        g_z = _tc_s3_backward('conv2', c2, sv['x2c'], g, grads['conv2.0.weight'], grads['conv2.0.bias'])
-    else:
-        _wgrad(c2, sv['z_head'], g, grads['conv2.0.weight'], grads['conv2.0.bias'])
-        g_z = _dgrad(c2, g, sv['z_head'].shape)
-    for i in range(len(blocks) - 1, -1, -1) if not sv.get('cp8') else ():
-        name, conv = blocks[i]
-        z_in, act, xc = sv['blocks'][i]
-        site[0] -= 1
-        g_conv = _pool_bwd_dropout(act, g_z, 3, ops.ACT_LRELU, a, p, seed, site[0])
-        if xc is not None:
-            g_in = TcConv.backward(name, conv, xc, g_conv, grads[f'{name}.0.weight'], grads[f'{name}.0.bias'], need_dx=True)
+        call('pool3_dropout_split_cp8', yc.ptr(), zc.ptr(), B, C, T, F, yc.pitch, yc.pf, yc.pt, fmt, float(p), ctypes_u64(self.seed),
+             ctypes_u64(off), sd, sm, split, zc.pitch if split else 0, stream_ptr())
+        out = Node(zc)
+
+        def bwd():
+            gz, gc = out.g, TcConv._buf(name + ':g', B, C, T, F, dev, fmt)
+            sd, sm = _step_args()
+            call('pool3_bwd_dropout_split_cp8', yc.ptr(), gz.ptr(), gc.ptr(), B, C, T, F, yc.pitch, yc.pf, yc.pt, fmt, ops.ACT_LRELU, float(a),
+                 float(p), ctypes_u64(self.seed), ctypes_u64(off), sd, sm, split, gz.pitch if split else 0, stream_ptr())
+            x.acc(TcConv.backward_cp8(name, conv, xc, gc, self.grads[name + '.weight'], self.grads[name + '.bias'], need_dx=True))
+        self.push(bwd)
+        return out
+
+    def conv2_pool(self, name, conv, x, p, a, split=0):
+        """Head conv2 (3x3, stride (1,3); basic_cnns.py:36) -> LeakyReLU -> MaxPool((13,1)) -> dropout, in fp32 NCHW (72 bins).  x: fp32
+        NCHW, or the CP8 planes of a CP8-resident producer (split = 3: phase-split planes, conv2 in its stride-1 3x1 form), which receives
+        its gradient in the same form."""
+        planes = isinstance(x.d, ops.CP8)
+        if split:
+            y, xc = _tc_s3_forward_split(name, conv, x.d, ops.ACT_LRELU, a)
+        elif planes or _tc_s3_eligible(self.model, conv, x.d.shape[3]):
+            y, xc = _tc_s3_forward(name, conv, x.d, ops.ACT_LRELU, a)
         else:
-            _wgrad(conv, z_in, g_conv, grads[f'{name}.0.weight'], grads[f'{name}.0.bias'])
-            g_in = _dgrad(conv, g_conv, z_in.shape)
-        g_z = _add(g_in, g_z) if (residual and i > 0) else g_in
-    x = sv['x']
+            y, xc = _conv_fwd(conv, x.d, ops.ACT_LRELU, a), None
+        off = self._take_site()
+        out = Node(_pool_dropout(y, 13, None, p, self.seed, off))
+
+        def bwd():
+            g = _pool_bwd_dropout(y, out.g, 13, ops.ACT_LRELU, a, p, self.seed, off)
+            gw, gb = self.grads[name + '.weight'], self.grads[name + '.bias']
+            if split:
+                gx = _tc_s3_backward_split(name, conv, xc, g, gw, gb)
+            elif xc is not None:
+                gx = _tc_s3_backward(name, conv, xc, g, gw, gb, keep_cp8=planes)
+            else:
+                _wgrad(conv, x.d, g, gw, gb)
+                gx = _dgrad(conv, g, x.d.shape)
+            x.acc(gx)
+        self.push(bwd)
+        return out
+
+    def head(self, x, p, split=0, conv4_rows_tc=True):
+        """The 72-bin head of both families (basic_cnns.py:34-40): conv2 stage -> conv3 (75x1) -> conv4 (1x1, then 1xK + sigmoid).
+        conv4_rows_tc: conv4.0 (a one-row 1x1 convolution after conv3) may take the tensor-core GEMMs of conv3; False keeps it on the
+        fp32 conv_rows kernels."""
+        m, a = self.model, self.model.a_lrelu
+        h = self.conv2_pool('conv2.0', m.conv2[0], x, p, a, split)
+        h = self.dropout(self.conv('conv3.0', m.conv3[0], h, ops.ACT_LRELU, a), p)
+        h = self.dropout(self.conv('conv4.0', m.conv4[0], h, ops.ACT_LRELU, a, rows_tc=conv4_rows_tc), p)
+        return self.conv('conv4.3', m.conv4[3], h, ops.ACT_SIGMOID)
+
+
+def cnn_train_forward(model, x, grads, seed=0, step=0):
+    """-> (y_pred Node [B,1,T-74,72], None, tape).  Train mode: dropout active when model.p_dropout > 0.  bf16 models without the residual
+    path keep the block activations and gradients on the CP8 planes (_cp8_resident)."""
+    a, p = model.a_lrelu, (model.p_dropout if model.training else 0.0)
+    tp = Tape(grads, seed, step, SITES_PER_STEP, model)
+    blocks = _exec.cnn_blocks(model)
     B, C, T, F = x.shape
-    call('layernorm_cf_param_grad_f32', x, g_z, grads['layernorm.weight'], grads['layernorm.bias'], B, C, T, F,
-         float(model.layernorm.eps), 0.0, stream_ptr())
-    return grads
+    split = 0
+    if _cp8_resident(model, blocks, F) and C <= 8:
+        z = tp.layernorm_cf_cp8(model.layernorm, x, TcConv._buf(blocks[0][0] + '.0:x', B, C, T, F, x.device, ops.FMT_BF16))
+        split = 3 if _s3_split_eligible(model, model.conv2[0], F) else 0
+        for i, (name, conv) in enumerate(blocks):
+            z = tp.block_cp8(name + '.0', conv, z, p, a, split if i == len(blocks) - 1 else 0)
+    else:
+        z = tp.layernorm_cf(model.layernorm, x)
+        residual = getattr(model, 'residual', False)
+        for i, (name, conv) in enumerate(blocks):
+            z = tp.block(name + '.0', conv, z, p, a, residual and i > 0)
+    # conv4.0 of the CNN family runs on the fp32 conv_rows kernels whatever its width (its tensor-core form is not measured for this family)
+    return tp.head(z, p, split, conv4_rows_tc=False), None, tp
 
 
-class CnnTrainFunction(torch.autograd.Function):
+class TrainFunction(torch.autograd.Function):
+    """Drop-in autograd bridge: `model.train(); y = model(x); loss.backward()` runs the tape that `build` (cnn_train_forward,
+    training_unet.unet_train_forward) recorded."""
+
     @staticmethod
-    def forward(ctx, model, x, seed, step, *params):
-        with torch.no_grad():
-            y, sv = cnn_train_forward(model, x, seed, step)
-        ctx.model, ctx.sv = model, sv
-        return y
-
-    @staticmethod
-    def backward(ctx, g_y):
-        model = ctx.model
+    def forward(ctx, build, model, x, seed, step, *params):
         named = list(model.named_parameters())
         with torch.no_grad():
-            grads = {n: torch.empty_like(p) for n, p in named}
-            cnn_train_backward(model, ctx.sv, g_y, grads)
-        return (None, None, None, None) + tuple(grads[n] for n, _ in named)
+            grads = {n: torch.zeros_like(p) for n, p in named}
+            y, n_pred, tape = build(model, x, grads, seed, step)
+        ctx.model, ctx.tape, ctx.grads, ctx.nodes = model, tape, grads, (y, n_pred)
+        if n_pred is None:
+            return y.d
+        return y.d, n_pred.d
+
+    @staticmethod
+    def backward(ctx, g_y, g_n=None):
+        y, n_pred = ctx.nodes
+        with torch.no_grad():
+            y.g = g_y.contiguous()
+            if n_pred is not None:
+                n_pred.g = g_n.contiguous() if g_n is not None else torch.zeros_like(n_pred.d)
+            ctx.tape.backward()
+        named = list(ctx.model.named_parameters())
+        return (None, None, None, None, None) + tuple(ctx.grads[n] for n, _ in named)
 
 
-def cnn_forward_train(model, x):
+def forward_train(build, model, x):
     """Entry used by model.forward when autograd is recording."""
     model._train_calls = getattr(model, '_train_calls', 0) + 1
     seed = getattr(model, 'dropout_seed', 0x5EED)
-    return CnnTrainFunction.apply(model, x, seed, model._train_calls, *[p for _, p in model.named_parameters()])
+    return TrainFunction.apply(build, model, x, seed, model._train_calls, *[p for _, p in model.named_parameters()])
 
 
 class FusedTrainStep:
-    """Fused training step on flat parameter / gradient / moment buffers: the subclass's forward, loss and backward, ONE gradient all-reduce
-    (NCCL, when a process group is active), fused AdamW.  A subclass supplies `_forward_backward` and `sites_per_step`; one whose parameters
-    start with an encoder trunk sets `n_trunk` and supplies `_trunk_backward` (UnetTrainStep)."""
+    """Fused training step on flat parameter / gradient / moment buffers: the forward the subclass's builder records on a Tape, BCE (+ CE
+    when the builder returns a count prediction: UnetTrainStep's `ce_scale`), the tape's backward, ONE gradient all-reduce (NCCL, when a
+    process group is active), fused AdamW.  A subclass supplies `sites_per_step` and `build`; one whose parameters start with an encoder
+    trunk sets `n_trunk` (UnetTrainStep)."""
     sites_per_step = None
+    build = None          # (model, x, grads, seed, step) -> (y Node, n_pred Node or None, Tape)
 
     def __init__(self, model, lr=1e-3, betas=(0.9, 0.999), eps=1e-8, weight_decay=0.01, seed=0x5EED, process_group=None, graph=False):
         """graph=True: after two eager steps forward + loss + backward are captured ONCE into a CUDA graph and replayed (fixed input shape;
@@ -678,10 +748,27 @@ class FusedTrainStep:
         self.n_trunk, self.overlap_comm = 0, False     # no trunk split: one flat all-reduce after the backward
         self.comm_events = None                        # bench.py: a list that receives CUDA events around the all-reduce
         self._state = StepState(dev, self.sites_per_step)
+        self._tape = None
 
     def _forward_backward(self, x, target, tape_step, split):
         """-> loss (the step state is active).  split: stop the backward at the trunk (its part follows in _trunk_backward)."""
-        raise NotImplementedError
+        y, n_pred, tape = self.build(self.model, x, self.grads, self.seed, tape_step)
+        target = target.contiguous()
+        loss, y.g = ops.bce_fwd_bwd(y.d, target)
+        if n_pred is not None:
+            B, K = n_pred.d.shape[0], n_pred.d.shape[1]
+            n_pred.g = torch.empty_like(n_pred.d)
+            call('ce_count_fwd_bwd_f32', n_pred.d, target, loss, n_pred.g, B, K, target.numel() // B, float(self.ce_scale), 1, stream_ptr())
+        if split:
+            tape.backward(lo=tape.trunk_mark)
+            self._tape = tape
+        else:
+            tape.backward()
+        return loss
+
+    def _trunk_backward(self):
+        tape, self._tape = self._tape, None
+        tape.backward()
 
     def release(self):
         """Free the pooled activation planes and the pack plan of this step, and the captured graphs that point into them (dropping the
@@ -760,11 +847,6 @@ class FusedTrainStep:
 
 class TrainStep(FusedTrainStep):
     """Fused training step of the CNN family.  Its backward is one piece: n_trunk stays 0 (its parameter names begin with `layernorm.`
-    like a U-Net trunk's, but the CNN tape cannot stop half-way)."""
+    like a U-Net trunk's, but its builder marks no trunk on the tape)."""
     sites_per_step = SITES_PER_STEP
-
-    def _forward_backward(self, x, target, tape_step, split):
-        y, sv = cnn_train_forward(self.model, x, self.seed, tape_step)
-        loss, g_y = ops.bce_fwd_bwd(y, target.contiguous())
-        cnn_train_backward(self.model, sv, g_y, self.grads)
-        return loss
+    build = staticmethod(cnn_train_forward)

@@ -1,6 +1,7 @@
 """Training path of the U-Net family (simple_u_net_largekernels / _doubleselfattn / _polyphony_classif_softmax):
 train-mode forward (BatchNorm batch statistics, dropout, batch-axis attention) with saved activations and the
-hand-written backward of every stage — all libmpa kernels (fp32), sequenced by a small reverse-mode tape.
+hand-written backward of every stage — all libmpa kernels (fp32), sequenced by the reverse-mode tape of training.py (UnetTape adds
+the stages only this family has).
 
 Reference loop being replaced (experiments/Exp2_SectionIV-C/RETRAIN4_exp180d_..._doubleselfattn_moresamples.py, same
 shape as exp126a...py:315-329; PUnet: RETRAIN4_exp195f..._rerun1.py:337-350):
@@ -19,102 +20,14 @@ import torch
 from . import _lib, ops
 from ._lib import call, stream_ptr
 from .libdl.nn_models import _exec
-from .training import (FusedTrainStep, TcConv, ctypes_u64, _s3_split_eligible, _split_buf, _step_args, _tc_s3_backward_split, _tc_s3_forward_split,
-                       _rows_tc_backward, _rows_tc_eligible, _rows_tc_forward, _act_bwd, _add, _conv_fwd, _dgrad, _dropout, _pool_bwd, _tc_s3_backward,
-                       _tc_s3_eligible, _tc_s3_forward, _wgrad)
+from .training import FusedTrainStep, Node, Tape, TcConv, ctypes_u64, _act_bwd, _add, _s3_split_eligible, _split_buf, _step_args, _tc_s3_eligible
 
 SITES_PER_STEP = 256      # dropout sites reserved per step of the U-Net tape: offset = step * 256 + site
 
 
-class Node:
-    """An activation and its (lazily accumulated) gradient."""
-    __slots__ = ('d', 'g')
-
-    def __init__(self, d):
-        self.d, self.g = d, None
-
-    def acc(self, g):
-        self.g = g if self.g is None else _add(self.g, g)
-
-
-class Tape:
-    def __init__(self, grads, seed, step, model=None):
-        self.ops, self.grads, self.seed, self.site, self.model = [], grads, seed, step * SITES_PER_STEP, model
-        self.trunk_mark = 0
-
-    def push(self, fn):
-        self.ops.append(fn)
-
-    def backward(self, lo=0, hi=None):
-        """Run the recorded stages ops[lo:hi] in reverse (default: all).  `trunk_mark` = number of stages of the encoder trunk: running
-        [trunk_mark, end) first and [0, trunk_mark) second splits the backward where the gradients of everything but the trunk are final."""
-        hi = len(self.ops) if hi is None else hi
-        for fn in reversed(self.ops[lo:hi]):
-            fn()
-        del self.ops[lo:hi]
-
-    # ---------------------------------------------------------------------------------------------- stages
-    def dropout(self, x, p):
-        if p <= 0.0:
-            return x
-        self.site += 1
-        off = self.site
-        out = Node(_dropout(x.d, p, self.seed, off))
-        self.push(lambda: x.acc(_dropout(out.g, p, self.seed, off)))
-        return out
-
-    def conv(self, name, conv, x, act=ops.ACT_NONE, a=0.0, need_dx=True):
-        """Conv2d (+ bias, + fused pointwise activation); stride-1 'same' convolutions of a bf16 model run on the tensor cores."""
-        if self.model is not None and TcConv.eligible(self.model, conv, x.d.shape[3]) and x.d.shape[2] >= 2:
-            y, xc = TcConv.forward(name, conv, x.d, act, a)
-            out = Node(y)
-
-            def bwd_tc():
-                g = out.g if act == ops.ACT_NONE else _act_bwd(out.d, out.g, act, a)
-                gx = TcConv.backward(name, conv, xc, g, self.grads[name + '.weight'], self.grads[name + '.bias'], need_dx)
-                if need_dx:
-                    x.acc(gx)
-            self.push(bwd_tc)
-            return out
-        if _rows_tc_eligible(self.model, conv, x.d):
-            out = Node(_rows_tc_forward(conv, x.d, act, a))
-
-            def bwd_rows():
-                g = out.g if act == ops.ACT_NONE else _act_bwd(out.d, out.g, act, a)
-                gx = _rows_tc_backward(conv, x.d, g, self.grads[name + '.weight'], self.grads[name + '.bias'], need_dx)
-                if need_dx:
-                    x.acc(gx)
-            self.push(bwd_rows)
-            return out
-        out = Node(_conv_fwd(conv, x.d, act, a))
-
-        def bwd():
-            g = out.g if act == ops.ACT_NONE else _act_bwd(out.d, out.g, act, a)
-            _wgrad(conv, x.d, g, self.grads[name + '.weight'], self.grads[name + '.bias'])
-            if need_dx:
-                x.acc(_dgrad(conv, g, x.d.shape))
-        self.push(bwd)
-        return out
-
-    def conv_act_pool_time(self, name, conv, x, k, a):
-        """Conv2d -> LeakyReLU -> MaxPool((k,1), stride 1, pad k//2)  (head conv2, basic_cnns.py:391-393)."""
-        xc = None
-        if self.model is not None and _tc_s3_eligible(self.model, conv, x.d.shape[3]):
-            y, xc = _tc_s3_forward(name, conv, x.d, ops.ACT_LRELU, a)
-            act = Node(y)
-        else:
-            act = Node(_conv_fwd(conv, x.d, ops.ACT_LRELU, a))
-        out = Node(ops.maxpool_time(act.d, k))
-
-        def bwd():
-            g = _pool_bwd(act.d, out.g, k, ops.ACT_LRELU, a)
-            if xc is not None:
-                x.acc(_tc_s3_backward(name, conv, xc, g, self.grads[name + '.weight'], self.grads[name + '.bias']))
-                return
-            _wgrad(conv, x.d, g, self.grads[name + '.weight'], self.grads[name + '.bias'])
-            x.acc(_dgrad(conv, g, x.d.shape))
-        self.push(bwd)
-        return out
+class UnetTape(Tape):
+    """The U-Net family's stages: BatchNorm, double_conv, max-pool / up-sampling / concat (fp32 NCHW and on the CP8 planes), the encoder
+    layer and the BLSTM."""
 
     def bn_relu(self, name, bn, y):
         """BatchNorm2d in training mode (batch statistics) + ReLU; running statistics updated as nn.BatchNorm2d does."""
@@ -164,26 +77,6 @@ class Tape:
             skip.acc(g_skip)
             low.acc(g_low)
         self.push(bwd)
-        return out
-
-    def layernorm_cf(self, ln, x):
-        """LayerNorm([C,F]) on the network input: only the affine parameters receive gradients."""
-        out = Node(ops.layernorm_cf(x, ln.weight, ln.bias, ln.eps))
-
-        def bwd():
-            B, C, T, F = x.shape
-            call('layernorm_cf_param_grad_f32', x, out.g, self.grads['layernorm.weight'], self.grads['layernorm.bias'], B, C, T, F,
-                 float(ln.eps), 0.0, stream_ptr())
-        self.push(bwd)
-        return out
-
-    def layernorm_cf_cp8(self, ln, x, dst):
-        """LayerNorm([C,F]) on the network input, written straight into the first convolution's planes; the parameter gradients read the
-        planes the first convolution's data gradient wrote."""
-        B, _, T, F = x.shape
-        stats = torch.empty(B * T, 2, dtype=torch.float32, device=x.device) if F <= 256 else None     # (mean, rstd) rows for the parameter gradient
-        out = Node(ops.layernorm_cf_cp8(x, ln.weight, ln.bias, ln.eps, dst, stats=stats))
-        self.push(lambda: ops.layernorm_cf_param_grad_cp8(x, out.g, self.grads['layernorm.weight'], self.grads['layernorm.bias'], ln.eps, stats=stats))
         return out
 
     # ---------------------------------------------------------------------------------------------- CP8-resident stages (bf16)
@@ -263,22 +156,6 @@ class Tape:
 
         def bwd():
             x.acc(ops.cp8_to_nchw(out.g))
-        self.push(bwd)
-        return out
-
-    def head_conv2_cp8(self, name, conv, u, k, a, split=0):
-        """Head conv2 (3x3, stride (1,3)) on the planes (split: phase-split input, stride-1 3x1 form) -> LeakyReLU -> MaxPool((k,1)) in fp32
-        NCHW (72 bins)."""
-        y, xc = (_tc_s3_forward_split if split else _tc_s3_forward)(name, conv, u.d, ops.ACT_LRELU, a)
-        act = Node(y)
-        out = Node(ops.maxpool_time(act.d, k))
-
-        def bwd():
-            g = _pool_bwd(act.d, out.g, k, ops.ACT_LRELU, a)
-            if split:
-                u.g = _tc_s3_backward_split(name, conv, xc, g, self.grads[name + '.weight'], self.grads[name + '.bias'])
-            else:
-                u.g = _tc_s3_backward(name, conv, xc, g, self.grads[name + '.weight'], self.grads[name + '.bias'], keep_cp8=True)
         self.push(bwd)
         return out
 
@@ -573,9 +450,9 @@ def cp8_tape_eligible(model, x):
 def _unet_train_forward_cp8(model, x, grads, seed, step):
     """The CP8-resident tape: LayerNorm -> planes -> [conv -> BN stats -> BN+ReLU]* with max-pool / up-sampling / concat on the planes ->
     (encoder layers in fp32 tokens) -> head conv2 on the planes -> fp32 72-bin head."""
-    a, p = model.a_lrelu, (model.p_dropout if model.training else 0.0)
+    p = model.p_dropout if model.training else 0.0
     fmt = ops.FMT_BF16
-    tp = Tape(grads, seed, step, model)
+    tp = UnetTape(grads, seed, step, SITES_PER_STEP, model)
     B, C, T, F = x.shape
     dev = x.device
     geo = _exec.level_geometry(T, F)
@@ -605,11 +482,7 @@ def _unet_train_forward_cp8(model, x, grads, seed, step):
         dst = _split_buf('upconv4:as', B, up_out[3], T, F, 3, dev, fmt) if last else None       # hand-over to conv2 in phase-split planes
         u = tp.double_conv_cp8(f'upconv{i + 1}', getattr(model, f'upconv{i + 1}'), tp.upcat_cp8(f'up{i + 1}', u, xs[lv], cat[lv], c[lv]), dst,
                                split=split if last else 0)
-    h = tp.dropout(tp.head_conv2_cp8('conv2.0', model.conv2[0], u, 13, a, split), p)
-    h = tp.dropout(tp.conv('conv3.0', model.conv3[0], h, ops.ACT_LRELU, a), p)
-    h = tp.dropout(tp.conv('conv4.0', model.conv4[0], h, ops.ACT_LRELU, a), p)
-    y = tp.conv('conv4.3', model.conv4[3], h, ops.ACT_SIGMOID)
-    return y, None, tp
+    return tp.head(u, p, split), None, tp
 
 
 def unet_train_forward(model, x, grads, seed=0, step=0):
@@ -617,7 +490,7 @@ def unet_train_forward(model, x, grads, seed=0, step=0):
     if cp8_tape_eligible(model, x):
         return _unet_train_forward_cp8(model, x, grads, seed, step)
     a, p = model.a_lrelu, (model.p_dropout if model.training else 0.0)
-    tp = Tape(grads, seed, step, model)
+    tp = UnetTape(grads, seed, step, SITES_PER_STEP, model)
     z = tp.layernorm_cf(model.layernorm, x)
     x1 = tp.double_conv('inc', model.inc, z)       # (the gradient wrt z feeds the LayerNorm parameter gradients)
     xs = [x1]
@@ -640,10 +513,7 @@ def unet_train_forward(model, x, grads, seed=0, step=0):
     u = x5
     for i, lv in enumerate((3, 2, 1, 0)):
         u = tp.double_conv(f'upconv{i + 1}', getattr(model, f'upconv{i + 1}'), tp.upconcat(u, xs[lv]))
-    h = tp.dropout(tp.conv_act_pool_time('conv2.0', model.conv2[0], u, 13, a), p)
-    h = tp.dropout(tp.conv('conv3.0', model.conv3[0], h, ops.ACT_LRELU, a), p)
-    h = tp.dropout(tp.conv('conv4.0', model.conv4[0], h, ops.ACT_LRELU, a), p)
-    y = tp.conv('conv4.3', model.conv4[3], h, ops.ACT_SIGMOID)
+    y = tp.head(u, p)
     n_pred = None
     if hasattr(model, 'convP'):
         q = tp.conv('convP.0', model.convP[0], x5, ops.ACT_LRELU, a)
@@ -652,42 +522,11 @@ def unet_train_forward(model, x, grads, seed=0, step=0):
     return y, n_pred, tp
 
 
-class UnetTrainFunction(torch.autograd.Function):
-    """Drop-in autograd bridge: `model.train(); y = model(x); loss.backward()` runs the tape above."""
-
-    @staticmethod
-    def forward(ctx, model, x, seed, step, *params):
-        named = list(model.named_parameters())
-        with torch.no_grad():
-            grads = {n: torch.zeros_like(p) for n, p in named}
-            y, n_pred, tape = unet_train_forward(model, x, grads, seed, step)
-        ctx.model, ctx.tape, ctx.grads, ctx.nodes = model, tape, grads, (y, n_pred)
-        if n_pred is None:
-            return y.d
-        return y.d, n_pred.d
-
-    @staticmethod
-    def backward(ctx, g_y, g_n=None):
-        y, n_pred = ctx.nodes
-        with torch.no_grad():
-            y.g = g_y.contiguous()
-            if n_pred is not None:
-                n_pred.g = g_n.contiguous() if g_n is not None else torch.zeros_like(n_pred.d)
-            ctx.tape.backward()
-        named = list(ctx.model.named_parameters())
-        return (None, None, None, None) + tuple(ctx.grads[n] for n, _ in named)
-
-
-def unet_forward_train(model, x):
-    model._train_calls = getattr(model, '_train_calls', 0) + 1
-    seed = getattr(model, 'dropout_seed', 0x5EED)
-    return UnetTrainFunction.apply(model, x, seed, model._train_calls, *[p for _, p in model.named_parameters()])
-
-
 class UnetTrainStep(FusedTrainStep):
     """Fused training step of a U-Net-family model (FusedTrainStep): forward, BCE (+ CE/25 for the PUnet), backward, ONE gradient
     all-reduce, fused AdamW.  graph=True replays ~3,500 kernel launches of the SAUnet:L (more host launch time than GPU time) from one graph."""
     sites_per_step = SITES_PER_STEP
+    build = staticmethod(unet_train_forward)
 
     def __init__(self, model, lr=1e-3, betas=(0.9, 0.999), eps=1e-8, weight_decay=0.01, seed=0x5EED, process_group=None, ce_scale=1.0 / 25.0,
                  graph=False, overlap_comm=True):
@@ -707,23 +546,3 @@ class UnetTrainStep(FusedTrainStep):
                 self.n_trunk += p.numel()
             else:
                 seen_other = True
-        self._tape = None
-
-    def _forward_backward(self, x, target, tape_step, split):
-        y, n_pred, tape = unet_train_forward(self.model, x, self.grads, self.seed, tape_step)
-        target = target.contiguous()
-        loss, y.g = ops.bce_fwd_bwd(y.d, target)
-        if n_pred is not None:
-            B, K = n_pred.d.shape[0], n_pred.d.shape[1]
-            n_pred.g = torch.empty_like(n_pred.d)
-            call('ce_count_fwd_bwd_f32', n_pred.d, target, loss, n_pred.g, B, K, target.numel() // B, float(self.ce_scale), 1, stream_ptr())
-        if split:
-            tape.backward(lo=tape.trunk_mark)
-            self._tape = tape
-        else:
-            tape.backward()
-        return loss
-
-    def _trunk_backward(self):
-        tape, self._tape = self._tape, None
-        tape.backward()

@@ -69,7 +69,7 @@ def test_model_loss_and_grads_match_reference_golden(nn_golden, name):
     m.p_dropout = 0.0
     m = m.cuda().train()
     x, t = synth_patches(B, seed).cuda(), synth_targets(B, seed).cuda()
-    y = m(x)                                                    # autograd path (CnnTrainFunction)
+    y = m(x)                                                    # autograd path (training.TrainFunction)
     loss = torch.nn.BCELoss(reduction='mean')(y, t)
     loss.backward()
     assert abs(loss.item() - float(nn_golden[tag + '__loss'][0])) < 1e-5
@@ -116,6 +116,32 @@ def test_fused_train_step_matches_torch_adamw_on_oracle():
         y = m(x.cuda()).cpu()
         yr = NO.cnn_forward({k: v.detach() for k, v in ref.items()}, x)
     assert (y - yr).abs().max() < 1e-3
+
+
+def test_wide_cnn_head_conv4_stays_on_the_fp32_row_kernels(monkeypatch):
+    """bf16 CNN whose conv3 and conv4.0 both have more than 10 output channels: conv3 takes the tensor-core GEMMs, conv4.0 (one-row 1x1
+    after conv3) the fp32 conv_rows kernels, in the fused step and in the autograd path."""
+    from multipitch_architectures_b200 import training as TR
+    from multipitch_architectures_b200.libdl import nn_models as M
+    calls = []
+
+    def spy(name):
+        orig = getattr(TR, name)
+
+        def fn(conv, *args):
+            calls.append((name, tuple(conv.weight.shape)))
+            return orig(conv, *args)
+        return fn
+    for name in ('_rows_tc_forward', '_rows_tc_backward'):
+        monkeypatch.setattr(TR, name, spy(name))
+    m = M.basic_cnn_segm_sigmoid(n_chan_input=6, n_chan_layers=[20, 20, 16, 16], n_bins_in=216, n_bins_out=72, precision='bf16')
+    m.load_state_dict(fill_state_dict(m.state_dict(), 3, scheme='torch_default'))
+    m = m.cuda().train()
+    x, t = synth_patches(3, 5).cuda(), synth_targets(3, 5).cuda()
+    torch.nn.BCELoss()(m(x), t).backward()
+    TR.TrainStep(m)(x, t)
+    conv3 = tuple(m.conv3[0].weight.shape)
+    assert calls == [('_rows_tc_forward', conv3), ('_rows_tc_backward', conv3)] * 2, calls
 
 
 def test_cnn_graph_replayed_step_equals_eager_step():

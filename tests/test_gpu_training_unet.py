@@ -136,7 +136,7 @@ def test_model_loss_grads_and_running_stats_match_reference_golden(train_golden,
     _zero_dropout(m)
     m = m.cuda().train()
     x, t = synth_patches(B, seed).cuda(), synth_targets(B, seed).cuda()
-    y = m(x)                                                    # autograd path (UnetTrainFunction)
+    y = m(x)                                                    # autograd path (training.TrainFunction)
     if isinstance(y, tuple):
         y, n_pred = y
         assert np.abs(n_pred.detach().cpu().numpy() - train_golden[tag + '__n']).max() < 1e-3
