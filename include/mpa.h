@@ -75,6 +75,17 @@ int mpa_layernorm_cf_cp8_stats(const float* x, const float* ln_w, const float* l
                                int pitch, int pf, int pt, float eps, float gamma_log, int fmt, void* stream);
 int mpa_layernorm_cf_param_grad_cp8_stats(const float* x, const void* g_cp8, const float* stats, float* g_w, float* g_b, int B, int C, int T,
                                           int F, int pitch, int pf, int pt, int fmt, float gamma_log, void* stream);
+/* LayerNorm([C,F]) backward to the INPUT with the parameter gradients of the same pass (saliency maps, adversarial checks, eval-mode
+ * backward): per (b,t) row dx = rstd * (gh - mean(gh) - xhat * mean(gh * xhat)), gh = g * ln_w, means over the C*F elements (times
+ * gamma_log / (1 + gamma_log * x) when the log compression is fused); g_w / g_b overwritten as by the parameter-only calls above, dx fp32
+ * NCHW [B,C,T,F] overwritten.  One thread per bin with all C <= 8 channels, F <= 256.
+ *   _cp8_stats  g in the CP8 planes (one chunk) and (mean, rstd) from the rows mpa_layernorm_cf_cp8_stats saved
+ *   _f32        g fp32 NCHW; the row statistics are re-reduced from x (the fp32 tape, or planes converted to NCHW) */
+int mpa_layernorm_cf_input_grad_cp8_stats(const float* x, const void* g_cp8, const float* stats, const float* ln_w, float* dx, float* g_w,
+                                          float* g_b, int B, int C, int T, int F, int pitch, int pf, int pt, int fmt, float gamma_log,
+                                          void* stream);
+int mpa_layernorm_cf_input_grad_f32(const float* x, const float* g_out, const float* ln_w, float* dx, float* g_w, float* g_b, int B, int C,
+                                    int T, int F, float eps, float gamma_log, void* stream);
 
 /* Frame-major variant used by the streaming inference engine: frames [C][N][F] (the HCQT layout) ->
  * normalised frames; rows s with s < lead or s >= lead+N are the patch zero padding and come out as ln_b
@@ -460,6 +471,13 @@ int mpa_maxpool2x2_bwd_cp8(const void* a_cp8, const void* g_pool_cp8, const void
                            int fmt, void* stream);
 int mpa_upsample2x_bwd_cp8(const void* g_up_cp8, void* g_low_cp8, int B, int C, int Tl, int Fl, int pitch_l, int pf_l, int pt_l,
                            int ncs_low, int Ts, int Fs, int pitch_s, int pf_s, int pt_s, int ncs_up, int fmt, void* stream);
+/* Eval-mode backward of BatchNorm2d -> ReLU on the planes (BatchNorm frozen: `stats` = [running_mean | running_var], the format
+ * mpa_bn_relu_apply_cp8 reads; nothing is updated): g' = g * [out > 0] (out recomputed from y), dy = weight * rstd * g' written as CP8,
+ * g_weight = sum g' * xhat, g_bias = sum g', g_conv_bias (optional) = sum dy — the convolution's bias gradient, NOT zero here.  One launch
+ * on the (chunk, slice) grid of mpa_bn_relu_bwd_cp8 with the same ordered merge (bit-reproducible); g_split / g_pitch as there. */
+int mpa_bn_relu_bwd_frozen_cp8(const void* g_cp8, const void* y_cp8, void* dy_cp8, const float* stats, const float* weight, const float* bias,
+                               float eps, float* g_weight, float* g_bias, float* g_conv_bias, int B, int C, int T, int F, int pitch, int pf,
+                               int pt, int ncs_g, int ncs_y, int ncs_dy, int g_split, int g_pitch, int fmt, void* stream);
 /* Training path of the attention half of transformer_enc_layer (libdl/nn_models/unet_cnns.py:131-153: q/k/v Linear -> nn.MultiheadAttention over
  * the BATCH axis -> o Linear -> Dropout -> add -> LayerNorm1), fp32, one CTA per bottleneck position (enc_train.cu).
  *   mpa_enc_fold_f32        w_qkv [3E,E] (+ transpose w_qkvT [E,3E]) = in_proj_weight_z . {q,k,v}_linear.weight, w_proj [E,E] (+ w_projT) =
@@ -576,6 +594,10 @@ int mpa_channel_sum_f32(const float* x, float* out, int B, int C, int HW, void* 
  * stats = [mean | biased var] from mpa_bn_stats_f32; scratch2c: 2*C floats. */
 int mpa_bn_relu_bwd_f32(const float* x, const float* out, const float* dy, const float* stats, const float* w, float* dx,
                         float* dw, float* db, float* scratch2c, int B, int C, int HW, float eps, int relu, void* stream);
+/* The same with BatchNorm2d frozen (eval mode): stats = [running_mean | running_var]; dx = w * rstd * dy' (dy' = dy * [out > 0] when
+ * relu), dw = sum dy' * xhat, db = sum dy'; d_conv_bias (optional) = sum dx, the preceding convolution's bias gradient. */
+int mpa_bn_relu_bwd_frozen_f32(const float* x, const float* out, const float* dy, const float* stats, const float* w, float* dx, float* dw,
+                               float* db, float* d_conv_bias, float* scratch2c, int B, int C, int HW, float eps, int relu, void* stream);
 /* MaxPool2d((kh,kw), stride (sh,sw)) backward, floor mode, gradient to the first maximum of each window. */
 int mpa_maxpool2d_bwd_f32(const float* x, const float* g_out, float* g_in, int B, int C, int H, int W, int kh, int kw,
                           int sh, int sw, void* stream);

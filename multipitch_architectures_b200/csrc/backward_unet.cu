@@ -62,6 +62,18 @@ __global__ void bn_relu_bwd_apply_vec4_kernel(const float4* __restrict__ x, cons
   }
 }
 
+// ---- BatchNorm2d(eval: running statistics) + ReLU backward: dx = w * rstd * dy' (nothing depends on the batch) ------------------
+__global__ void bn_relu_bwd_frozen_apply_kernel(const float* __restrict__ out, const float* __restrict__ dy, const float* __restrict__ stats,
+                                                const float* __restrict__ w, float eps, float* __restrict__ dx, long long total, int C, int HW,
+                                                int relu) {
+  for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
+    const int c = (int)((i / HW) % C);
+    float g = dy[i];
+    if (relu && !(out[i] > 0.f)) g = 0.f;
+    dx[i] = w[c] * rsqrtf(stats[C + c] + eps) * g;
+  }
+}
+
 // ---- MaxPool2d backward, any kernel / stride, no padding, floor mode; first arg-max in row-major window order ---------
 __global__ void maxpool2d_bwd_kernel(const float* __restrict__ x, const float* __restrict__ g_out, float* __restrict__ g_in, long long total, int H,
                                      int W, int Ho, int Wo, int kh, int kw, int sh, int sw) {
@@ -419,6 +431,28 @@ int mpa_bn_relu_bwd_f32(const float* x, const float* out, const float* dy, const
   else
     bn_relu_bwd_apply_kernel<<<grid_for(total, 256), 256, 0, st>>>(x, out, dy, stats, w, scratch2c, eps, dx, total, C, HW, 1.f / ((float)B * HW), relu);
   MPA_CHECK_LAUNCH("bn_relu_bwd_apply");
+  return MPA_OK;
+}
+
+int mpa_bn_relu_bwd_frozen_f32(const float* x, const float* out, const float* dy, const float* stats, const float* w, float* dx, float* dw, float* db,
+                               float* d_conv_bias, float* scratch2c, int B, int C, int HW, float eps, int relu, void* stream) {
+  MPA_CHECK_ARCH();
+  MPA_REQUIRE(x && out && dy && stats && w && dx && dw && db && scratch2c && B > 0 && C > 0 && HW > 0, "bn_relu_bwd_frozen: bad argument");
+  cudaStream_t st = (cudaStream_t)stream;
+  {
+    // d beta = sum dy', d gamma = sum dy' * xhat with xhat formed from the running statistics
+    int rc = bn_bwd_sums_launch(x, out, dy, stats, eps, scratch2c, dw, db, B, C, HW, relu, st);
+    if (rc != MPA_OK) return rc;
+  }
+  MPA_CHECK_LAUNCH("bn_relu_bwd_frozen_reduce");
+  const long long total = (long long)B * C * HW;
+  bn_relu_bwd_frozen_apply_kernel<<<grid_for(total, 256), 256, 0, st>>>(out, dy, stats, w, eps, dx, total, C, HW, relu);
+  MPA_CHECK_LAUNCH("bn_relu_bwd_frozen_apply");
+  if (d_conv_bias) {
+    int rc = channel_sum_launch(dx, d_conv_bias, B, C, HW, st);
+    if (rc != MPA_OK) return rc;
+    MPA_CHECK_LAUNCH("bn_relu_bwd_frozen_conv_bias");
+  }
   return MPA_OK;
 }
 

@@ -407,6 +407,110 @@ __global__ void __launch_bounds__(kLnPixThreads, 4) layernorm_pix_param_grad_cp8
   }
 }
 
+// LayerNorm([C,F]) backward to the input, with the parameter gradients of the same rows in the same pass (gradients wrt the network input:
+// saliency maps, eval-mode backward).  Per (b,t) row, with v the LayerNorm input (log(1 + gamma_log * x) when the compression is fused),
+// xhat = (v - mean) * rstd and gh = g * w over the C*F elements:
+//   dv = rstd * (gh - mean(gh) - xhat * mean(gh * xhat)),  dx = dv (* gamma_log / (1 + gamma_log * x)),  gw += g * xhat,  gb += g
+// Layout of layernorm_pix_param_grad_cp8_kernel: a thread owns bin f with all C <= 8 channels, the two row means are one CTA reduction.
+// G16 = MPA_FMT_* + 1: g is in the CP8 planes the first convolution's data gradient wrote and (mean, rstd) come from the forward's stats;
+// G16 = 0: g is fp32 NCHW and the row statistics are re-reduced (two-pass, as the forward kernels do).  dx fp32 NCHW (overwritten).
+template <int G16>
+__global__ void __launch_bounds__(kLnPixThreads, 2) layernorm_pix_input_grad_kernel(const float* __restrict__ x, const float* __restrict__ g32,
+                                                                                 const uint4* __restrict__ g16, const float2* __restrict__ stats,
+                                                                                 const float* __restrict__ w, float* __restrict__ dx,
+                                                                                 float* __restrict__ gw, float* __restrict__ gb, int rows, int rpb,
+                                                                                 int C, int T, int F, int TP, int P, int pf, int pt, float eps,
+                                                                                 float gamma_log) {
+  __shared__ float sh[32];       // two regions, used alternately: a reduction's barrier frees the region the one before it read
+  int region = 0;
+  const int f = threadIdx.x;
+  const bool on = f < F;
+  float wc[8], aw[8], ab[8];
+#pragma unroll
+  for (int c = 0; c < 8; ++c) {
+    wc[c] = (on && c < C) ? w[c * F + f] : 0.f;
+    aw[c] = ab[c] = 0.f;
+  }
+  const float inv_n = 1.f / (float)(C * F);
+  const size_t cs = (size_t)T * F;
+  const int r0 = blockIdx.x * rpb, r1 = min(rows, r0 + rpb);
+  for (int r = r0; r < r1; ++r) {
+    const int b = r / T, t = r - b * T;
+    const size_t row = ((size_t)b * C * T + t) * F + f;
+    float v[8], gv[8];
+#pragma unroll
+    for (int c = 0; c < 8; ++c) {
+      v[c] = (on && c < C) ? x[row + c * cs] : 0.f;
+      if constexpr (G16 == 0) gv[c] = (on && c < C) ? g32[row + c * cs] : 0.f;
+    }
+    if constexpr (G16 != 0) {
+      if (on) {
+        unpack8<G16 - 1>(g16[((size_t)b * TP + pt + t) * P + pf + f], gv);
+      } else {
+#pragma unroll
+        for (int c = 0; c < 8; ++c) gv[c] = 0.f;
+      }
+    }
+    if (gamma_log > 0.f) {
+#pragma unroll
+      for (int c = 0; c < 8; ++c)
+        if (on && c < C) v[c] = logf(__fadd_rn(1.f, __fmul_rn(gamma_log, v[c])));
+    }
+    float mean, rstd;
+    if (stats) {
+      const float2 st = stats[r];
+      mean = st.x;
+      rstd = st.y;
+    } else {
+      float s = 0.f, unused = 0.f;
+#pragma unroll
+      for (int c = 0; c < 8; ++c) s += v[c];
+      block_sum2_8w(s, unused, sh + 16 * (region++ & 1));
+      mean = s * inv_n;
+      float q = 0.f;
+#pragma unroll
+      for (int c = 0; c < 8; ++c) {
+        if (on && c < C) {
+          const float d = v[c] - mean;
+          q = fmaf(d, d, q);
+        }
+      }
+      block_sum2_8w(q, unused, sh + 16 * (region++ & 1));
+      rstd = rsqrtf(q * inv_n + eps);
+    }
+    float s1 = 0.f, s2 = 0.f;
+#pragma unroll
+    for (int c = 0; c < 8; ++c) {
+      const float gh = gv[c] * wc[c];          // zero outside the row (wc = 0 there)
+      s1 += gh;
+      s2 = fmaf(gh, (v[c] - mean) * rstd, s2);
+    }
+    block_sum2_8w(s1, s2, sh + 16 * (region++ & 1));
+    const float m1 = s1 * inv_n, m2 = s2 * inv_n;
+    if (on) {
+#pragma unroll
+      for (int c = 0; c < 8; ++c) {
+        if (c < C) {
+          const float xh = (v[c] - mean) * rstd;
+          float d = rstd * (gv[c] * wc[c] - m1 - xh * m2);
+          if (gamma_log > 0.f) d *= gamma_log / __fadd_rn(1.f, __fmul_rn(gamma_log, x[row + c * cs]));
+          dx[row + c * cs] = d;
+          aw[c] = fmaf(gv[c], xh, aw[c]);
+          ab[c] += gv[c];
+        }
+      }
+    }
+  }
+  if (!on) return;
+#pragma unroll
+  for (int c = 0; c < 8; ++c) {
+    if (c < C) {
+      atomicAdd(&gw[c * F + f], aw[c]);
+      atomicAdd(&gb[c * F + f], ab[c]);
+    }
+  }
+}
+
 static inline int ln_rows_per_block(int rows, int ctas_per_sm) {
   int rpb = ceil_div(rows, 148 * ctas_per_sm);
   rpb = (rpb + 1) & ~1;
@@ -540,6 +644,44 @@ int mpa_layernorm_cf_param_grad_cp8_stats(const float* x, const void* g_cp8, con
     layernorm_pix_param_grad_cp8_kernel<MPA_FMT_F16><<<grid, kLnPixThreads, 0, st>>>(x, (const uint4*)g_cp8, (const float2*)stats, g_w, g_b, rows, rpb,
                                                                                     C, T, F, T + 2 * pt, pitch, pf, pt, gamma_log);
   MPA_CHECK_LAUNCH("layernorm_cf_param_grad_cp8_stats");
+  return MPA_OK;
+}
+
+int mpa_layernorm_cf_input_grad_cp8_stats(const float* x, const void* g_cp8, const float* stats, const float* ln_w, float* dx, float* g_w, float* g_b,
+                                          int B, int C, int T, int F, int pitch, int pf, int pt, int fmt, float gamma_log, void* stream) {
+  MPA_CHECK_ARCH();
+  MPA_REQUIRE(x && g_cp8 && stats && ln_w && dx && g_w && g_b && B > 0 && C > 0 && C <= 8 && T > 0 && F > 0 && F <= kLnPixThreads &&
+                  pitch >= pf + F && pt >= 0 && (fmt == MPA_FMT_BF16 || fmt == MPA_FMT_F16) && (long long)B * T < (1ll << 31),
+              "layernorm_cf_input_grad_cp8_stats: bad argument (C <= 8, F <= 256, 16-bit formats)");
+  cudaStream_t st = (cudaStream_t)stream;
+  cudaMemsetAsync(g_w, 0, sizeof(float) * (size_t)C * F, st);
+  cudaMemsetAsync(g_b, 0, sizeof(float) * (size_t)C * F, st);
+  const int rows = B * T, rpb = ln_rows_per_block(rows, 4), grid = ceil_div(rows, rpb);
+  if (fmt == MPA_FMT_BF16)
+    layernorm_pix_input_grad_kernel<MPA_FMT_BF16 + 1><<<grid, kLnPixThreads, 0, st>>>(x, nullptr, (const uint4*)g_cp8, (const float2*)stats, ln_w, dx,
+                                                                                     g_w, g_b, rows, rpb, C, T, F, T + 2 * pt, pitch, pf, pt, 0.f,
+                                                                                     gamma_log);
+  else
+    layernorm_pix_input_grad_kernel<MPA_FMT_F16 + 1><<<grid, kLnPixThreads, 0, st>>>(x, nullptr, (const uint4*)g_cp8, (const float2*)stats, ln_w, dx,
+                                                                                    g_w, g_b, rows, rpb, C, T, F, T + 2 * pt, pitch, pf, pt, 0.f,
+                                                                                    gamma_log);
+  MPA_CHECK_LAUNCH("layernorm_cf_input_grad_cp8_stats");
+  return MPA_OK;
+}
+
+int mpa_layernorm_cf_input_grad_f32(const float* x, const float* g_out, const float* ln_w, float* dx, float* g_w, float* g_b, int B, int C, int T,
+                                    int F, float eps, float gamma_log, void* stream) {
+  MPA_CHECK_ARCH();
+  MPA_REQUIRE(x && g_out && ln_w && dx && g_w && g_b && B > 0 && C > 0 && C <= 8 && T > 0 && F > 0 && F <= kLnPixThreads &&
+                  (long long)B * T < (1ll << 31),
+              "layernorm_cf_input_grad_f32: bad argument (C <= 8, F <= 256)");
+  cudaStream_t st = (cudaStream_t)stream;
+  cudaMemsetAsync(g_w, 0, sizeof(float) * (size_t)C * F, st);
+  cudaMemsetAsync(g_b, 0, sizeof(float) * (size_t)C * F, st);
+  const int rows = B * T, rpb = ln_rows_per_block(rows, 4), grid = ceil_div(rows, rpb);
+  layernorm_pix_input_grad_kernel<0><<<grid, kLnPixThreads, 0, st>>>(x, g_out, nullptr, nullptr, ln_w, dx, g_w, g_b, rows, rpb, C, T, F, 0, 0, 0, 0,
+                                                                     eps, gamma_log);
+  MPA_CHECK_LAUNCH("layernorm_cf_input_grad_f32");
   return MPA_OK;
 }
 

@@ -11,6 +11,7 @@
 // bn_stats -> bn_apply -> nchw_to_cp8 forward, cp8_to_nchw -> two reductions -> bn_bwd_apply -> nchw_to_cp8 backward, 11 + 9 launches per
 // convolution, 2 x 4 bytes per element and direction instead of 2).  All sums are formed in fp32; the per-channel reductions run on a
 // (chunk, slice) grid with an ordered merge (bit-reproducible), only the (mathematically zero) conv-bias gradient meets in atomics.
+// Eval-mode backward (BatchNorm frozen at its running statistics) has its own one-pass kernel below: dy = gamma * rstd * g'.
 #include "common.cuh"
 #include "cp8.cuh"
 
@@ -335,6 +336,67 @@ __global__ void __launch_bounds__(kUT) bn_relu_bwd_apply_cp8_kernel(const uint4*
   }
 }
 
+// ---- backward with frozen statistics (eval-mode BatchNorm: running mean / variance, nothing depends on the batch) ------------------
+// g' = g * [a > 0];  dy = gamma * rstd * g' (one pass, written as CP8);  d gamma = sum g' * xhat, d beta = sum g', d conv-bias = sum dy.
+// Same (chunk, slice) grid and ordered last-block merge as the batch-statistics backward; the conv-bias gradient is a third ordered sum
+// here (it is not zero: the statistics do not follow the convolution's bias).
+template <int FMT>
+__global__ void __launch_bounds__(kUT) bn_relu_bwd_frozen_cp8_kernel(const uint4* __restrict__ g, const uint4* __restrict__ y, uint4* __restrict__ dy,
+                                                                     const float* __restrict__ stats, const float* __restrict__ w,
+                                                                     const float* __restrict__ bias, float eps, float* __restrict__ partial,
+                                                                     unsigned n, Cp8Geo geo, int C, int ncs_g, int ncs_y, int ncs_dy, int S,
+                                                                     BnBwdFinal f, int g_split, int Pg) {
+  __shared__ float sh[kUT / 32 * 24];
+  const int ck = blockIdx.x, s = blockIdx.y;
+  const unsigned i0 = (unsigned)((unsigned long long)n * s / S), i1 = (unsigned)((unsigned long long)n * (s + 1) / S);
+  float mean[8], rstd[8], wc[8], bc[8], acc[24];
+#pragma unroll
+  for (int e = 0; e < 8; ++e) {
+    const int c = ck * 8 + e;
+    mean[e] = stats[c];
+    rstd[e] = rsqrtf(stats[C + c] + eps);
+    wc[e] = w[c];
+    bc[e] = bias[c];
+    acc[e] = acc[8 + e] = acc[16 + e] = 0.f;
+  }
+  for (unsigned i = i0 + threadIdx.x; i < i1; i += kUT) {
+    float gv[8], yv[8], r[8];
+    unpack8<FMT>(g[g_split ? geo.at_split(i, gridDim.x, ck, g_split, Pg) : geo.at(i, ncs_g, ck)], gv);
+    unpack8<FMT>(y[geo.at(i, ncs_y, ck)], yv);
+#pragma unroll
+    for (int e = 0; e < 8; ++e) {
+      const float gp = bn_val(yv[e], mean[e], rstd[e], wc[e], bc[e]) > 0.f ? gv[e] : 0.f;
+      r[e] = wc[e] * rstd[e] * gp;
+      acc[e] += gp;
+      acc[8 + e] = fmaf(gp, (yv[e] - mean[e]) * rstd[e], acc[8 + e]);
+      acc[16 + e] += r[e];
+    }
+    dy[geo.at(i, ncs_dy, ck)] = pack8<FMT>(r);
+  }
+  block_sum_n<24>(acc, sh);
+  if (threadIdx.x < 24) {
+    const int e = threadIdx.x & 7, which = threadIdx.x >> 3;
+    partial[(size_t)(which * C + ck * 8 + e) * S + s] = acc[threadIdx.x];
+  }
+  unsigned* counter = reinterpret_cast<unsigned*>(partial) - 64 + ck;
+  if (!last_block_done(counter)) return;
+  // the 24 rows of this chunk (s1 | s2 | sum dy per channel), three per warp, each summed lane-strided + shuffle tree (fixed order)
+#pragma unroll
+  for (int which = 0; which < 3; ++which) {
+    const int c = ck * 8 + (threadIdx.x >> 5);
+    const int k = which * C + c;
+    float t = 0.f;
+    for (int sl = threadIdx.x & 31; sl < S; sl += 32) t += __ldcg(&partial[(size_t)k * S + sl]);
+    t = warp_sum(t);
+    if ((threadIdx.x & 31) == 0) {
+      if (which == 0) f.db[c] = t;
+      else if (which == 1) f.dw[c] = t;
+      else if (f.conv_gb) f.conv_gb[c] = t;
+    }
+  }
+  if (threadIdx.x == 0) *counter = 0u;
+}
+
 // ---- MaxPool2d(2) backward + skip-gradient add ----------------------------------------------------------------------------------------
 // thread = one pixel-chunk of the un-pooled level: out = addend + [this pixel is the first maximum of its window] * g_pool[window]
 template <int FMT>
@@ -516,6 +578,34 @@ int mpa_bn_relu_bwd_cp8(const void* g_cp8, const void* y_cp8, void* dy_cp8, cons
                                                                      sums, eps, inv_n, g_conv_bias, C, NCk, T, F, T + 2 * pt, pitch, pf, pt, ncs_g,
                                                                      ncs_y, ncs_dy, g_split, g_pitch);
   MPA_CHECK_LAUNCH("bn_relu_bwd_apply_cp8");
+  return MPA_OK;
+}
+
+int mpa_bn_relu_bwd_frozen_cp8(const void* g_cp8, const void* y_cp8, void* dy_cp8, const float* stats, const float* weight, const float* bias,
+                               float eps, float* g_weight, float* g_bias, float* g_conv_bias, int B, int C, int T, int F, int pitch, int pf, int pt,
+                               int ncs_g, int ncs_y, int ncs_dy, int g_split, int g_pitch, int fmt, void* stream) {
+  UNET_CP8_COMMON("bn_relu_bwd_frozen_cp8");
+  MPA_REQUIRE(g_cp8 && y_cp8 && dy_cp8 && stats && weight && bias && g_weight && g_bias, "bn_relu_bwd_frozen_cp8: null pointer");
+  MPA_REQUIRE(g_split == 0 || (g_split > 1 && F % g_split == 0 && g_pitch >= pf + F / g_split), "bn_relu_bwd_frozen_cp8: bad phase split");
+  float* scratch = unet_scratch();
+  MPA_REQUIRE(scratch, "bn_relu_bwd_frozen_cp8: scratch allocation failed");
+  const int NCk = C / 8;
+  if (ncs_g <= 0) ncs_g = NCk;
+  if (ncs_y <= 0) ncs_y = NCk;
+  if (ncs_dy <= 0) ncs_dy = NCk;
+  const unsigned n = (unsigned)B * T * F;
+  const int S = slices_for(n, NCk);
+  MPA_REQUIRE((size_t)3 * C * S <= (1u << 20) && NCk <= 64, "bn_relu_bwd_frozen_cp8: too many channels (<= 512)");
+  const Cp8Geo geo{T, F, T + 2 * pt, pitch, pf, pt};
+  const BnBwdFinal f{nullptr, g_weight, g_bias, g_conv_bias};
+  cudaStream_t st = (cudaStream_t)stream;
+  if (fmt == MPA_FMT_BF16)
+    bn_relu_bwd_frozen_cp8_kernel<MPA_FMT_BF16><<<dim3(NCk, S), kUT, 0, st>>>((const uint4*)g_cp8, (const uint4*)y_cp8, (uint4*)dy_cp8, stats, weight,
+                                                                             bias, eps, scratch, n, geo, C, ncs_g, ncs_y, ncs_dy, S, f, g_split, g_pitch);
+  else
+    bn_relu_bwd_frozen_cp8_kernel<MPA_FMT_F16><<<dim3(NCk, S), kUT, 0, st>>>((const uint4*)g_cp8, (const uint4*)y_cp8, (uint4*)dy_cp8, stats, weight,
+                                                                            bias, eps, scratch, n, geo, C, ncs_g, ncs_y, ncs_dy, S, f, g_split, g_pitch);
+  MPA_CHECK_LAUNCH("bn_relu_bwd_frozen_cp8");
   return MPA_OK;
 }
 

@@ -41,6 +41,10 @@ def _head(model, c0, n_ch, n_bins_in, n_bins_out, a, p):
 
 
 class _MpaModel(nn.Module):
+    # eval mode + autograd recording: True records the eval tape (dropout off, BatchNorm frozen at its running statistics) even when the
+    # input needs no gradient — fine-tuning with frozen statistics; False (default) keeps that forward on the inference path, no grad_fn
+    eval_backward = False
+
     def _init_common(self, n_chan_input, n_bins_in, a_lrelu, p_dropout, precision):
         if precision is None:
             precision = _exec.DEFAULT_PRECISION          # the reference's constructors take no such keyword: package-level default
@@ -53,9 +57,10 @@ class _MpaModel(nn.Module):
 
 
 def _dispatch(model, x):
-    """Autograd recording -> the training tape; train mode under no_grad -> the training forward with its tape discarded (dropout stays
-    active exactly as in the reference, whose validation pass runs in train mode: exp126a...py:333-345); eval -> inference path."""
-    if torch.is_grad_enabled() and (model.training or x.requires_grad):
+    """Autograd recording -> the training tape (in eval mode only when a graph is asked for: x requires grad, or model.eval_backward; then
+    with dropout off); train mode under no_grad -> the training forward with its tape discarded (dropout stays active exactly as in the
+    reference, whose validation pass runs in train mode: exp126a...py:333-345); eval -> inference path."""
+    if torch.is_grad_enabled() and (model.training or x.requires_grad or model.eval_backward):
         from ...training import cnn_train_forward, forward_train
         return forward_train(cnn_train_forward, model, x)
     if model.training and model.p_dropout > 0:

@@ -204,6 +204,12 @@ class _UnetBase(_MpaModel):
     def _bn_train(self):
         return self.training
 
+    def _eval_tape(self, x):
+        """Eval mode, autograd recording, and a graph asked for: x requires grad (saliency), or `eval_backward` is set (fine-tuning with
+        frozen BatchNorm statistics).  Anything else in eval mode — the reference's `model.eval(); model(batch)` test loop included — takes
+        the inference path and returns a tensor without grad_fn."""
+        return not self.training and torch.is_grad_enabled() and (x.requires_grad or self.eval_backward)
+
     def predict_frames(self, plane, i0, n):
         """Eval-mode forward of the n stride-1 patches starting at frames i0.. of a recording whose LayerNorm'ed (+ log-compressed) frames
         sit in the 16-bit frame-major `plane` [rows][pitch][8] (mpa_layernorm_frames; engine.predict_patchwise builds it once per
@@ -229,8 +235,12 @@ class _UnetBase(_MpaModel):
             self._train_calls = getattr(self, '_train_calls', 0) + 1
             y, n_pred, _ = unet_train_forward(self, x, {}, getattr(self, 'dropout_seed', 0x5EED), self._train_calls)
             return y.d, (n_pred.d if n_pred is not None else None)
-        if torch.is_grad_enabled() and x.requires_grad:
-            raise NotImplementedError('eval-mode forward does not record gradients; call .train() (reference scripts train in train mode)')
+        if self._eval_tape(x):
+            # eval mode with a graph asked for: the training tape with dropout off and BatchNorm frozen at its running statistics
+            from ...training import forward_train
+            from ...training_unet import unet_train_forward
+            out = forward_train(unet_train_forward, self, x)
+            return out if isinstance(out, tuple) else (out, None)
         train = self._bn_train()
         if _exec.unet_tc_eligible(self, x):
             y, x5c = _exec.unet_forward_tc(self, x)
@@ -328,8 +338,8 @@ class simple_u_net_polyphony_classif_softmax(_UnetBase):
 
     def forward(self, x):
         y, x5 = self._run(x)
-        if self.training:
-            return y, x5                     # the training path evaluates convP itself (x5 slot = n_pred)
+        if self.training or self._eval_tape(x):
+            return y, x5                     # the training tape evaluates convP itself (x5 slot = n_pred)
         return self._finish(y, x5)
 
     def _finish(self, y, x5):

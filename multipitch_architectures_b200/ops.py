@@ -60,6 +60,22 @@ def layernorm_cf_param_grad_cp8(x, g, gw, gb, eps, gamma_log=0.0, stats=None):
              stream_ptr())
 
 
+def layernorm_cf_input_grad(x, g, w, gw, gb, eps, gamma_log=0.0, stats=None):
+    """-> dx [B,C,T,F] fp32: gradient wrt the LayerNorm([C,F]) input x; gw / gb [C,F] (overwritten) as layernorm_cf_param_grad_cp8 leaves
+    them, from the same pass.  g: CP8 planes together with the forward's (mean, rstd) rows `stats`, or fp32 NCHW (stats None: the row
+    statistics are re-reduced)."""
+    B, C, T, F = x.shape
+    dx = torch.empty_like(x)
+    if isinstance(g, CP8):
+        assert (g.B, g.T, g.F) == (B, T, F) and g.ncs == 1 and stats is not None
+        call('layernorm_cf_input_grad_cp8_stats', _f32(x), g.ptr(), stats, _f32(w), dx, gw, gb, B, C, T, F, g.pitch, g.pf, g.pt, g.fmt,
+             float(gamma_log), stream_ptr())
+    else:
+        assert stats is None and tuple(g.shape) == (B, C, T, F)
+        call('layernorm_cf_input_grad_f32', _f32(x), _f32(g), _f32(w), dx, gw, gb, B, C, T, F, float(eps), float(gamma_log), stream_ptr())
+    return dx
+
+
 def conv2d(x, wp, bias, Cout, ksize, stride=(1, 1), padding=(0, 0), act=ACT_NONE, act_param=0.0,
            scale=None, shift=None, x2=None):
     B, C1, H, W = x.shape
@@ -338,6 +354,25 @@ def bn_relu_bwd_cp8(g, y, stats, bn, dy, g_weight, g_bias, g_conv_bias=None, spl
         assert (y.B, y.C, y.T, y.F, y.pitch, y.pf, y.pt) == (g.B, g.C, g.T, g.F, g.pitch, g.pf, g.pt)
     call('bn_relu_bwd_cp8', g.ptr(), y.ptr(), dy.ptr(), stats, bn.weight, bn.bias, float(bn.eps), g_weight, g_bias, g_conv_bias, y.B, y.C, y.T, y.F,
          y.pitch, y.pf, y.pt, g.ncs, y.ncs, dy.ncs, int(split), g.pitch if split else 0, y.fmt, stream_ptr())
+    return dy
+
+
+def bn_frozen_stats(bn):
+    """[2C] fp32 = [running_mean | running_var] of an eval-mode nn.BatchNorm2d: the statistics operand of bn_apply / bn_relu_apply_cp8 and
+    of the frozen backward kernels (a parameter preparation; the buffers themselves are only read)."""
+    return torch.cat([bn.running_mean.detach(), bn.running_var.detach()]).float().contiguous()
+
+
+def bn_relu_bwd_frozen_cp8(g, y, stats, bn, dy, g_weight, g_bias, g_conv_bias=None, split=0):
+    """Eval-mode form of bn_relu_bwd_cp8 (stats = bn_frozen_stats(bn)): dy (CP8, written) = weight * rstd * g * [out > 0];
+    g_weight / g_bias / g_conv_bias (= sum dy, not zero here) overwritten."""
+    assert (y.B, y.C, y.T, y.F, y.pitch, y.pf, y.pt) == (dy.B, dy.C, dy.T, dy.F, dy.pitch, dy.pf, dy.pt)
+    if split:
+        assert (g.B, g.C, g.T, g.F) == (y.B, split * y.C, y.T, y.F // split)
+    else:
+        assert (y.B, y.C, y.T, y.F, y.pitch, y.pf, y.pt) == (g.B, g.C, g.T, g.F, g.pitch, g.pf, g.pt)
+    call('bn_relu_bwd_frozen_cp8', g.ptr(), y.ptr(), dy.ptr(), stats, bn.weight, bn.bias, float(bn.eps), g_weight, g_bias, g_conv_bias, y.B, y.C,
+         y.T, y.F, y.pitch, y.pf, y.pt, g.ncs, y.ncs, dy.ncs, int(split), g.pitch if split else 0, y.fmt, stream_ptr())
     return dy
 
 

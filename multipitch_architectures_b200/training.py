@@ -488,11 +488,15 @@ class Node:
 class Tape:
     """Reverse-mode tape of a train-mode forward: each stage computes its output Node and records the closure of its own backward, which
     reads the output's gradient and accumulates its input's.  A dropout stage takes its Philox offset (step * sites_per_step + site, sites
-    counted in forward order) once, in the forward, and its backward reuses it."""
+    counted in forward order) once, in the forward, and its backward reuses it.
+    need_input_grad: the LayerNorm stage on the network input also leaves the gradient wrt that input in `input_grad` (one fused kernel
+    instead of the parameter-only one; every other launch is unchanged).  frozen_bn: BatchNorm stages (UnetTape) use and keep the running
+    statistics — the eval-mode tape."""
 
-    def __init__(self, grads, seed, step, sites_per_step, model):
+    def __init__(self, grads, seed, step, sites_per_step, model, need_input_grad=False, frozen_bn=False):
         self.ops, self.grads, self.seed, self.site, self.model = [], grads, seed, step * sites_per_step, model
         self.trunk_mark = 0
+        self.need_input_grad, self.frozen_bn, self.input_grad = bool(need_input_grad), bool(frozen_bn), None
 
     def push(self, fn):
         self.ops.append(fn)
@@ -553,10 +557,14 @@ class Tape:
         return out
 
     def layernorm_cf(self, ln, x):
-        """LayerNorm([C,F]) on the network input: only the affine parameters receive gradients."""
+        """LayerNorm([C,F]) on the network input: the affine parameters receive gradients, and the input too when need_input_grad."""
         out = Node(ops.layernorm_cf(x, ln.weight, ln.bias, ln.eps))
 
         def bwd():
+            if self.need_input_grad:
+                self.input_grad = ops.layernorm_cf_input_grad(x, out.g, ln.weight, self.grads['layernorm.weight'], self.grads['layernorm.bias'],
+                                                              ln.eps)
+                return
             B, C, T, F = x.shape
             call('layernorm_cf_param_grad_f32', x, out.g, self.grads['layernorm.weight'], self.grads['layernorm.bias'], B, C, T, F,
                  float(ln.eps), 0.0, stream_ptr())
@@ -569,7 +577,15 @@ class Tape:
         B, _, T, F = x.shape
         stats = torch.empty(B * T, 2, dtype=torch.float32, device=x.device) if (F <= 256 and LN_PIXEL) else None
         out = Node(ops.layernorm_cf_cp8(x, ln.weight, ln.bias, ln.eps, dst, stats=stats, pixel=LN_PIXEL))
-        self.push(lambda: ops.layernorm_cf_param_grad_cp8(x, out.g, self.grads['layernorm.weight'], self.grads['layernorm.bias'], ln.eps, stats=stats))
+
+        def bwd():
+            gw, gb = self.grads['layernorm.weight'], self.grads['layernorm.bias']
+            if self.need_input_grad:       # without the saved rows (LN_PIXEL = False) the fp32 kernel re-reduces them from the converted planes
+                g = out.g if stats is not None else ops.cp8_to_nchw(out.g)
+                self.input_grad = ops.layernorm_cf_input_grad(x, g, ln.weight, gw, gb, ln.eps, stats=stats)
+                return
+            ops.layernorm_cf_param_grad_cp8(x, out.g, gw, gb, ln.eps, stats=stats)
+        self.push(bwd)
         return out
 
     # The fused pool + dropout stages below take their dropout site whatever p is: the CP8 kernels receive the offset even when p = 0.
@@ -658,11 +674,23 @@ class Tape:
         return self.conv('conv4.3', m.conv4[3], h, ops.ACT_SIGMOID)
 
 
-def cnn_train_forward(model, x, grads, seed=0, step=0):
-    """-> (y_pred Node [B,1,T-74,72], None, tape).  Train mode: dropout active when model.p_dropout > 0.  bf16 models without the residual
-    path keep the block activations and gradients on the CP8 planes (_cp8_resident)."""
+def note_fp32_tape(model):
+    """An eval-mode backward of a tensor-core model that runs on the fp32 NCHW tape says so, once per model class."""
+    prec = getattr(model, 'precision', 'fp32')
+    if prec == 'bf16':
+        _exec.note_path(model, 'eval-mode backward runs on the fp32 NCHW training tape (tensor-core convolutions behind nchw<->CP8 converters), '
+                               'not on the CP8-resident tape')
+    elif prec in _exec.TC_PRECISIONS:
+        _exec.note_path(model, 'eval-mode backward runs on the fp32 NCHW training tape (fp32 CUDA-core kernels): the training kernels have no '
+                               f'{prec} form')
+
+
+def cnn_train_forward(model, x, grads, seed=0, step=0, need_input_grad=False, frozen_bn=False):
+    """-> (y_pred Node [B,1,T-74,72], None, tape).  Train mode: dropout active when model.p_dropout > 0; eval mode: dropout off.  bf16 models
+    without the residual path keep the block activations and gradients on the CP8 planes (_cp8_resident).  need_input_grad: the tape also
+    leaves the gradient wrt x in tape.input_grad.  frozen_bn: accepted for the common builder signature (the CNN family has no BatchNorm)."""
     a, p = model.a_lrelu, (model.p_dropout if model.training else 0.0)
-    tp = Tape(grads, seed, step, SITES_PER_STEP, model)
+    tp = Tape(grads, seed, step, SITES_PER_STEP, model, need_input_grad, frozen_bn)
     blocks = _exec.cnn_blocks(model)
     B, C, T, F = x.shape
     split = 0
@@ -672,6 +700,8 @@ def cnn_train_forward(model, x, grads, seed=0, step=0):
         for i, (name, conv) in enumerate(blocks):
             z = tp.block_cp8(name + '.0', conv, z, p, a, split if i == len(blocks) - 1 else 0)
     else:
+        if not model.training:
+            note_fp32_tape(model)
         z = tp.layernorm_cf(model.layernorm, x)
         residual = getattr(model, 'residual', False)
         for i, (name, conv) in enumerate(blocks):
@@ -682,14 +712,15 @@ def cnn_train_forward(model, x, grads, seed=0, step=0):
 
 class TrainFunction(torch.autograd.Function):
     """Drop-in autograd bridge: `model.train(); y = model(x); loss.backward()` runs the tape that `build` (cnn_train_forward,
-    training_unet.unet_train_forward) recorded."""
+    training_unet.unet_train_forward) recorded.  A model in eval mode records the eval tape (dropout off, BatchNorm frozen at its running
+    statistics); x receives its gradient when it requires one."""
 
     @staticmethod
     def forward(ctx, build, model, x, seed, step, *params):
         named = list(model.named_parameters())
         with torch.no_grad():
             grads = {n: torch.zeros_like(p) for n, p in named}
-            y, n_pred, tape = build(model, x, grads, seed, step)
+            y, n_pred, tape = build(model, x, grads, seed, step, need_input_grad=ctx.needs_input_grad[2], frozen_bn=not model.training)
         ctx.model, ctx.tape, ctx.grads, ctx.nodes = model, tape, grads, (y, n_pred)
         if n_pred is None:
             return y.d
@@ -704,7 +735,7 @@ class TrainFunction(torch.autograd.Function):
                 n_pred.g = g_n.contiguous() if g_n is not None else torch.zeros_like(n_pred.d)
             ctx.tape.backward()
         named = list(ctx.model.named_parameters())
-        return (None, None, None, None, None) + tuple(ctx.grads[n] for n, _ in named)
+        return (None, None, ctx.tape.input_grad, None, None) + tuple(ctx.grads[n] for n, _ in named)
 
 
 def forward_train(build, model, x):

@@ -20,7 +20,8 @@ import torch
 from . import _lib, ops
 from ._lib import call, stream_ptr
 from .libdl.nn_models import _exec
-from .training import FusedTrainStep, Node, Tape, TcConv, ctypes_u64, _act_bwd, _add, _s3_split_eligible, _split_buf, _step_args, _tc_s3_eligible
+from .training import (FusedTrainStep, Node, Tape, TcConv, ctypes_u64, note_fp32_tape, _act_bwd, _add, _s3_split_eligible, _split_buf, _step_args,
+                       _tc_s3_eligible)
 
 SITES_PER_STEP = 256      # dropout sites reserved per step of the U-Net tape: offset = step * 256 + site
 
@@ -30,8 +31,21 @@ class UnetTape(Tape):
     layer and the BLSTM."""
 
     def bn_relu(self, name, bn, y):
-        """BatchNorm2d in training mode (batch statistics) + ReLU; running statistics updated as nn.BatchNorm2d does."""
+        """BatchNorm2d in training mode (batch statistics) + ReLU; running statistics updated as nn.BatchNorm2d does.  frozen_bn: eval mode
+        (the running statistics normalise and stay untouched; the convolution's own backward sums its bias gradient from dx)."""
         B, C, H, W = y.d.shape
+        if self.frozen_bn:
+            stats = ops.bn_frozen_stats(bn)
+            out = Node(ops.bn_apply(y.d, stats, bn.weight, bn.bias, bn.eps, ops.ACT_RELU, 0.0))
+
+            def bwd_frozen():
+                dx = torch.empty_like(y.d)
+                scratch = torch.empty(2 * C, dtype=torch.float32, device=y.d.device)
+                call('bn_relu_bwd_frozen_f32', y.d, out.d, out.g, stats, bn.weight, dx, self.grads[name + '.weight'], self.grads[name + '.bias'],
+                     None, scratch, B, C, H * W, float(bn.eps), 1, stream_ptr())
+                y.acc(dx)
+            self.push(bwd_frozen)
+            return out
         stats = ops.bn_stats(y.d)
         if bn.track_running_stats:
             n = B * H * W
@@ -95,15 +109,17 @@ class UnetTape(Tape):
 
     def bn_relu_cp8(self, name, bn, y, dst, conv_bias_name, split=0, conv_bias=None):
         """BatchNorm2d (train mode, running statistics updated) + ReLU on the planes, written into `dst` (a buffer or a channel view of a
-        concat buffer; split = s: phase-split planes, the hand-over to the head's stride-(1, s) convolution and back)."""
-        stats = ops.bn_stats_cp8(y.d, bn, pivot=conv_bias)
+        concat buffer; split = s: phase-split planes, the hand-over to the head's stride-(1, s) convolution and back).  frozen_bn: eval mode,
+        normalised with the running statistics, which stay untouched."""
+        frozen = self.frozen_bn
+        stats = ops.bn_frozen_stats(bn) if frozen else ops.bn_stats_cp8(y.d, bn, pivot=conv_bias)
         out = Node(ops.bn_relu_apply_cp8(y.d, stats, bn, dst, split))
 
         def bwd():
             yc = y.d
             dy = TcConv._buf(name + ':dy', yc.B, yc.C, yc.T, yc.F, yc.buf.device, yc.fmt)
-            y.g = ops.bn_relu_bwd_cp8(out.g, yc, stats, bn, dy, self.grads[name + '.weight'], self.grads[name + '.bias'],
-                                        self.grads[conv_bias_name], split)
+            bwd_fn = ops.bn_relu_bwd_frozen_cp8 if frozen else ops.bn_relu_bwd_cp8
+            y.g = bwd_fn(out.g, yc, stats, bn, dy, self.grads[name + '.weight'], self.grads[name + '.bias'], self.grads[conv_bias_name], split)
         self.push(bwd)
         return out
 
@@ -447,12 +463,12 @@ def cp8_tape_eligible(model, x):
     return geo[4][0] >= 1 and _tc_s3_eligible(model, model.conv2[0], F) and model.conv2[0].weight.shape[1] % 8 == 0
 
 
-def _unet_train_forward_cp8(model, x, grads, seed, step):
+def _unet_train_forward_cp8(model, x, grads, seed, step, need_input_grad=False, frozen_bn=False):
     """The CP8-resident tape: LayerNorm -> planes -> [conv -> BN stats -> BN+ReLU]* with max-pool / up-sampling / concat on the planes ->
     (encoder layers in fp32 tokens) -> head conv2 on the planes -> fp32 72-bin head."""
     p = model.p_dropout if model.training else 0.0
     fmt = ops.FMT_BF16
-    tp = UnetTape(grads, seed, step, SITES_PER_STEP, model)
+    tp = UnetTape(grads, seed, step, SITES_PER_STEP, model, need_input_grad, frozen_bn)
     B, C, T, F = x.shape
     dev = x.device
     geo = _exec.level_geometry(T, F)
@@ -485,12 +501,16 @@ def _unet_train_forward_cp8(model, x, grads, seed, step):
     return tp.head(u, p, split), None, tp
 
 
-def unet_train_forward(model, x, grads, seed=0, step=0):
-    """-> (y_pred [B,1,T-74,72], n_pred or None, tape).  Train mode: BatchNorm batch statistics, dropout when p > 0."""
+def unet_train_forward(model, x, grads, seed=0, step=0, need_input_grad=False, frozen_bn=False):
+    """-> (y_pred [B,1,T-74,72], n_pred or None, tape).  Train mode: BatchNorm batch statistics, dropout when p > 0.  Eval mode: dropout
+    off (encoder layers and convP included); frozen_bn: BatchNorm normalises with its running statistics and leaves them as they are.
+    need_input_grad: the tape also leaves the gradient wrt x in tape.input_grad."""
     if cp8_tape_eligible(model, x):
-        return _unet_train_forward_cp8(model, x, grads, seed, step)
+        return _unet_train_forward_cp8(model, x, grads, seed, step, need_input_grad, frozen_bn)
+    if not model.training:
+        note_fp32_tape(model)
     a, p = model.a_lrelu, (model.p_dropout if model.training else 0.0)
-    tp = UnetTape(grads, seed, step, SITES_PER_STEP, model)
+    tp = UnetTape(grads, seed, step, SITES_PER_STEP, model, need_input_grad, frozen_bn)
     z = tp.layernorm_cf(model.layernorm, x)
     x1 = tp.double_conv('inc', model.inc, z)       # (the gradient wrt z feeds the LayerNorm parameter gradients)
     xs = [x1]
