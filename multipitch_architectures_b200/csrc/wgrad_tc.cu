@@ -15,6 +15,11 @@
 // The g rows live in a shared-memory ring whose slots ascend with t (one new row per x row; the RS-1 wrapping slots are mirrored).
 // KH x 1 filters (`wide`): with one tap an MMA per input chunk would have N = 16 columns; instead up to 16 input chunks of a group are the
 // N groups of ONE MMA (their slabs sit at a uniform stride in the x stage: SBO = slab bytes), N = 8 * chunks <= 128, one accumulator.
+// Because K walks every pixel of the padded row, the result is right only when the inputs keep these conditions:
+//   - the gap columns of g's real channels are zero (its pad rows are never read);
+//   - the x pixels within KW/2 of a real bin are zero where they are not real bins themselves, counted along the flattened rows: the band
+//     right of a row may continue into the next row's first columns;
+//   - every byte it reads is finite (NaN * 0 = NaN).
 #include "common.cuh"
 #include <cuda.h>
 #include <string.h>

@@ -520,7 +520,9 @@ def _zero_row(device, nbytes):
 
 
 def conv_wgrad_tc(x, g, gw, ksize):
-    """gw [Cout, Cin, KH, KW] fp32 (overwritten) = weight gradient of the stride-1 'same' convolution; x, g: CP8 of one geometry."""
+    """gw [Cout, Cin, KH, KW] fp32 (overwritten) = weight gradient of the stride-1 'same' convolution; x, g: CP8 of one geometry.
+    The kernel sums over every pixel of the padded rows, so the planes must keep: the gap columns of g's real channels zero; the x pixels
+    within KW/2 of a real bin (along the flattened rows) zero; everything finite."""
     Cout_t, Cin_t, KH, KW = gw.shape
     assert (KH, KW) == tuple(ksize) and x.B == g.B and (x.T, x.F, x.pitch, x.pf, x.pt) == (g.T, g.F, g.pitch, g.pf, g.pt)
     gw.zero_()

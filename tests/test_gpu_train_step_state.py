@@ -78,6 +78,48 @@ def test_dropped_step_leaves_nothing_to_the_next_one(a, b):
     assert len(step._state.plan.jobs) == ref_jobs > 0
 
 
+def _cp8_entries(v):
+    from multipitch_architectures_b200 import ops
+    if isinstance(v, ops.CP8):
+        yield v
+    elif isinstance(v, dict):
+        for u in v.values():
+            yield from _cp8_entries(u)
+    elif isinstance(v, (list, tuple)):
+        for u in v:
+            yield from _cp8_entries(u)
+
+
+@pytest.mark.parametrize('name', ['cnn_xs', 'saunet_tiny'])
+def test_pooled_planes_keep_the_zero_gap_condition(name):
+    """mpa_conv_wgrad_tc sums over every pixel of the padded rows, so its results are right only when the gap columns of its planes are
+    zero and everything it reads is finite.  After three bf16 training steps with dropout on, every pooled CP8 buffer with pad rows holds
+    zeros in the pad rows and gap columns of its real channels, and no NaN or Inf anywhere."""
+    model = _model(name, 4)
+    assert model.p_dropout > 0
+    step = _step(name, model)
+    for x, t in _batches(name, 3):
+        step(x, t)
+    torch.cuda.synchronize()
+    seen = 0
+    for key, a in step._state.pool.items():
+        for v in _cp8_entries(a):
+            if v.pt < 1:
+                continue
+            seen += 1
+            assert bool(torch.isfinite(v.buf).all()), f'{key}: non-finite values'
+            pl = v.buf[:v.B, v.chunk0:v.chunk0 + v.NC].float()
+            real = torch.zeros(pl.shape[2:4], dtype=torch.bool, device=pl.device)
+            real[v.pt:v.pt + v.T, v.pf:v.pf + v.F] = True
+            for k in range(v.NC):
+                nl = min(8, v.C - 8 * k)
+                gap = pl[:, k][:, ~real][..., :nl]
+                bad = int((gap != 0).sum())
+                assert bad == 0, f'{key}: {bad} non-zero values in the pad rows / gap columns of chunk {k}'
+    print(f'{name}: {seen} pooled CP8 buffers checked')
+    assert seen > 0
+
+
 @pytest.mark.parametrize('name,stage', [('cnn_xs', 'channel_sum_cp8'), ('saunet_tiny', 'gemm_tc_chunks')])
 def test_stage_that_raises_leaves_the_step_usable(name, stage, monkeypatch):
     """A Python stage raises once after weight gradients were forked onto the side stream: the exception reaches the caller, no step state
