@@ -523,6 +523,17 @@ int mpa_layernorm_cf_param_grad_f32(const float* x, const float* g_out, float* g
 /* torch.optim.AdamW step on one flat tensor (exp126a…py:103-108,293); grad is multiplied by grad_scale first. */
 int mpa_adamw_f32(float* param, const float* grad, float* exp_avg, float* exp_avg_sq, long long n, float lr,
                   float beta1, float beta2, float eps, float weight_decay, int step, float grad_scale, void* stream);
+/* Dynamic loss scaling of fp16 training (torch.amp.GradScaler defaults in the caller: 2^16, x2 after 2000 clean steps, x0.5 on an overflow).
+ * The state lives in device memory, so a step needs no host synchronisation and a CUDA-graph replay behaves as the eager step.
+ * *found_inf = 1 when any of x[0, n) is an inf or a NaN, else 0 (overwritten; any alignment, any n). */
+int mpa_nonfinite_check_f32(const float* x, long long n, int* found_inf, void* stream);
+/* mpa_adamw_f32 on grad * grad_scale / *loss_scale (grad_scale: the world-size factor of an all-reduced gradient), bias-corrected for step
+ * *applied_steps + 1 — or, when *found_inf is set, nothing at all (param, exp_avg, exp_avg_sq untouched).  Then the scaler update:
+ * overflow -> *loss_scale *= backoff_factor, *growth_tracker = 0; else ++*applied_steps, and after growth_interval clean steps in a row
+ * *loss_scale *= growth_factor (kept if finite), *growth_tracker = 0. */
+int mpa_adamw_scaled_f32(float* param, const float* grad, float* exp_avg, float* exp_avg_sq, long long n, float lr, float beta1, float beta2,
+                         float eps, float weight_decay, float grad_scale, const int* found_inf, float* loss_scale, int* growth_tracker,
+                         int* applied_steps, float growth_factor, float backoff_factor, int growth_interval, void* stream);
 
 /* ---- tcgen05 GEMM for the token-wise Linear layers of transformer_enc_layer (unet_cnns.py:131-157) ------------------------
  * Y[M,N] fp32 row-major = act(X[M,K] * W[N,K]^T + bias[N]) with 16-bit operands in the chunk layout [ceil(K/64)*8][rows padded][8]
@@ -624,10 +635,16 @@ int mpa_nchw_tokens_f32(const float* src, float* dst, int B, int E, int S, int t
  * class = (long) sum_p y_true[b,p]) forward (added to *loss_sum when accumulate_loss, else overwriting) + d/d logits. */
 int mpa_ce_count_fwd_bwd_f32(const float* logits, const float* y_true, float* loss_sum, float* grad_logits, int B, int K,
                              int P, float scale, int accumulate_loss, void* stream);
+/* The same with grad_logits multiplied by *loss_scale (device memory; the loss of fp16 training is scaled for its backward only). */
+int mpa_ce_count_fwd_bwd_scaled_f32(const float* logits, const float* y_true, float* loss_sum, float* grad_logits, int B, int K, int P,
+                                    float scale, int accumulate_loss, const float* loss_scale, void* stream);
 
 /* ---- N11: BCELoss(mean) on sigmoid outputs with the -100 log clamp, forward + d(loss)/d(pred) ---------- */
 int mpa_bce_fwd_bwd_f32(const float* y_pred, const float* y_true, float* loss_sum, float* grad_pred, long long n,
                         void* stream);
+/* The same with grad_pred multiplied by *loss_scale (device memory); *loss_sum stays the unscaled loss. */
+int mpa_bce_fwd_bwd_scaled_f32(const float* y_pred, const float* y_true, float* loss_sum, float* grad_pred, long long n,
+                               const float* loss_scale, void* stream);
 
 #ifdef __cplusplus
 }

@@ -495,6 +495,48 @@ __global__ void adamw_kernel(float* __restrict__ p, const float* __restrict__ g,
   }
 }
 
+// AdamW of an fp16 training step with dynamic loss scaling (torch.amp.GradScaler + torch.optim.AdamW): skipped entirely when the overflow
+// check set *found_inf; otherwise the update of adamw_kernel on g * grad_scale / *loss_scale, bias-corrected for the (*applied + 1)-th
+// applied step.  Everything the decision needs is read from device memory: no host synchronisation, the same in eager and replayed steps.
+__global__ void adamw_scaled_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m, float* __restrict__ v, long long n,
+                                    float lr, float b1, float b2, float eps, float wd, float grad_scale, const int* __restrict__ found_inf,
+                                    const float* __restrict__ loss_scale, const int* __restrict__ applied) {
+  if (*found_inf) return;
+  const float step = (float)(*applied + 1);
+  const float bc1 = 1.f - powf(b1, step), bc2_sqrt = sqrtf(1.f - powf(b2, step));
+  const float gs = grad_scale * (1.f / *loss_scale);
+  for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
+    const float gi = g[i] * gs;
+    float pi = p[i] * (1.f - lr * wd);
+    const float mi = b1 * m[i] + (1.f - b1) * gi;
+    const float vi = b2 * v[i] + (1.f - b2) * gi * gi;
+    m[i] = mi;
+    v[i] = vi;
+    const float denom = sqrtf(vi) / bc2_sqrt + eps;
+    p[i] = pi - (lr / bc1) * (mi / denom);
+  }
+}
+
+// torch.amp.GradScaler.update after the step: on an overflow the scale backs off and the growth tracker restarts; otherwise the step
+// counts as applied and, after growth_interval clean steps in a row, the scale grows (unless that would make it non-finite).
+__global__ void loss_scale_update_kernel(const int* __restrict__ found_inf, float* __restrict__ loss_scale, int* __restrict__ growth_tracker,
+                                         int* __restrict__ applied, float growth_factor, float backoff_factor, int growth_interval) {
+  if (*found_inf) {
+    *loss_scale *= backoff_factor;
+    *growth_tracker = 0;
+    return;
+  }
+  *applied += 1;
+  const int clean = *growth_tracker + 1;
+  if (clean >= growth_interval) {
+    const float grown = *loss_scale * growth_factor;
+    if (isfinite(grown)) *loss_scale = grown;
+    *growth_tracker = 0;
+  } else {
+    *growth_tracker = clean;
+  }
+}
+
 }  // namespace mpa
 
 using namespace mpa;
@@ -672,6 +714,21 @@ int mpa_adamw_f32(float* param, const float* grad, float* exp_avg, float* exp_av
   adamw_kernel<<<grid_for(n, 256), 256, 0, (cudaStream_t)stream>>>(param, grad, exp_avg, exp_avg_sq, n, lr, beta1, beta2, eps, weight_decay, bc1,
                                                                     bc2s, grad_scale);
   MPA_CHECK_LAUNCH("adamw");
+  return MPA_OK;
+}
+
+int mpa_adamw_scaled_f32(float* param, const float* grad, float* exp_avg, float* exp_avg_sq, long long n, float lr, float beta1, float beta2,
+                         float eps, float weight_decay, float grad_scale, const int* found_inf, float* loss_scale, int* growth_tracker,
+                         int* applied_steps, float growth_factor, float backoff_factor, int growth_interval, void* stream) {
+  MPA_CHECK_ARCH();
+  MPA_REQUIRE(param && grad && exp_avg && exp_avg_sq && found_inf && loss_scale && growth_tracker && applied_steps && n > 0 && growth_interval >= 1,
+              "adamw_scaled: bad argument");
+  cudaStream_t st = (cudaStream_t)stream;
+  adamw_scaled_kernel<<<grid_for(n, 256), 256, 0, st>>>(param, grad, exp_avg, exp_avg_sq, n, lr, beta1, beta2, eps, weight_decay, grad_scale,
+                                                        found_inf, loss_scale, applied_steps);
+  MPA_CHECK_LAUNCH("adamw_scaled");
+  loss_scale_update_kernel<<<1, 1, 0, st>>>(found_inf, loss_scale, growth_tracker, applied_steps, growth_factor, backoff_factor, growth_interval);
+  MPA_CHECK_LAUNCH("loss_scale_update");
   return MPA_OK;
 }
 

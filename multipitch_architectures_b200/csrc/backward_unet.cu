@@ -385,9 +385,10 @@ __global__ void tok_to_nchw_kernel(const float* __restrict__ tok, float* __restr
 }
 
 // CrossEntropyLoss(mean) * scale over K classes, target class = number of active labels of the item (PUnet degree-of-polyphony
-// head: n_target = sum(labels, -1).long(), RETRAIN4_exp195f...rerun1.py:343-345).  One warp per item.
+// head: n_target = sum(labels, -1).long(), RETRAIN4_exp195f...rerun1.py:343-345).  One warp per item.  grad_mul (optional, device
+// memory): the gradient is multiplied by *grad_mul (the loss scale of fp16 training); the loss is not.
 __global__ void __launch_bounds__(128) ce_count_kernel(const float* __restrict__ logits, const float* __restrict__ y_true, float* __restrict__ loss_sum,
-                                                       float* __restrict__ grad, int B, int K, int P, float scale) {
+                                                       float* __restrict__ grad, int B, int K, int P, float scale, const float* __restrict__ grad_mul) {
   const int b = blockIdx.x * 4 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
   if (b >= B) return;
   float cnt = 0.f;
@@ -403,9 +404,11 @@ __global__ void __launch_bounds__(128) ce_count_kernel(const float* __restrict__
   den = warp_sum(den);
   const float lse = mx + logf(den);
   if (lane == 0) atomicAdd(loss_sum, (lse - logits[(size_t)b * K + cls]) * scale / B);
-  if (grad)
+  if (grad) {
+    const float gm = grad_mul ? *grad_mul : 1.f;
     for (int k = lane; k < K; k += 32)
-      grad[(size_t)b * K + k] = (expf(logits[(size_t)b * K + k] - lse) - (k == cls ? 1.f : 0.f)) * scale / B;
+      grad[(size_t)b * K + k] = (expf(logits[(size_t)b * K + k] - lse) - (k == cls ? 1.f : 0.f)) * scale / B * gm;
+  }
 }
 
 }  // namespace mpa
@@ -551,8 +554,18 @@ int mpa_ce_count_fwd_bwd_f32(const float* logits, const float* y_true, float* lo
   MPA_CHECK_ARCH();
   MPA_REQUIRE(logits && y_true && loss_sum && B > 0 && K > 0 && P > 0, "ce_count: bad argument");
   if (!accumulate_loss) cudaMemsetAsync(loss_sum, 0, sizeof(float), (cudaStream_t)stream);
-  ce_count_kernel<<<ceil_div(B, 4), 128, 0, (cudaStream_t)stream>>>(logits, y_true, loss_sum, grad_logits, B, K, P, scale);
+  ce_count_kernel<<<ceil_div(B, 4), 128, 0, (cudaStream_t)stream>>>(logits, y_true, loss_sum, grad_logits, B, K, P, scale, nullptr);
   MPA_CHECK_LAUNCH("ce_count");
+  return MPA_OK;
+}
+
+int mpa_ce_count_fwd_bwd_scaled_f32(const float* logits, const float* y_true, float* loss_sum, float* grad_logits, int B, int K, int P, float scale,
+                                    int accumulate_loss, const float* loss_scale, void* stream) {
+  MPA_CHECK_ARCH();
+  MPA_REQUIRE(logits && y_true && loss_sum && grad_logits && loss_scale && B > 0 && K > 0 && P > 0, "ce_count_scaled: bad argument");
+  if (!accumulate_loss) cudaMemsetAsync(loss_sum, 0, sizeof(float), (cudaStream_t)stream);
+  ce_count_kernel<<<ceil_div(B, 4), 128, 0, (cudaStream_t)stream>>>(logits, y_true, loss_sum, grad_logits, B, K, P, scale, loss_scale);
+  MPA_CHECK_LAUNCH("ce_count_scaled");
   return MPA_OK;
 }
 

@@ -342,11 +342,13 @@ __global__ void bias_act_kernel(const float* __restrict__ x, const float* __rest
   }
 }
 
+// grad_mul (optional, device memory): the gradient is multiplied by *grad_mul (the loss scale of fp16 training); the loss is not
 __global__ void __launch_bounds__(256) bce_kernel(const float* __restrict__ yp, const float* __restrict__ yt, float* __restrict__ loss_sum,
-                                                  float* __restrict__ grad, long long n) {
+                                                  float* __restrict__ grad, long long n, const float* __restrict__ grad_mul) {
   __shared__ float sh[8];
   float acc = 0.f;
   const float inv_n = 1.f / (float)n;
+  const float gm = grad_mul ? *grad_mul : 1.f;
   for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
     float p = yp[i], t = yt[i];
     float lp = fmaxf(logf(p), -100.f), l1p = fmaxf(logf(1.f - p), -100.f);
@@ -354,7 +356,7 @@ __global__ void __launch_bounds__(256) bce_kernel(const float* __restrict__ yp, 
     if (grad) {
       // d/dp of the clamped loss: the clamp kills the gradient where log < -100 (torch: p clamped via eps 1e-12)
       float g = (p - t) / fmaxf(p * (1.f - p), 1e-12f);
-      grad[i] = g * inv_n;
+      grad[i] = g * inv_n * gm;
     }
   }
   float tot = block_sum(acc, sh);
@@ -529,8 +531,18 @@ int mpa_bce_fwd_bwd_f32(const float* y_pred, const float* y_true, float* loss_su
   MPA_CHECK_ARCH();
   MPA_REQUIRE(y_pred && y_true && loss_sum && n > 0, "bce: bad argument");
   cudaMemsetAsync(loss_sum, 0, sizeof(float), (cudaStream_t)stream);
-  bce_kernel<<<grid_for(n, 256), 256, 0, (cudaStream_t)stream>>>(y_pred, y_true, loss_sum, grad_pred, n);
+  bce_kernel<<<grid_for(n, 256), 256, 0, (cudaStream_t)stream>>>(y_pred, y_true, loss_sum, grad_pred, n, nullptr);
   MPA_CHECK_LAUNCH("bce");
+  return MPA_OK;
+}
+
+int mpa_bce_fwd_bwd_scaled_f32(const float* y_pred, const float* y_true, float* loss_sum, float* grad_pred, long long n, const float* loss_scale,
+                               void* stream) {
+  MPA_CHECK_ARCH();
+  MPA_REQUIRE(y_pred && y_true && loss_sum && grad_pred && loss_scale && n > 0, "bce_scaled: bad argument");
+  cudaMemsetAsync(loss_sum, 0, sizeof(float), (cudaStream_t)stream);
+  bce_kernel<<<grid_for(n, 256), 256, 0, (cudaStream_t)stream>>>(y_pred, y_true, loss_sum, grad_pred, n, loss_scale);
+  MPA_CHECK_LAUNCH("bce_scaled");
   return MPA_OK;
 }
 

@@ -204,6 +204,21 @@ __global__ void bn_stats_final_kernel(const float* __restrict__ partial, float* 
   stats[C + c] = m2 / (float)n_tot;
 }
 
+// *found = 1 when any of x[0, n) is an inf or a NaN (the loss-scale overflow check over the flat gradient of fp16 training; the caller
+// cleared the flag).  vec: x is 16-byte aligned — float4 loads over the first n / 4 * 4 elements, the ragged tail element by element.
+__global__ void __launch_bounds__(kRedThreads) nonfinite_kernel(const float* __restrict__ x, long long n, int vec, int* __restrict__ found) {
+  const long long tid = blockIdx.x * (long long)blockDim.x + threadIdx.x, stride = (long long)gridDim.x * blockDim.x;
+  const long long n4 = vec ? n >> 2 : 0;
+  bool bad = false;
+  const float4* x4 = reinterpret_cast<const float4*>(x);
+  for (long long i = tid; i < n4; i += stride) {
+    const float4 v = x4[i];
+    bad |= !isfinite(v.x) | !isfinite(v.y) | !isfinite(v.z) | !isfinite(v.w);
+  }
+  for (long long i = n4 * 4 + tid; i < n; i += stride) bad |= !isfinite(x[i]);
+  if (__syncthreads_or(bad) && threadIdx.x == 0) *found = 1;
+}
+
 // Shared with backward.cu / backward_unet.cu -------------------------------------------------------------------------------
 int channel_sum_launch(const float* x, float* out, int B, int C, int HW, cudaStream_t st) {
   float* scratch = reduce_scratch();
@@ -260,6 +275,19 @@ int bn_stats_launch(const float* x, float* stats, int B, int C, int HW, cudaStre
 using namespace mpa;
 
 extern "C" {
+
+int mpa_nonfinite_check_f32(const float* x, long long n, int* found_inf, void* stream) {
+  MPA_CHECK_ARCH();
+  MPA_REQUIRE(x && found_inf && n > 0, "nonfinite_check: bad argument");
+  cudaStream_t st = (cudaStream_t)stream;
+  cudaMemsetAsync(found_inf, 0, sizeof(int), st);
+  const int vec = ((uintptr_t)x & 15) == 0;
+  long long blocks = ((vec ? n / 4 : n) + kRedThreads - 1) / kRedThreads;
+  blocks = blocks < 1 ? 1 : (blocks > 148LL * 8 ? 148LL * 8 : blocks);        // a grid-stride loop over about 8 blocks per SM
+  nonfinite_kernel<<<(int)blocks, kRedThreads, 0, st>>>(x, n, vec, found_inf);
+  MPA_CHECK_LAUNCH("nonfinite_check");
+  return MPA_OK;
+}
 
 int mpa_channel_sum_f32(const float* x, float* out, int B, int C, int HW, void* stream) {
   MPA_CHECK_ARCH();

@@ -126,10 +126,15 @@ def bn_apply(x, stats, w, b, eps=1e-5, act=ACT_NONE, act_param=0.0):
     return out
 
 
-def bce_fwd_bwd(y_pred, y_true, want_grad=True):
+def bce_fwd_bwd(y_pred, y_true, want_grad=True, loss_scale=None):
+    """-> (mean BCE loss [1], its gradient wrt y_pred).  loss_scale: float32[1] on the device — the gradient is multiplied by it (fp16
+    training), the loss is not."""
     n = y_pred.numel()
     loss = torch.empty(1, dtype=torch.float32, device=y_pred.device)
     grad = torch.empty_like(y_pred) if want_grad else None
+    if loss_scale is not None:
+        call('bce_fwd_bwd_scaled_f32', _f32(y_pred), _f32(y_true), loss, grad, _lib.i64(n), loss_scale, stream_ptr())
+        return loss, grad
     call('bce_fwd_bwd_f32', _f32(y_pred), _f32(y_true), loss, grad, _lib.i64(n), stream_ptr())
     return loss, grad
 

@@ -10,9 +10,11 @@ Two ways in:
     — `model.forward` routes through `TrainFunction` (a torch.autograd.Function whose backward runs the tape);
   * fused: `TrainStep(model, lr=...)(x, t)` — BCE forward/backward kernel, backward, (optional) gradient all-reduce over
     NCCL on ONE flat buffer, fused AdamW; no torch operator touches an activation or a gradient.
-With `precision='bf16'` the convolutions run on the tensor cores (TcConv) and, for the models without the residual path, activations and
-gradients stay in the 16-bit CP8 planes between the block convolutions (`_cp8_resident`: pool + dropout forward / backward and the bias
-gradients are train_cp8.cu kernels; bit-identical to crossing the nchw<->CP8 converters around the fp32 kernels).
+With `precision='bf16'` or `'fp16'` the convolutions run on the tensor cores (TcConv) in that 16-bit format (`tape_fmt`) and, for the
+models without the residual path, activations and gradients stay in the 16-bit CP8 planes between the block convolutions (`_cp8_resident`:
+pool + dropout forward / backward and the bias gradients are train_cp8.cu kernels; bit-identical to crossing the nchw<->CP8 converters
+around the fp32 kernels).  fp16 cannot hold gradients as small as bf16 can, so the fused step of an fp16 model scales its loss
+(`LossScaler`, torch.amp.GradScaler's policy); drop-in fp16 training wants a torch.amp.GradScaler, as fp16 AMP always does.
 Dropout uses a Philox stream (seed, per-site offset); the reference's torch RNG stream cannot be reproduced, so parity
 tests run with p_dropout = 0 (SURVEY.md §7).
 
@@ -30,6 +32,13 @@ from .libdl.nn_models import _exec
 from ._lib import call, stream_ptr
 
 SITES_PER_STEP = 64       # dropout sites reserved per step of the CNN path: offset = step * 64 + site
+_TAPE_FMT = {'bf16': ops.FMT_BF16, 'fp16': ops.FMT_F16}
+
+
+def tape_fmt(model):
+    """16-bit operand / plane format of the tensor-core training tapes: bf16 and fp16 models; None for the others (fp32, and fp16x3,
+    which trains on the fp32 tape)."""
+    return _TAPE_FMT.get(getattr(model, 'precision', 'fp32'))
 
 
 class StepState:
@@ -162,17 +171,16 @@ def _wgrad(conv, x, g, gw, gb):
 
 
 def _rows_tc_eligible(model, conv, x):
-    """The head's full-height 75x1 convolution of a bf16 model with more than 10 output channels: forward and both gradients as tcgen05
+    """The head's full-height 75x1 convolution of a bf16 / fp16 model with more than 10 output channels: forward and both gradients as tcgen05
     GEMMs.  Thinner ones (CNN:XS 20 -> 10, DRCNN 30 -> 10) are HBM-bound matrix-vector products and stay on the conv_rows_thin_* kernels (the
     tensor-core form was measured at batch 256: 3.39 -> 3.48 ms per CNN:XS step — two operand-chunking passes over x outweigh the GEMMs)."""
-    return (getattr(model, 'precision', 'fp32') == 'bf16' and _is_rows_conv(conv, x.shape[2])
+    return (tape_fmt(model) is not None and _is_rows_conv(conv, x.shape[2])
             and conv.weight.shape[0] > 10 and x.shape[3] % 8 == 0 and conv.bias is not None)
 
 
-def _rows_tc_forward(conv, x, act, a):
-    """Y[b][co][w] = act(sum_k W[co][k] x[b][k][w] + bias[co]), k = (ci, frame): tokens (b, w) x K on the tensor cores (bf16 operands, fp32
-    accumulate, K slices in atomics), then bias + activation in place."""
-    fm = ops.FMT_BF16
+def _rows_tc_forward(conv, x, act, a, fm=ops.FMT_BF16):
+    """Y[b][co][w] = act(sum_k W[co][k] x[b][k][w] + bias[co]), k = (ci, frame): tokens (b, w) x K on the tensor cores (16-bit operands of
+    format fm, fp32 accumulate, K slices in atomics), then bias + activation in place."""
     B, Cin, H, W = x.shape
     Cout, K, Mt = conv.weight.shape[0], Cin * H, B * W
     xf = ops.strided_chunks(x, Mt, K, 256, fm, (W, K * W, 1), (K, 0, W))
@@ -183,10 +191,9 @@ def _rows_tc_forward(conv, x, act, a):
     return y
 
 
-def _rows_tc_backward(conv, x, g, gw, gb, need_dx):
+def _rows_tc_backward(conv, x, g, gw, gb, need_dx, fm=ops.FMT_BF16):
     """g: gradient wrt the convolution output (activation already differentiated away).  Weight gradient [Cout][K] = g^T x over the B*W
     tokens, data gradient [b][k][w] = W^T g written straight into NCHW."""
-    fm = ops.FMT_BF16
     B, Cin, H, W = x.shape
     Cout, K, Mt = conv.weight.shape[0], Cin * H, B * W
     def wgrad():
@@ -251,7 +258,7 @@ def _pool_bwd(a_in, g_pool, k, act, a):
 
 
 class TcConv:
-    """bf16 tensor-core forward / backward of a stride-1 'same' nn.Conv2d inside the fp32 NCHW training graph:
+    """bf16 / fp16 tensor-core forward / backward of a stride-1 'same' nn.Conv2d inside the fp32 NCHW training graph:
     forward = mpa_conv_tc_f16 on CP8 planes, data gradient = the same kernel with the transposed / flipped weights, weight gradient =
     mpa_conv_wgrad_tc, bias gradient = a channel reduction.  Activations and gradients cross the boundary through nchw<->CP8 converters
     (16-bit operands, fp32 accumulation; the optimiser state and every element-wise stage stay fp32)."""
@@ -260,7 +267,7 @@ class TcConv:
     @staticmethod
     def eligible(model, conv, F):
         KH, KW = conv.kernel_size
-        return (getattr(model, 'precision', 'fp32') == 'bf16' and tuple(conv.stride) == (1, 1) and KH % 2 == 1 and KW % 2 == 1 and 3 <= KW <= 15 and KH >= 3
+        return (tape_fmt(model) is not None and tuple(conv.stride) == (1, 1) and KH % 2 == 1 and KW % 2 == 1 and 3 <= KW <= 15 and KH >= 3
                 and tuple(conv.padding) == (KH // 2, KW // 2) and F + TcConv.PF + 15 < 272 and conv.bias is not None)
 
     @classmethod
@@ -312,16 +319,15 @@ class TcConv:
         return z
 
     @classmethod
-    def forward(cls, tag, conv, x, act, a):
-        fmt = ops.FMT_BF16
+    def forward(cls, tag, conv, x, act, a, fmt=ops.FMT_BF16):
         B, Cin, T, F = x.shape
         xc = ops.nchw_to_cp8(x, out=cls._buf(tag + ':x', B, Cin, T, F, x.device, fmt), fmt=fmt)
         return ops.cp8_to_nchw(cls.forward_cp8(tag, conv, xc, act, a)), xc
 
     @classmethod
     def forward_cp8(cls, tag, conv, xc, act, a):
-        """CP8 in -> CP8 out (pooled buffer `tag:y`)."""
-        fmt = ops.FMT_BF16
+        """CP8 in -> CP8 out (pooled buffer `tag:y`, in the format of xc)."""
+        fmt = xc.fmt
         B, Cin, T, F = xc.B, xc.C, xc.T, xc.F
         Cout, _, KH, KW = conv.weight.shape
         yc = cls._buf(tag + ':y', B, Cout, T, F, xc.buf.device, fmt)
@@ -335,7 +341,7 @@ class TcConv:
     @classmethod
     def backward(cls, tag, conv, xc, g, gw, gb, need_dx):
         """g: fp32 gradient wrt the convolution output (before the activation has been differentiated away by the caller)."""
-        fmt = ops.FMT_BF16
+        fmt = xc.fmt
         B, Cout, T, F = g.shape
         gc = ops.nchw_to_cp8(g, out=cls._buf(tag + ':g', B, Cout, T, F, g.device, fmt), fmt=fmt)
         ops.channel_sum(g, out=gb)
@@ -346,7 +352,7 @@ class TcConv:
     def backward_cp8(cls, tag, conv, xc, gc, gw, gb, need_dx):
         """gc: CP8 gradient wrt the convolution output; -> CP8 gradient wrt its input (pooled buffer `tag:gx`).  gb (optional): bias
         gradient summed from the 16-bit planes."""
-        fmt = ops.FMT_BF16
+        fmt = gc.fmt
         B, Cout, T, F = gc.B, gc.C, gc.T, gc.F
         _, Cin, KH, KW = conv.weight.shape
         dev = gc.buf.device
@@ -368,15 +374,14 @@ class TcConv:
 def _tc_s3_eligible(model, conv, F):
     """The head's 3x3 / stride (1,3) / pad (1,0) convolution (basic_cnns.py:391) = the stride-1 'same' 3x3 convolution sampled at
     columns 1, 4, 7, ... ; its backward is the stride-1 backward of the zero-inserted output gradient."""
-    return (getattr(model, 'precision', 'fp32') == 'bf16' and tuple(conv.kernel_size) == (3, 3) and tuple(conv.stride) == (1, 3)
+    return (tape_fmt(model) is not None and tuple(conv.kernel_size) == (3, 3) and tuple(conv.stride) == (1, 3)
             and tuple(conv.padding) == (1, 0) and F % 3 == 0 and F + TcConv.PF + 15 < 272 and conv.bias is not None)
 
 
-def _tc_s3_forward(tag, conv, x, act, a):
-    """x: fp32 NCHW or the CP8 planes a preceding CP8-resident block left behind."""
-    fmt = ops.FMT_BF16
+def _tc_s3_forward(tag, conv, x, act, a, fmt=ops.FMT_BF16):
+    """x: fp32 NCHW (converted to fmt planes) or the CP8 planes a preceding CP8-resident block left behind."""
     if isinstance(x, ops.CP8):
-        xc = x
+        xc, fmt = x, x.fmt
     else:
         B, Cin, T, F = x.shape
         xc = ops.nchw_to_cp8(x, out=TcConv._buf(tag + ':x', B, Cin, T, F, x.device, fmt), fmt=fmt)
@@ -392,7 +397,7 @@ def _tc_s3_forward(tag, conv, x, act, a):
 
 
 def _tc_s3_backward(tag, conv, xc, g, gw, gb, keep_cp8=False):
-    fmt = ops.FMT_BF16
+    fmt = xc.fmt
     B, Cout, T, Fo = g.shape
     Cin, F = conv.weight.shape[1], xc.F
     gc = TcConv._buf(tag + ':g3', B, Cout, T, F, g.device, fmt)
@@ -468,7 +473,7 @@ LN_PIXEL = True
 
 
 def _cp8_resident(model, blocks, F):
-    """bf16 mode, no residual path: activations and gradients stay in the CP8 planes between the convolutions of the blocks
+    """bf16 / fp16 mode, no residual path: activations and gradients stay in the CP8 planes between the convolutions of the blocks
     (pool + dropout forward / backward and the bias gradients run on the planes, train_cp8.cu)."""
     return (CP8_RESIDENT and not getattr(model, 'residual', False) and F % 4 == 0 and all(TcConv.eligible(model, c, F) for _, c in blocks)
             and _tc_s3_eligible(model, model.conv2[0], F))
@@ -523,10 +528,11 @@ class Tape:
         return out
 
     def conv(self, name, conv, x, act=ops.ACT_NONE, a=0.0, need_dx=True, rows_tc=True):
-        """Conv2d (+ bias, + fused pointwise activation); stride-1 'same' convolutions of a bf16 model run on the tensor cores, and so do
-        full-height ones with more than 10 output channels unless rows_tc is False (_rows_tc_eligible)."""
+        """Conv2d (+ bias, + fused pointwise activation); stride-1 'same' convolutions of a bf16 / fp16 model run on the tensor cores, and so
+        do full-height ones with more than 10 output channels unless rows_tc is False (_rows_tc_eligible)."""
+        fmt = tape_fmt(self.model)
         if TcConv.eligible(self.model, conv, x.d.shape[3]) and x.d.shape[2] >= 2:
-            y, xc = TcConv.forward(name, conv, x.d, act, a)
+            y, xc = TcConv.forward(name, conv, x.d, act, a, fmt)
             out = Node(y)
 
             def bwd_tc():
@@ -537,11 +543,11 @@ class Tape:
             self.push(bwd_tc)
             return out
         if rows_tc and _rows_tc_eligible(self.model, conv, x.d):
-            out = Node(_rows_tc_forward(conv, x.d, act, a))
+            out = Node(_rows_tc_forward(conv, x.d, act, a, fmt))
 
             def bwd_rows():
                 g = out.g if act == ops.ACT_NONE else _act_bwd(out.d, out.g, act, a)
-                gx = _rows_tc_backward(conv, x.d, g, self.grads[name + '.weight'], self.grads[name + '.bias'], need_dx)
+                gx = _rows_tc_backward(conv, x.d, g, self.grads[name + '.weight'], self.grads[name + '.bias'], need_dx, fmt)
                 if need_dx:
                     x.acc(gx)
             self.push(bwd_rows)
@@ -593,7 +599,7 @@ class Tape:
         """CNN block on fp32 NCHW: Conv2d (tensor cores behind the nchw<->CP8 converters when TcConv is eligible) -> LeakyReLU ->
         MaxPool((3,1)) -> dropout (+ x when `residual`)."""
         if TcConv.eligible(self.model, conv, x.d.shape[3]):
-            act, xc = TcConv.forward(name, conv, x.d, ops.ACT_LRELU, a)
+            act, xc = TcConv.forward(name, conv, x.d, ops.ACT_LRELU, a, tape_fmt(self.model))
         else:
             act, xc = _conv_fwd(conv, x.d, ops.ACT_LRELU, a), None
         off = self._take_site()
@@ -643,7 +649,7 @@ class Tape:
         if split:
             y, xc = _tc_s3_forward_split(name, conv, x.d, ops.ACT_LRELU, a)
         elif planes or _tc_s3_eligible(self.model, conv, x.d.shape[3]):
-            y, xc = _tc_s3_forward(name, conv, x.d, ops.ACT_LRELU, a)
+            y, xc = _tc_s3_forward(name, conv, x.d, ops.ACT_LRELU, a, tape_fmt(self.model))
         else:
             y, xc = _conv_fwd(conv, x.d, ops.ACT_LRELU, a), None
         off = self._take_site()
@@ -677,7 +683,7 @@ class Tape:
 def note_fp32_tape(model):
     """An eval-mode backward of a tensor-core model that runs on the fp32 NCHW tape says so, once per model class."""
     prec = getattr(model, 'precision', 'fp32')
-    if prec == 'bf16':
+    if tape_fmt(model) is not None:
         _exec.note_path(model, 'eval-mode backward runs on the fp32 NCHW training tape (tensor-core convolutions behind nchw<->CP8 converters), '
                                'not on the CP8-resident tape')
     elif prec in _exec.TC_PRECISIONS:
@@ -687,7 +693,7 @@ def note_fp32_tape(model):
 
 def cnn_train_forward(model, x, grads, seed=0, step=0, need_input_grad=False, frozen_bn=False):
     """-> (y_pred Node [B,1,T-74,72], None, tape).  Train mode: dropout active when model.p_dropout > 0; eval mode: dropout off.  bf16 models
-    without the residual path keep the block activations and gradients on the CP8 planes (_cp8_resident).  need_input_grad: the tape also
+    (and fp16) without the residual path keep the block activations and gradients on the CP8 planes (_cp8_resident).  need_input_grad: the tape also
     leaves the gradient wrt x in tape.input_grad.  frozen_bn: accepted for the common builder signature (the CNN family has no BatchNorm)."""
     a, p = model.a_lrelu, (model.p_dropout if model.training else 0.0)
     tp = Tape(grads, seed, step, SITES_PER_STEP, model, need_input_grad, frozen_bn)
@@ -695,7 +701,7 @@ def cnn_train_forward(model, x, grads, seed=0, step=0, need_input_grad=False, fr
     B, C, T, F = x.shape
     split = 0
     if _cp8_resident(model, blocks, F) and C <= 8:
-        z = tp.layernorm_cf_cp8(model.layernorm, x, TcConv._buf(blocks[0][0] + '.0:x', B, C, T, F, x.device, ops.FMT_BF16))
+        z = tp.layernorm_cf_cp8(model.layernorm, x, TcConv._buf(blocks[0][0] + '.0:x', B, C, T, F, x.device, tape_fmt(model)))
         split = 3 if _s3_split_eligible(model, model.conv2[0], F) else 0
         for i, (name, conv) in enumerate(blocks):
             z = tp.block_cp8(name + '.0', conv, z, p, a, split if i == len(blocks) - 1 else 0)
@@ -745,11 +751,35 @@ def forward_train(build, model, x):
     return TrainFunction.apply(build, model, x, seed, model._train_calls, *[p for _, p in model.named_parameters()])
 
 
+class LossScaler:
+    """Dynamic loss scale of an fp16 fused step, with torch.amp.GradScaler's policy and defaults: the loss gradient is multiplied by `scale`
+    (2^16 at first); a step whose all-reduced flat gradient holds an inf or a NaN is skipped and halves the scale; `growth_interval` clean
+    steps in a row double it.  The state lives in device memory — the scale, the growth tracker (clean steps since the scale last changed),
+    the found-inf flag of the last step and the number of applied steps, from which AdamW's bias correction is formed (a skipped step does
+    not count, as torch.optim leaves state['step'] alone) — so a step needs no host synchronisation, and eager and graph-replayed steps
+    behave the same."""
+
+    def __init__(self, dev, init_scale=2.0 ** 16, growth_factor=2.0, backoff_factor=0.5, growth_interval=2000):
+        self.scale = torch.full((1,), float(init_scale), dtype=torch.float32, device=dev)
+        self.growth_tracker = torch.zeros(1, dtype=torch.int32, device=dev)
+        self.found_inf = torch.zeros(1, dtype=torch.int32, device=dev)
+        self.applied_steps = torch.zeros(1, dtype=torch.int32, device=dev)
+        self.growth_factor, self.backoff_factor, self.growth_interval = growth_factor, backoff_factor, growth_interval
+
+    def adamw(self, step, grad_scale):
+        """The overflow check over step.flat_g, then AdamW on the unscaled gradient (or nothing on an overflow), then the scale update."""
+        n = _lib.i64(step.flat_p.numel())
+        call('nonfinite_check_f32', step.flat_g, n, self.found_inf, stream_ptr())
+        call('adamw_scaled_f32', step.flat_p, step.flat_g, step.m, step.v, n, float(step.lr), float(step.betas[0]), float(step.betas[1]),
+             float(step.eps), float(step.wd), float(grad_scale), self.found_inf, self.scale, self.growth_tracker, self.applied_steps,
+             float(self.growth_factor), float(self.backoff_factor), int(self.growth_interval), stream_ptr())
+
+
 class FusedTrainStep:
     """Fused training step on flat parameter / gradient / moment buffers: the forward the subclass's builder records on a Tape, BCE (+ CE
     when the builder returns a count prediction: UnetTrainStep's `ce_scale`), the tape's backward, ONE gradient all-reduce (NCCL, when a
     process group is active), fused AdamW.  A subclass supplies `sites_per_step` and `build`; one whose parameters start with an encoder
-    trunk sets `n_trunk` (UnetTrainStep)."""
+    trunk sets `n_trunk` (UnetTrainStep).  An fp16 model's step scales its loss dynamically (`scaler`, a LossScaler; None otherwise)."""
     sites_per_step = None
     build = None          # (model, x, grads, seed, step) -> (y Node, n_pred Node or None, Tape)
 
@@ -780,16 +810,27 @@ class FusedTrainStep:
         self.comm_events = None                        # bench.py: a list that receives CUDA events around the all-reduce
         self._state = StepState(dev, self.sites_per_step)
         self._tape = None
+        self.scaler = LossScaler(dev) if getattr(model, 'precision', 'fp32') == 'fp16' else None
+
+    @property
+    def loss_scale(self):
+        """The current loss scale (read from the device), or None when this step does not scale its loss."""
+        return None if self.scaler is None else float(self.scaler.scale.item())
 
     def _forward_backward(self, x, target, tape_step, split):
         """-> loss (the step state is active).  split: stop the backward at the trunk (its part follows in _trunk_backward)."""
         y, n_pred, tape = self.build(self.model, x, self.grads, self.seed, tape_step)
         target = target.contiguous()
-        loss, y.g = ops.bce_fwd_bwd(y.d, target)
+        ls = None if self.scaler is None else self.scaler.scale
+        loss, y.g = ops.bce_fwd_bwd(y.d, target, loss_scale=ls)
         if n_pred is not None:
             B, K = n_pred.d.shape[0], n_pred.d.shape[1]
             n_pred.g = torch.empty_like(n_pred.d)
-            call('ce_count_fwd_bwd_f32', n_pred.d, target, loss, n_pred.g, B, K, target.numel() // B, float(self.ce_scale), 1, stream_ptr())
+            if ls is None:
+                call('ce_count_fwd_bwd_f32', n_pred.d, target, loss, n_pred.g, B, K, target.numel() // B, float(self.ce_scale), 1, stream_ptr())
+            else:
+                call('ce_count_fwd_bwd_scaled_f32', n_pred.d, target, loss, n_pred.g, B, K, target.numel() // B, float(self.ce_scale), 1, ls,
+                     stream_ptr())
         if split:
             tape.backward(lo=tape.trunk_mark)
             self._tape = tape
@@ -868,8 +909,11 @@ class FusedTrainStep:
                     e1.record()
                     ev.append((e0, e1))
                 scale = 1.0 / dist.get_world_size(self.group)
-            call('adamw_f32', self.flat_p, self.flat_g, self.m, self.v, _lib.i64(self.flat_p.numel()), float(self.lr), float(self.betas[0]),
-                 float(self.betas[1]), float(self.eps), float(self.wd), self.step_count, float(scale), stream_ptr())
+            if self.scaler is not None:            # every rank checks the same summed gradient: all ranks skip together
+                self.scaler.adamw(self, scale)
+            else:
+                call('adamw_f32', self.flat_p, self.flat_g, self.m, self.v, _lib.i64(self.flat_p.numel()), float(self.lr), float(self.betas[0]),
+                     float(self.betas[1]), float(self.eps), float(self.wd), self.step_count, float(scale), stream_ptr())
         # the raw-pointer AdamW leaves data_ptr / _version unchanged: every ParamCache of the module tree (model, encoder layers, BLSTM
         # layers) is stale now
         _exec.invalidate_caches(self.model)

@@ -20,8 +20,8 @@ import torch
 from . import _lib, ops
 from ._lib import call, stream_ptr
 from .libdl.nn_models import _exec
-from .training import (FusedTrainStep, Node, Tape, TcConv, ctypes_u64, note_fp32_tape, _act_bwd, _add, _s3_split_eligible, _split_buf, _step_args,
-                       _tc_s3_eligible)
+from .training import (FusedTrainStep, Node, Tape, TcConv, ctypes_u64, note_fp32_tape, tape_fmt, _act_bwd, _add, _s3_split_eligible, _split_buf,
+                       _step_args, _tc_s3_eligible)
 
 SITES_PER_STEP = 256      # dropout sites reserved per step of the U-Net tape: offset = step * 256 + site
 
@@ -93,7 +93,7 @@ class UnetTape(Tape):
         self.push(bwd)
         return out
 
-    # ---------------------------------------------------------------------------------------------- CP8-resident stages (bf16)
+    # ---------------------------------------------------------------------------------------------- CP8-resident stages (bf16 / fp16)
     # Nodes whose .d / .g are ops.CP8 planes: between two tensor-core convolutions nothing leaves the 16-bit planes (train_unet_cp8.cu).
     # Every such node has ONE consumer, except the skip connections (max-pool + concat), whose two gradients meet in maxpool_cp8's backward.
     def conv_cp8(self, name, conv, x, need_dx=True):
@@ -316,13 +316,13 @@ class UnetTape(Tape):
             self.push(bwd_ln1)
 
         # -- MLP
-        tc_mlp = self.model is not None and getattr(self.model, 'precision', 'fp32') == 'bf16'
+        fm = tape_fmt(self.model)
+        tc_mlp = fm is not None
         if tc_mlp:
-            # Both Linear layers and the four products of their backward on the tensor cores (bf16 operands, fp32 accumulate).  The hidden
+            # Both Linear layers and the four products of their backward on the tensor cores (16-bit operands, fp32 accumulate).  The hidden
             # activation [M, mlp_dim] and its gradient exist ONLY as 16-bit operand-layout copies written by the GEMM epilogues
             # (token-chunked for the weight-gradient products, feature-chunked for the next layer): no fp32 round trip, no converter pass,
             # ReLU backward and the bias gradient inside the epilogue (mpa_gemm_tc_ex_f16).
-            fm = ops.FMT_BF16
             Mp, KCt, rows_t, Np8 = (M + 255) // 256 * 256, (M + 63) // 64 * 8, (Dm + 255) // 256 * 256, (Dm + 127) // 128 * 16
             hid_tok = TcConv._raw(name + ':hid_tok', KCt * rows_t * 16, True, dev)
             hid_feat = TcConv._raw(name + ':hid_feat', Np8 * Mp * 16, False, dev)
@@ -445,9 +445,9 @@ CP8_TAPE = True            # test knob: False = the fp32 NCHW tape with converte
 
 
 def cp8_tape_eligible(model, x):
-    """bf16 U-Net / SAUnet whose every double_conv convolution runs on the tensor cores with whole channel chunks: the training step keeps
+    """bf16 / fp16 U-Net / SAUnet whose every double_conv convolution runs on the tensor cores with whole channel chunks: the training step keeps
     activations and gradients on the CP8 planes between the convolutions."""
-    if not CP8_TAPE or getattr(model, 'precision', 'fp32') != 'bf16':
+    if not CP8_TAPE or tape_fmt(model) is None:
         return False
     if hasattr(model, 'convP') or hasattr(model, 'attention3') or getattr(model, 'lstm_depth', 0) > 0:
         return False
@@ -467,7 +467,7 @@ def _unet_train_forward_cp8(model, x, grads, seed, step, need_input_grad=False, 
     """The CP8-resident tape: LayerNorm -> planes -> [conv -> BN stats -> BN+ReLU]* with max-pool / up-sampling / concat on the planes ->
     (encoder layers in fp32 tokens) -> head conv2 on the planes -> fp32 72-bin head."""
     p = model.p_dropout if model.training else 0.0
-    fmt = ops.FMT_BF16
+    fmt = tape_fmt(model)
     tp = UnetTape(grads, seed, step, SITES_PER_STEP, model, need_input_grad, frozen_bn)
     B, C, T, F = x.shape
     dev = x.device
