@@ -285,6 +285,10 @@ int mpa_conv_tc_pack_weights_split_dev(const float* w_dev, void* packed_dev, int
 size_t mpa_conv_tc_pack_table_bytes(int n_jobs);
 int mpa_conv_tc_pack_table_build(const mpa_pack_job* jobs, int n_jobs, void* table_host);
 int mpa_conv_tc_pack_weights_multi(const void* table_dev, int n_jobs, int n_blocks, void* stream);
+/* MPA_FMT_F16X3 jobs (split == 0; the same x3 layout as mpa_conv_tc_pack_weights, with the transposed / flipped weights for transpose_flip)
+ * need their per-channel scales first: this launch writes them for every x3 job of the table and must precede mpa_conv_tc_pack_weights_multi
+ * (a table without x3 jobs does not need it).  mpa_conv_tc_pack_weights_dev / _split_dev with MPA_FMT_F16X3 issue both launches. */
+int mpa_conv_tc_pack_scales_multi(const void* table_dev, int n_jobs, void* stream);
 /* HOST functions: un-duplicated weight pieces for weights_layout 1 (one filter row per piece; Cout a multiple of 8). */
 size_t mpa_conv_tc_ring_packed_bytes(int Cin, int Cout, int KH, int KW, int J);
 int mpa_conv_tc_ring_pack_weights(const float* w_host, void* packed_host, int Cin, int Cout, int KH, int KW, int fmt, int J);
@@ -313,7 +317,8 @@ int mpa_upsample2x_cp8(const void* low_cp8, void* out_cp8, int n, int C, int Tl,
 int mpa_nchw_to_cp8(const float* x, void* out_cp8, int B, int C, int T, int F, int pitch, int pf, int pt, int fmt,
                     int ncs_out, void* stream);
 /* x [B][C][T][Fs] fp32 -> CP8 planes of width F with source column f on column offset + f*stride; the other real columns are NOT
- * written (they must hold the zeros of the initial allocation): zero-inserted gradient of a stride-(1,stride) convolution. */
+ * written (they must hold the zeros of the initial allocation): zero-inserted gradient of a stride-(1,stride) convolution.
+ * MPA_FMT_F16X3 writes hi and lo planes (even ncs_out; 0 = 2 * ceil(C/8)); the columns not written stay zero in both halves. */
 int mpa_nchw_to_cp8_strided(const float* x, void* out_cp8, int B, int C, int T, int Fs, int F, int stride, int offset, int pitch,
                             int pf, int pt, int fmt, int ncs_out, void* stream);
 int mpa_cp8_to_nchw(const void* in_cp8, float* out, int B, int C, int T, int F, int pitch, int pf, int pt, int fmt,
@@ -597,6 +602,12 @@ int mpa_gemm_tc_strided_to_chunks(const float* x, void* out_chunks, int rows, in
 int mpa_conv_wgrad_tc(const void* x_cp8, const void* g_cp8, const void* zero_row, float* gw, int n_items, int Cin, int Cout, int T,
                       int F, int KH, int KW, int pitch, int pf, int pt, int x_nc_stride, int g_nc_stride, int Cin_total, int ci0,
                       int Cout_total, int co0, int fmt, void* stream);
+/* The same weight gradient in split precision: x / g are MPA_FMT_F16X3 planes (hi planes in the first half of each item's chunk stride, lo
+ * planes in the second; the strides must be even, 0 = 2 * ceil(C/8)); three MMA passes per K step, g_hi.x_hi + g_lo.x_hi + g_hi.x_lo, into
+ * one fp32 accumulator.  KW >= 3 (there is no KW == 1 form).  Other arguments and conditions as mpa_conv_wgrad_tc. */
+int mpa_conv_wgrad_tc_x3(const void* x_cp8, const void* g_cp8, const void* zero_row, float* gw, int n_items, int Cin, int Cout, int T,
+                         int F, int KH, int KW, int pitch, int pf, int pt, int x_nc_stride, int g_nc_stride, int Cin_total, int ci0,
+                         int Cout_total, int co0, void* stream);
 /* out[c] = sum_{b,hw} x[b][c][hw] (bias gradient of a convolution). */
 int mpa_channel_sum_f32(const float* x, float* out, int B, int C, int HW, void* stream);
 

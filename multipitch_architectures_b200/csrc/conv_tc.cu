@@ -1065,7 +1065,8 @@ __global__ void nchw_to_cp8_kernel(const float* __restrict__ x, uint16_t* __rest
 }
 
 // x [B][C][T][Fs] -> CP8 planes of width F: source column f lands on column offset + f*stride (every other real column keeps the
-// zero it was initialised with): the zero-inserted gradient of a stride-(1,s) convolution evaluated as a sub-sampled stride-1 one
+// zero it was initialised with): the zero-inserted gradient of a stride-(1,s) convolution evaluated as a sub-sampled stride-1 one.
+// MPA_FMT_F16X3 writes the hi plane and, NCs/2 chunks further, the lo plane of each chunk.
 __global__ void nchw_to_cp8_strided_kernel(const float* __restrict__ x, uint16_t* __restrict__ out, long long total, int C, int T, int Fs, int NCk,
                                            int NCs, int TP, int P, int pf, int pt, int fmt, int stride, int offset) {
   const bool small = total < (1ll << 31);
@@ -1073,13 +1074,27 @@ __global__ void nchw_to_cp8_strided_kernel(const float* __restrict__ x, uint16_t
     int f, t, ck;
     long long b;
     decode_ftcb(i, small, Fs, T, NCk, f, t, ck, b);
+    const long long col = pf + offset + (long long)f * stride;
     __align__(16) uint16_t v[8];
+    if (fmt == MPA_FMT_F16X3) {
+      __align__(16) uint16_t lo[8];
+#pragma unroll
+      for (int e = 0; e < 8; ++e) {
+        const int c = ck * 8 + e;
+        const float xv = c < C ? x[(((size_t)b * C + c) * T + t) * Fs + f] : 0.f;
+        v[e] = split16(xv, 0);
+        lo[e] = split16(xv, 1);
+      }
+      *reinterpret_cast<uint4*>(out + ((((size_t)b * NCs + ck) * TP + pt + t) * P + col) * 8) = *reinterpret_cast<uint4*>(v);
+      *reinterpret_cast<uint4*>(out + ((((size_t)b * NCs + NCs / 2 + ck) * TP + pt + t) * P + col) * 8) = *reinterpret_cast<uint4*>(lo);
+      continue;
+    }
 #pragma unroll
     for (int e = 0; e < 8; ++e) {
       int c = ck * 8 + e;
       v[e] = cvt16(c < C ? x[(((size_t)b * C + c) * T + t) * Fs + f] : 0.f, fmt);
     }
-    *reinterpret_cast<uint4*>(out + ((((size_t)b * NCs + ck) * TP + pt + t) * P + pf + offset + f * stride) * 8) = *reinterpret_cast<uint4*>(v);
+    *reinterpret_cast<uint4*>(out + ((((size_t)b * NCs + ck) * TP + pt + t) * P + col) * 8) = *reinterpret_cast<uint4*>(v);
   }
 }
 
@@ -1420,7 +1435,10 @@ __global__ void upsample2x_x3_kernel(const uint4* __restrict__ low, uint4* __res
 // change every step.  transpose_flip: pack the DATA-GRADIENT convolution w'[co'][ci'][kh][kw] = w[ci'][co'][KH-1-kh][KW-1-kw].
 __device__ __forceinline__ void pack_weights_range(const float* __restrict__ w, uint16_t* __restrict__ out, long long total, int Cin, int Cout,
                                                    int KH, int KW, int J, int NC, int mpr, int fmt, int transpose_flip, int Cout_total, int co0,
-                                                   long long first, long long step, int split = 0, int C0 = 0) {
+                                                   long long first, long long step, int split = 0, int C0 = 0,
+                                                   const float* __restrict__ inv = nullptr) {
+  // MPA_FMT_F16X3 (inv = the 128 inverse channel scales already written by pack_scales_range): the layout of mpa_conv_tc_pack_weights, three
+  // tile passes per filter row (W_hi, W_lo, W_hi) of the scaled weights
   // one thread per 16-byte group = the 8 input channels of one (tile row, K slice): the position is decoded once per group and the group
   // leaves as one 16-byte store; the all-zero groups of the shifted row blocks (j >= J, filter row outside [0, KH)) touch no weight.
   // (One thread per 16-bit element: 134 us per SAUnet:L training step for ~25 M elements, bound by the index arithmetic.)
@@ -1481,15 +1499,62 @@ __device__ __forceinline__ void pack_weights_range(const float* __restrict__ w, 
       }
     }
     uint32_t h[4];
+    if (fmt == MPA_FMT_F16X3) {
+      const float sc = 1.f / inv[co];                   // a power of two: exact
+      uint32_t l[4];
+#pragma unroll
+      for (int e = 0; e < 8; ++e) {
+        const float ws = __fmul_rn(v[e], sc);
+        const __half hi = __float2half_rn(ws);
+        const uint32_t hb = __half_as_ushort(hi), lb = __half_as_ushort(__float2half_rn(__fsub_rn(ws, __half2float(hi))));
+        if (e & 1) { h[e >> 1] |= hb << 16; l[e >> 1] |= lb << 16; }
+        else { h[e >> 1] = hb; l[e >> 1] = lb; }
+      }
+      const long long g3 = (tile / mpr * 3 * mpr + q) * 256 + (g & 255), pass = (long long)mpr * 256;
+      *reinterpret_cast<uint4*>(out + g3 * 8) = make_uint4(h[0], h[1], h[2], h[3]);
+      *reinterpret_cast<uint4*>(out + (g3 + pass) * 8) = make_uint4(l[0], l[1], l[2], l[3]);
+      *reinterpret_cast<uint4*>(out + (g3 + 2 * pass) * 8) = make_uint4(h[0], h[1], h[2], h[3]);
+      continue;
+    }
 #pragma unroll
     for (int e = 0; e < 4; ++e) h[e] = (uint32_t)cvt16(v[2 * e], fmt) | ((uint32_t)cvt16(v[2 * e + 1], fmt) << 16);
     *reinterpret_cast<uint4*>(out + g * 8) = make_uint4(h[0], h[1], h[2], h[3]);
   }
 }
+// MPA_FMT_F16X3: the per-packed-channel inverse scales of mpa_conv_tc_pack_weights (max |w| of the channel's row scaled into [256, 512) by a
+// power of two, exponent clamped to +-60; 1 for empty and padded channels), one warp per channel, written after the three tile passes.
+// transpose_flip: the packed channel co0 + co is the forward weight's input channel; its row runs over the Cin forward output channels.
+__device__ __forceinline__ void pack_scales_range(const float* __restrict__ w, float* __restrict__ inv, int Cin, int Cout, int KH, int KW,
+                                                  int transpose_flip, int Cout_total, int co0, int warp, int n_warps) {
+  const int lane = threadIdx.x & 31, K2 = KH * KW;
+  for (int co = warp; co < 128; co += n_warps) {
+    float m = 0.f;
+    if (co < Cout && co0 + co < Cout_total)
+      for (int i = lane; i < Cin * K2; i += 32) {
+        const int ci = i / K2, k = i - ci * K2;
+        m = fmaxf(m, fabsf(transpose_flip ? w[((size_t)ci * Cout_total + co0 + co) * K2 + k] : w[((size_t)(co0 + co) * Cin + ci) * K2 + k]));
+      }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
+    int e = 0;
+    if (m > 0.f && m < 3.0e38f) {
+      frexpf(m, &e);
+      e = 9 - e;
+      e = e > 60 ? 60 : (e < -60 ? -60 : e);
+    }
+    if (lane == 0) inv[co] = ldexpf(1.f, -e);
+  }
+}
+__global__ void pack_scales_kernel(const float* __restrict__ w, float* __restrict__ inv, int Cin, int Cout, int KH, int KW, int transpose_flip,
+                                   int Cout_total, int co0) {
+  pack_scales_range(w, inv, Cin, Cout, KH, KW, transpose_flip, Cout_total, co0, (blockIdx.x * blockDim.x + threadIdx.x) >> 5,
+                    (gridDim.x * blockDim.x) >> 5);
+}
 __global__ void pack_weights_kernel(const float* __restrict__ w, uint16_t* __restrict__ out, long long total, int Cin, int Cout, int KH, int KW,
                                     int J, int NC, int mpr, int fmt, int transpose_flip, int Cout_total, int co0, int split, int C0) {
   pack_weights_range(w, out, total, Cin, Cout, KH, KW, J, NC, mpr, fmt, transpose_flip, Cout_total, co0,
-                     blockIdx.x * (long long)blockDim.x + threadIdx.x, (long long)gridDim.x * blockDim.x, split, C0);
+                     blockIdx.x * (long long)blockDim.x + threadIdx.x, (long long)gridDim.x * blockDim.x, split, C0,
+                     fmt == MPA_FMT_F16X3 ? reinterpret_cast<const float*>(out + 3 * total) : nullptr);
 }
 // Every packed operand of a training step (forward and data-gradient tiles of all convolutions) in ONE launch: blockIdx.y = job of a
 // device-resident table (the step's 39 separate 7-us launches were 3.6 % of the SAUnet:L step)
@@ -1520,7 +1585,15 @@ __global__ void __launch_bounds__(256) pack_weights_multi_kernel(const PackJobDe
   const long long first = (long long)((int)blockIdx.x - j.block0) * kPackPerBlock;
   const long long last = first + kPackPerBlock < j.total ? first + kPackPerBlock : j.total;
   pack_weights_range(j.w, j.out, last, j.Cin, j.Cout, j.KH, j.KW, j.J, j.NC, j.mpr, j.fmt, j.transpose_flip, j.Cout_total, j.co0,
-                     (first >> 3) + threadIdx.x, 256, j.split, j.C0);       // 2048 elements per block = one 16-byte group per thread
+                     (first >> 3) + threadIdx.x, 256, j.split, j.C0,       // 2048 elements per block = one 16-byte group per thread
+                     j.fmt == MPA_FMT_F16X3 ? reinterpret_cast<const float*>(j.out + 3 * j.total) : nullptr);
+}
+// the scales of every MPA_FMT_F16X3 job of a table (blockIdx.y = job; the other jobs return at once), launched before pack_weights_multi_kernel
+__global__ void __launch_bounds__(256) pack_scales_multi_kernel(const PackJobDev* __restrict__ jobs) {
+  const PackJobDev& j = jobs[blockIdx.y];
+  if (j.fmt != MPA_FMT_F16X3) return;
+  pack_scales_range(j.w, reinterpret_cast<float*>(j.out + 3 * j.total), j.Cin, j.Cout, j.KH, j.KW, j.transpose_flip, j.Cout_total, j.co0,
+                    (blockIdx.x * blockDim.x + threadIdx.x) >> 5, (gridDim.x * blockDim.x) >> 5);
 }
 
 static inline int grid_for(long long total, int block) {
@@ -1628,9 +1701,16 @@ int mpa_conv_tc_pack_weights_split_dev(const float* w_dev, void* packed_dev, int
   MPA_REQUIRE(J >= 0 && J * Cout <= 128 && co0 >= 0 && co0 < Cout_total, "conv_tc_pack_weights_dev: bad J / channel block");
   MPA_REQUIRE(split == 0 || (split > 1 && KW == 1 && C0 > 0 && (transpose_flip ? Cout_total : Cin) % split == 0),
               "conv_tc_pack_weights_dev: bad phase split (KW must be 1, the split channel count a multiple of split)");
+  MPA_REQUIRE(fmt == MPA_FMT_F16 || fmt == MPA_FMT_BF16 || (fmt == MPA_FMT_F16X3 && split == 0),
+              "conv_tc_pack_weights_dev: fmt must be MPA_FMT_F16, MPA_FMT_BF16 or MPA_FMT_F16X3 (no phase-split form)");
   if (J == 0) J = j_blocks(Cout);
   const int NC = (Cin + 7) / 8, mpr = mmas_per_row(NC, KW);
   const long long total = (long long)(KH + J - 1) * mpr * (kATileBytes / 2);
+  if (fmt == MPA_FMT_F16X3) {
+    pack_scales_kernel<<<16, 256, 0, (cudaStream_t)stream>>>(w_dev, reinterpret_cast<float*>((uint16_t*)packed_dev + 3 * total), Cin, Cout, KH, KW,
+                                                             transpose_flip, Cout_total, co0);
+    MPA_CHECK_LAUNCH("conv_tc_pack_weights_dev (scales)");
+  }
   pack_weights_kernel<<<grid_for(total, 256), 256, 0, (cudaStream_t)stream>>>(w_dev, (uint16_t*)packed_dev, total, Cin, Cout, KH, KW, J, NC, mpr, fmt,
                                                                               transpose_flip, Cout_total, co0, split, C0);
   MPA_CHECK_LAUNCH("conv_tc_pack_weights_dev");
@@ -1651,7 +1731,8 @@ int mpa_conv_tc_pack_table_build(const mpa_pack_job* jobs, int n_jobs, void* tab
   for (int i = 0; i < n_jobs; ++i) {
     const mpa_pack_job& a = jobs[i];
     MPA_REQUIRE(a.w && a.packed && a.Cin > 0 && a.Cout > 0 && a.Cout <= 128 && a.KH > 0 && a.KW > 0 && a.J >= 0 && a.J * a.Cout <= 128 &&
-                    a.co0 >= 0 && a.co0 < a.Cout_total && (a.fmt == MPA_FMT_F16 || a.fmt == MPA_FMT_BF16),
+                    a.co0 >= 0 && a.co0 < a.Cout_total &&
+                    (a.fmt == MPA_FMT_F16 || a.fmt == MPA_FMT_BF16 || (a.fmt == MPA_FMT_F16X3 && a.split == 0)),
                 "conv_tc_pack_table_build: bad job");
     const int J = a.J == 0 ? j_blocks(a.Cout) : a.J, NC = (a.Cin + 7) / 8, mpr = mmas_per_row(NC, a.KW);
     const long long total = (long long)(a.KH + J - 1) * mpr * (kATileBytes / 2);
@@ -1669,6 +1750,14 @@ int mpa_conv_tc_pack_weights_multi(const void* table_dev, int n_jobs, int n_bloc
   MPA_REQUIRE(table_dev && n_jobs > 0 && n_blocks > 0, "conv_tc_pack_weights_multi: bad argument");
   pack_weights_multi_kernel<<<n_blocks, 256, 0, (cudaStream_t)stream>>>((const PackJobDev*)table_dev, n_jobs);
   MPA_CHECK_LAUNCH("conv_tc_pack_weights_multi");
+  return MPA_OK;
+}
+
+int mpa_conv_tc_pack_scales_multi(const void* table_dev, int n_jobs, void* stream) {
+  MPA_CHECK_ARCH();
+  MPA_REQUIRE(table_dev && n_jobs > 0 && n_jobs <= 65535, "conv_tc_pack_scales_multi: bad argument");
+  pack_scales_multi_kernel<<<dim3(16, n_jobs), 256, 0, (cudaStream_t)stream>>>((const PackJobDev*)table_dev);
+  MPA_CHECK_LAUNCH("conv_tc_pack_scales_multi");
   return MPA_OK;
 }
 
@@ -2158,7 +2247,8 @@ int mpa_nchw_to_cp8_strided(const float* x, void* out_cp8, int B, int C, int T, 
   MPA_REQUIRE(x && out_cp8 && B > 0 && C > 0 && stride >= 1 && offset >= 0 && offset + (Fs - 1) * stride < F && pitch >= pf + F,
               "nchw_to_cp8_strided: bad argument");
   const int NCk = (C + 7) / 8;
-  if (ncs_out <= 0) ncs_out = NCk;
+  if (ncs_out <= 0) ncs_out = (fmt == MPA_FMT_F16X3 ? 2 : 1) * NCk;
+  MPA_REQUIRE(fmt != MPA_FMT_F16X3 || !(ncs_out & 1), "nchw_to_cp8_strided(fp16x3): the chunk stride must be even");
   long long total = (long long)B * NCk * T * Fs;
   nchw_to_cp8_strided_kernel<<<grid_for(total, 256), 256, 0, (cudaStream_t)stream>>>(x, (uint16_t*)out_cp8, total, C, T, Fs, NCk, ncs_out, T + 2 * pt,
                                                                                        pitch, pf, pt, fmt, stride, offset);

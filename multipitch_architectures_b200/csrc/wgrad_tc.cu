@@ -20,6 +20,11 @@
 //   - the x pixels within KW/2 of a real bin are zero where they are not real bins themselves, counted along the flattened rows: the band
 //     right of a row may continue into the next row's first columns;
 //   - every byte it reads is finite (NaN * 0 = NaN).
+// Split precision (mpa_conv_wgrad_tc_x3, wgrad_tc_kernel<true>): x and g are (hi, lo) fp16 plane pairs. The ring holds the g rows' hi planes
+// and, ring_lo bytes further, their lo planes; an x stage holds the CG hi slabs and then the CG lo slabs. Each K step issues three MMAs into
+// the one accumulator, g_hi.x_hi + g_lo.x_hi + g_hi.x_lo (the lo.lo term is below 2^-22 of the product). Both halves double the shared
+// memory of a row, so the output chunks are split into co-blocks of NCo chunks (n_coblk of them, a work-item dimension) where the planes
+// are wide; only bulk copies are used.
 #include "common.cuh"
 #include <cuda.h>
 #include <string.h>
@@ -39,6 +44,10 @@ struct WgradParams {
   long long x_item_stride, x_chunk_stride, g_item_stride, g_chunk_stride;   // bytes
   int B, T, P, KH, KW, ph, pw, NC, NCo, Cin, Cout, Cin_total, co0, ci0;
   int RS, n_sets, CG, n_cgroups, n_splits, n_items;
+  // split precision only: NCo output chunks per co-block, NCo_all = ceil(Cout/8); lo planes x_lo / g_lo bytes after the hi planes;
+  // the lo half of the ring ring_lo bytes after the hi half
+  int NCo_all, n_coblk, ring_lo;
+  long long x_lo, g_lo;
   int slots, slot_bytes, gslab_bytes, xslab_bytes, xstage_bytes, x_off, bar_off;
   uint32_t idesc;
   int wide;                    // KW == 1: the CG input chunks of a group are the N groups of ONE accumulator (B descriptor SBO = slab stride)
@@ -121,11 +130,15 @@ __device__ __forceinline__ void wg_ld32(uint32_t taddr, uint32_t* r) {
 }
 
 struct WgItem {
-  int set, cg, q0, q1, kh_hi, nset, c0, nchunks;
+  int set, cg, q0, q1, kh_hi, nset, c0, nchunks, cob;
 };
+template <bool X3>
 __device__ __forceinline__ WgItem wg_decode(const WgradParams& p, int item) {
   WgItem it;
-  const int type = item / p.n_splits, sp = item - type * p.n_splits;
+  int type = item / p.n_splits;
+  const int sp = item - type * p.n_splits;
+  it.cob = 0;
+  if (X3) { it.cob = type % p.n_coblk; type /= p.n_coblk; }
   it.set = type / p.n_cgroups;
   it.cg = type - it.set * p.n_cgroups;
   const long long R = (long long)p.B * p.T;
@@ -139,10 +152,11 @@ __device__ __forceinline__ WgItem wg_decode(const WgradParams& p, int item) {
   return it;
 }
 
+template <bool X3>
 __global__ void __launch_bounds__(kWgThreads, 1) wgrad_tc_kernel(const __grid_constant__ WgradParams p) {
   extern __shared__ __align__(1024) uint8_t smem[];
-  uint8_t* ring = smem;                                   // [slots + RS - 1][NCo][P px][16 B]
-  uint8_t* xs = smem + p.x_off;                           // [kWgXStages][CG][slab px][16 B]
+  uint8_t* ring = smem;                                   // [slots + RS - 1][NCo][P px][16 B] (X3: then the same for the lo planes)
+  uint8_t* xs = smem + p.x_off;                           // [kWgXStages][CG (X3: hi, then lo: 2 * CG)][slab px][16 B]
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem + p.bar_off);
   uint64_t* g_full = bars;                                // [slots]
   uint64_t* g_empty = bars + kWgMaxSlots;                 // [slots]
@@ -170,6 +184,7 @@ __global__ void __launch_bounds__(kWgThreads, 1) wgrad_tc_kernel(const __grid_co
   asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
   const uint32_t tmem_base = *tmem_slot;
   const int ksteps = p.P >> 4;
+  constexpr int halves = X3 ? 2 : 1;
 
   if (warp == 0) {
     // ===================================================== producer: g rows (ring, ascending t) and x row slabs
@@ -180,7 +195,7 @@ __global__ void __launch_bounds__(kWgThreads, 1) wgrad_tc_kernel(const __grid_co
       int xst = 0;
       uint32_t xph = 0;
       for (int item = blockIdx.x; item < p.n_items; item += gridDim.x) {
-        const WgItem it = wg_decode(p, item);
+        const WgItem it = wg_decode<X3>(p, item);
         for (int q = it.q0; q < it.q1; ++q) {
           const int b = q / p.T, s = q - b * p.T;
           const int t_new = s + p.ph - it.kh_hi + it.nset - 1;            // newest g row of this x row's tile
@@ -191,12 +206,12 @@ __global__ void __launch_bounds__(kWgThreads, 1) wgrad_tc_kernel(const __grid_co
             const bool mirror = pos < p.RS - 1;
             if (lane == 0) {
               wg_mbar_wait(&g_empty[pos], ((n_row / (uint32_t)S) & 1u) ^ 1u);
-              wg_mbar_expect_tx(&g_full[pos], (uint32_t)(p.NCo * p.gslab_bytes) * (mirror ? 2u : 1u));
+              wg_mbar_expect_tx(&g_full[pos], (uint32_t)(p.NCo * p.gslab_bytes * halves) * (mirror ? 2u : 1u));
             }
             __syncwarp();
             uint8_t* dst = ring + (size_t)pos * p.slot_bytes;
             const bool inside = (t >= 0 && t < p.T);
-            const int n_copies = p.tma ? 0 : p.NCo * (mirror ? 2 : 1);
+            const int n_copies = p.tma ? 0 : p.NCo * (mirror ? 2 : 1) * halves;
             if (p.tma && lane == 0) {
               for (int mir = 0; mir < (mirror ? 2 : 1); ++mir)
                 asm volatile(
@@ -206,16 +221,21 @@ __global__ void __launch_bounds__(kWgThreads, 1) wgrad_tc_kernel(const __grid_co
                     : "memory");
             }
             for (int i = lane; i < n_copies; i += 32) {
-              const int ck = i % p.NCo, mir = i / p.NCo;
-              const uint8_t* src = inside ? p.g + (long long)b * p.g_item_stride + (long long)ck * p.g_chunk_stride + (long long)t * p.P * 16
-                                          : p.zero_row + (size_t)ck * p.gslab_bytes;
-              wg_bulk_g2s(dst + (mir ? (size_t)S * p.slot_bytes : 0) + (size_t)ck * p.gslab_bytes, src, (uint32_t)p.gslab_bytes, &g_full[pos]);
+              const int ck = i % p.NCo, rest = i / p.NCo;
+              const int mir = X3 ? rest >> 1 : rest, h = X3 ? rest & 1 : 0;
+              const int gck = it.cob * p.NCo + ck;                          // chunks past the last output chunk read zeros
+              const uint8_t* src = (inside && (!X3 || gck < p.NCo_all))
+                                       ? p.g + (long long)b * p.g_item_stride + (long long)gck * p.g_chunk_stride + (h ? p.g_lo : 0) +
+                                             (long long)t * p.P * 16
+                                       : p.zero_row + (size_t)ck * p.gslab_bytes;
+              wg_bulk_g2s(dst + (h ? (size_t)p.ring_lo : 0) + (mir ? (size_t)S * p.slot_bytes : 0) + (size_t)ck * p.gslab_bytes, src,
+                          (uint32_t)p.gslab_bytes, &g_full[pos]);
             }
             __syncwarp();
           }
           if (lane == 0) {
             wg_mbar_wait(&x_empty[xst], xph ^ 1);
-            wg_mbar_expect_tx(&x_full[xst], (uint32_t)((p.tma_x ? p.CG : it.nchunks) * p.xslab_bytes));
+            wg_mbar_expect_tx(&x_full[xst], (uint32_t)((p.tma_x ? p.CG : it.nchunks) * p.xslab_bytes * halves));
             if (p.tma_x)
               asm volatile(
                   "cp.async.bulk.tensor.4d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4, %5}], [%6];" ::"r"(
@@ -225,9 +245,11 @@ __global__ void __launch_bounds__(kWgThreads, 1) wgrad_tc_kernel(const __grid_co
           }
           __syncwarp();
           const uint8_t* xsrc = p.x + (long long)b * p.x_item_stride + ((long long)s * p.P - p.pw) * 16;
-          for (int c = lane; c < (p.tma_x ? 0 : it.nchunks); c += 32)
-            wg_bulk_g2s(xs + (size_t)xst * p.xstage_bytes + (size_t)c * p.xslab_bytes, xsrc + (long long)(it.c0 + c) * p.x_chunk_stride,
-                        (uint32_t)p.xslab_bytes, &x_full[xst]);
+          for (int i = lane; i < (p.tma_x ? 0 : it.nchunks * halves); i += 32) {
+            const int h = X3 ? i / it.nchunks : 0, c = i - h * it.nchunks;
+            wg_bulk_g2s(xs + (size_t)xst * p.xstage_bytes + (size_t)(h * p.CG + c) * p.xslab_bytes,
+                        xsrc + (long long)(it.c0 + c) * p.x_chunk_stride + (h ? p.x_lo : 0), (uint32_t)p.xslab_bytes, &x_full[xst]);
+          }
           __syncwarp();
           if (++xst == kWgXStages) { xst = 0; xph ^= 1; }
         }
@@ -247,7 +269,7 @@ __global__ void __launch_bounds__(kWgThreads, 1) wgrad_tc_kernel(const __grid_co
     int xst = 0;
     uint32_t xph = 0, k_item = 0;
     for (int item = blockIdx.x; item < p.n_items; item += gridDim.x, ++k_item) {
-      const WgItem it = wg_decode(p, item);
+      const WgItem it = wg_decode<X3>(p, item);
       wg_mbar_wait(acc_empty, (k_item & 1u) ^ 1u);
       asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
       uint32_t first = 1;
@@ -271,9 +293,15 @@ __global__ void __launch_bounds__(kWgThreads, 1) wgrad_tc_kernel(const __grid_co
             for (int c = 0; c < it.nchunks; ++c) {
               const uint32_t tmem_d = tmem_u + (uint32_t)c * 128u;
               const uint32_t b_lo = b_lo0 + (uint32_t)c * xsl16;
-              for (int ks = 0; ks < ksteps; ++ks)
-                wg_mma(tmem_d, ((uint64_t)a_hi << 32) | (uint64_t)(a_lo + (uint32_t)ks * 16u), ((uint64_t)b_hi << 32) | (uint64_t)(b_lo + (uint32_t)ks * 16u),
-                       p.idesc, (first && ks == 0) ? 0u : 1u);
+              for (int ks = 0; ks < ksteps; ++ks) {
+                const uint64_t ad = ((uint64_t)a_hi << 32) | (uint64_t)(a_lo + (uint32_t)ks * 16u);
+                const uint64_t bd = ((uint64_t)b_hi << 32) | (uint64_t)(b_lo + (uint32_t)ks * 16u);
+                wg_mma(tmem_d, ad, bd, p.idesc, (first && ks == 0) ? 0u : 1u);
+                if (X3) {
+                  wg_mma(tmem_d, ad + ((uint32_t)p.ring_lo >> 4), bd, p.idesc, 1u);                     // g_lo . x_hi
+                  wg_mma(tmem_d, ad, bd + (uint32_t)p.CG * xsl16, p.idesc, 1u);                          // g_hi . x_lo
+                }
+              }
             }
           }
           wg_commit(&x_empty[xst]);
@@ -297,10 +325,11 @@ __global__ void __launch_bounds__(kWgThreads, 1) wgrad_tc_kernel(const __grid_co
     const int ncols = p.KW * 8;
     uint32_t k_item = 0;
     for (int item = blockIdx.x; item < p.n_items; item += gridDim.x, ++k_item) {
-      const WgItem it = wg_decode(p, item);
+      const WgItem it = wg_decode<X3>(p, item);
       wg_mbar_wait(acc_full, k_item & 1u);
       asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-      const bool row_ok = (r < it.nset) && (co < p.Cout);
+      const int co_g = it.cob * p.NCo * 8 + co;            // output channel of the call (co-blocks: X3 only)
+      const bool row_ok = (r < it.nset) && (co_g < p.Cout);
       const int kh = it.kh_hi - r;
       if (p.wide) {
         // one accumulator: column n = (input chunk n / 8 of the group, channel n % 8), the single tap kw = 0
@@ -314,7 +343,7 @@ __global__ void __launch_bounds__(kWgThreads, 1) wgrad_tc_kernel(const __grid_co
               const int n = c0 + i;
               const int ci = (it.c0 + (n >> 3)) * 8 + (n & 7);
               if (n < it.nchunks * 8 && ci < p.Cin)
-                atomicAdd(p.gw + ((size_t)(p.co0 + co) * p.Cin_total + p.ci0 + ci) * p.KH + kh, __uint_as_float(v[i]));
+                atomicAdd(p.gw + ((size_t)(p.co0 + co_g) * p.Cin_total + p.ci0 + ci) * p.KH + kh, __uint_as_float(v[i]));
             }
           }
         }
@@ -330,7 +359,7 @@ __global__ void __launch_bounds__(kWgThreads, 1) wgrad_tc_kernel(const __grid_co
               const int n = c0 + i;
               const int kw = n >> 3, ci = (it.c0 + c) * 8 + (n & 7);
               if (n < ncols && ci < p.Cin)
-                atomicAdd(p.gw + (((size_t)(p.co0 + co) * p.Cin_total + p.ci0 + ci) * p.KH + kh) * p.KW + kw, __uint_as_float(v[i]));
+                atomicAdd(p.gw + (((size_t)(p.co0 + co_g) * p.Cin_total + p.ci0 + ci) * p.KH + kh) * p.KW + kw, __uint_as_float(v[i]));
             }
           }
         }
@@ -420,7 +449,7 @@ int mpa_conv_wgrad_tc(const void* x_cp8, const void* g_cp8, const void* zero_row
   p.idesc = (1u << 4) | (f << 7) | (f << 10) | (1u << 15) | (1u << 16) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
   {
     static unsigned char flags[64];
-    cudaError_t e = opt_in_max_smem(wgrad_tc_kernel, flags);
+    cudaError_t e = opt_in_max_smem(wgrad_tc_kernel<false>, flags);
     if (e != cudaSuccess) {
       set_error("conv_wgrad_tc: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
       return MPA_ERR_CUDA;
@@ -450,8 +479,100 @@ int mpa_conv_wgrad_tc(const void* x_cp8, const void* g_cp8, const void* zero_row
     }
   }
   const int grid = p.n_items < sms ? p.n_items : sms;
-  wgrad_tc_kernel<<<grid, kWgThreads, smem, (cudaStream_t)stream>>>(p);
+  wgrad_tc_kernel<false><<<grid, kWgThreads, smem, (cudaStream_t)stream>>>(p);
   MPA_CHECK_LAUNCH("conv_wgrad_tc");
+  return MPA_OK;
+}
+
+int mpa_conv_wgrad_tc_x3(const void* x_cp8, const void* g_cp8, const void* zero_row, float* gw, int n_items, int Cin, int Cout, int T, int F,
+                         int KH, int KW, int pitch, int pf, int pt, int x_nc_stride, int g_nc_stride, int Cin_total, int ci0, int Cout_total,
+                         int co0, void* stream) {
+  MPA_CHECK_ARCH();
+  MPA_REQUIRE(x_cp8 && g_cp8 && zero_row && gw && n_items > 0 && Cin > 0 && Cout > 0 && Cout <= 128,
+              "conv_wgrad_tc_x3: bad argument (Cout <= 128 per call)");
+  MPA_REQUIRE((KH & 1) && (KW & 1) && KW >= 3 && KW <= 15, "conv_wgrad_tc_x3: odd kernel sizes, 3 <= KW <= 15 (no KW == 1 form)");
+  MPA_REQUIRE(pitch % 16 == 0 && pitch >= 16 && pitch <= 256 && pf >= KW / 2 && pitch - F >= KW / 2 && pitch >= pf + F && pt >= 1,
+              "conv_wgrad_tc_x3: CP8 geometry (pitch %d, pf %d, F %d, KW %d)", pitch, pf, F, KW);
+  MPA_REQUIRE(ci0 >= 0 && co0 >= 0 && ci0 + Cin <= Cin_total && co0 + Cout <= Cout_total, "conv_wgrad_tc_x3: channel block outside the weight tensor");
+  MPA_REQUIRE((((uintptr_t)x_cp8 | (uintptr_t)g_cp8 | (uintptr_t)zero_row) & 15) == 0, "conv_wgrad_tc_x3: 16-byte alignment required");
+  const int NC = (Cin + 7) / 8, NCo_all = (Cout + 7) / 8;
+  const int xs_ = x_nc_stride > 0 ? x_nc_stride : 2 * NC, gs_ = g_nc_stride > 0 ? g_nc_stride : 2 * NCo_all;
+  MPA_REQUIRE(xs_ % 2 == 0 && gs_ % 2 == 0 && xs_ >= 2 * NC && gs_ >= 2 * NCo_all,
+              "conv_wgrad_tc_x3: the chunk strides (%d, %d) must be even and hold hi and lo planes of every chunk", xs_, gs_);
+  WgradParams p;
+  memset(&p, 0, sizeof(p));
+  p.B = n_items; p.T = T; p.P = pitch; p.KH = KH; p.KW = KW; p.ph = KH / 2; p.pw = KW / 2;
+  p.NC = NC; p.NCo_all = NCo_all;
+  p.Cin = Cin; p.Cout = Cout; p.Cin_total = Cin_total; p.co0 = co0; p.ci0 = ci0;
+  const long long plane = (long long)(T + 2 * pt) * pitch * 16;
+  p.x_chunk_stride = plane;
+  p.g_chunk_stride = plane;
+  p.x_item_stride = plane * xs_;
+  p.g_item_stride = plane * gs_;
+  p.x_lo = plane * (xs_ / 2);
+  p.g_lo = plane * (gs_ / 2);
+  p.x = (const uint8_t*)x_cp8 + (long long)pt * pitch * 16;
+  p.g = (const uint8_t*)g_cp8 + (long long)pt * pitch * 16;
+  p.zero_row = (const uint8_t*)zero_row;
+  p.gw = gw;
+  p.gslab_bytes = pitch * 16;
+  p.xslab_bytes = ((pitch + 2 * (KW / 2) + 1 + 7) / 8 * 8) * 16;
+  // Shared memory: both halves of the ring (slots + RS - 1 rows of NCo chunks each) and of kWgXStages x stages of CG chunks, 1 KB of
+  // barriers, and the reach of the last tile's M = 128 rows past the lo ring. Shrink RS, then CG, then halve the co-block until it fits;
+  // NCo = RS = CG = 1 at pitch 256 needs max(16 KB + 6 * 4.25 KB + 1 KB, 3 * 4 KB + 64 KB of reach) = 76 KB, so every admissible call fits.
+  auto need = [&](int NCo, int RS, int CG, int slots) {
+    const size_t slot = (size_t)NCo * p.gslab_bytes;
+    const size_t top = 2 * (size_t)(slots + RS - 1) * slot + (size_t)kWgXStages * 2 * CG * p.xslab_bytes + 1024;
+    const size_t reach = (size_t)(2 * slots + RS - 2) * slot + 16 * (size_t)p.gslab_bytes;
+    return top > reach ? top : reach;
+  };
+  const size_t kMax = 227 * 1024;
+  int NCo = NCo_all, RS, CG;
+  for (;;) {
+    RS = 16 / NCo < KH ? 16 / NCo : KH;
+    CG = NC < 4 ? NC : 4;
+    while (RS > 1 && need(NCo, RS, CG, RS + 1) > kMax) --RS;
+    while (CG > 1 && need(NCo, RS, CG, RS + 1) > kMax) --CG;
+    if (need(NCo, RS, CG, RS + 1) <= kMax || NCo == 1) break;
+    NCo = (NCo + 1) / 2;
+  }
+  p.NCo = NCo; p.RS = RS; p.CG = CG;
+  p.n_coblk = (NCo_all + NCo - 1) / NCo;
+  p.n_sets = (KH + RS - 1) / RS;
+  p.n_cgroups = (NC + CG - 1) / CG;
+  p.slot_bytes = NCo * p.gslab_bytes;
+  p.xstage_bytes = 2 * CG * p.xslab_bytes;
+  int slots = RS + 3;
+  while (slots > RS + 1 && need(NCo, RS, CG, slots) > kMax) --slots;
+  MPA_REQUIRE(need(NCo, RS, CG, slots) <= kMax, "conv_wgrad_tc_x3: the row ring does not fit in shared memory (Cout=%d pitch=%d)", Cout, pitch);
+  p.slots = slots;
+  p.ring_lo = (slots + RS - 1) * p.slot_bytes;
+  p.x_off = 2 * p.ring_lo;
+  p.bar_off = p.x_off + kWgXStages * p.xstage_bytes;
+  const size_t smem = need(NCo, RS, CG, slots);
+  int dev = 0, sms = 148;
+  cudaGetDevice(&dev);
+  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  const int n_types = p.n_sets * p.n_cgroups * p.n_coblk;
+  const long long R = (long long)n_items * T;
+  int splits = sms / n_types;
+  if (splits > R) splits = (int)R;
+  if (splits < 1) splits = 1;
+  p.n_splits = splits;
+  p.n_items = n_types * splits;
+  const int N = (KW * 8 + 15) / 16 * 16;
+  p.idesc = (1u << 4) | (1u << 15) | (1u << 16) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);   // fp16 x fp16 -> fp32
+  {
+    static unsigned char flags[64];
+    cudaError_t e = opt_in_max_smem(wgrad_tc_kernel<true>, flags);
+    if (e != cudaSuccess) {
+      set_error("conv_wgrad_tc_x3: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
+      return MPA_ERR_CUDA;
+    }
+  }
+  const int grid = p.n_items < sms ? p.n_items : sms;
+  wgrad_tc_kernel<true><<<grid, kWgThreads, smem, (cudaStream_t)stream>>>(p);
+  MPA_CHECK_LAUNCH("conv_wgrad_tc_x3");
   return MPA_OK;
 }
 

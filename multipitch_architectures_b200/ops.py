@@ -527,16 +527,21 @@ def _zero_row(device, nbytes):
 def conv_wgrad_tc(x, g, gw, ksize):
     """gw [Cout, Cin, KH, KW] fp32 (overwritten) = weight gradient of the stride-1 'same' convolution; x, g: CP8 of one geometry.
     The kernel sums over every pixel of the padded rows, so the planes must keep: the gap columns of g's real channels zero; the x pixels
-    within KW/2 of a real bin (along the flattened rows) zero; everything finite."""
+    within KW/2 of a real bin (along the flattened rows) zero; everything finite.
+    FMT_F16X3 planes go to the split-precision kernel (mpa_conv_wgrad_tc_x3, KW >= 3)."""
     Cout_t, Cin_t, KH, KW = gw.shape
     assert (KH, KW) == tuple(ksize) and x.B == g.B and (x.T, x.F, x.pitch, x.pf, x.pt) == (g.T, g.F, g.pitch, g.pf, g.pt)
+    assert x.fmt == g.fmt
     gw.zero_()
     for co0 in range(0, g.C, 128):
         co = min(128, g.C - co0)
         gv = g.channels(co0, co) if (co0 or co != g.C) else g
         z = _zero_row(gw.device, ((co + 7) // 8) * x.pitch * 16)
-        call('conv_wgrad_tc', x.ptr(), gv.ptr(), z, gw, x.B, x.C, co, x.T, x.F, KH, KW, x.pitch, x.pf, x.pt, x.ncs, gv.ncs, Cin_t, 0, Cout_t, co0,
-             x.fmt, stream_ptr())
+        args = (x.ptr(), gv.ptr(), z, gw, x.B, x.C, co, x.T, x.F, KH, KW, x.pitch, x.pf, x.pt, x.ncs, gv.ncs, Cin_t, 0, Cout_t, co0)
+        if x.fmt == FMT_F16X3:
+            call('conv_wgrad_tc_x3', *args, stream_ptr())
+        else:
+            call('conv_wgrad_tc', *args, x.fmt, stream_ptr())
     return gw
 
 
@@ -570,6 +575,8 @@ class PackPlan:
 
     def refresh(self):
         if self.table is not None:
+            if any(j.fmt == FMT_F16X3 for j in self.jobs):      # the per-channel scales of the split-precision jobs come first
+                call('conv_tc_pack_scales_multi', self.table, len(self.jobs), stream_ptr())
             call('conv_tc_pack_weights_multi', self.table, len(self.jobs), self.n_blocks, stream_ptr())
             self.fresh = True
 
@@ -597,7 +604,7 @@ def conv_tc_pack_dev(w, Cin, Cout, ksize, fmt, transpose_flip=False, Cout_total=
     key = (w.data_ptr(), Cin, Cout, KH, KW, fmt, int(bool(transpose_flip)), Ct, co0, J, split, C0)
     if plan is not None and plan.fresh and key in plan.index:
         return plan.index[key]
-    nbytes = _lib.lib().mpa_conv_tc_packed_bytes(Cin, Cout, KH, KW, J)
+    nbytes = _lib.lib().mpa_conv_tc_packed_bytes_fmt(Cin, Cout, KH, KW, J, fmt)
     if nbytes == 0:
         raise _lib.MpaError(f'conv_tc cannot pack Cin={Cin} Cout={Cout} K={KH}x{KW}')
     packed = plan.index.get(key) if plan is not None else None

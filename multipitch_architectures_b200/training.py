@@ -15,6 +15,8 @@ models without the residual path, activations and gradients stay in the 16-bit C
 pool + dropout forward / backward and the bias gradients are train_cp8.cu kernels; bit-identical to crossing the nchw<->CP8 converters
 around the fp32 kernels).  fp16 cannot hold gradients as small as bf16 can, so the fused step of an fp16 model scales its loss
 (`LossScaler`, torch.amp.GradScaler's policy); drop-in fp16 training wants a torch.amp.GradScaler, as fp16 AMP always does.
+With `precision='fp16x3'` only the convolution products move to the tensor cores, in split precision (`conv_fmt`), behind nchw<->CP8
+converters; its fused step scales the loss in the same way.
 Dropout uses a Philox stream (seed, per-site offset); the reference's torch RNG stream cannot be reproduced, so parity
 tests run with p_dropout = 0 (SURVEY.md §7).
 
@@ -37,8 +39,18 @@ _TAPE_FMT = {'bf16': ops.FMT_BF16, 'fp16': ops.FMT_F16}
 
 def tape_fmt(model):
     """16-bit operand / plane format of the tensor-core training tapes: bf16 and fp16 models; None for the others (fp32, and fp16x3,
-    which trains on the fp32 tape)."""
+    whose activations stay fp32 NCHW between the convolutions: see conv_fmt)."""
     return _TAPE_FMT.get(getattr(model, 'precision', 'fp32'))
+
+
+_CONV_FMT = dict(_TAPE_FMT, fp16x3=ops.FMT_F16X3)
+
+
+def conv_fmt(model):
+    """Format of the tensor-core convolutions of the fp32 NCHW training tape (TcConv, the head conv2 behind its converters): the tape
+    format, and split precision (MPA_FMT_F16X3) for an fp16x3 model; None for fp32.  Only the convolution products of an fp16x3 model move
+    to the tensor cores: every CP8-resident or gemm_tc path keys on tape_fmt, which is None for it."""
+    return _CONV_FMT.get(getattr(model, 'precision', 'fp32'))
 
 
 class StepState:
@@ -267,7 +279,7 @@ class TcConv:
     @staticmethod
     def eligible(model, conv, F):
         KH, KW = conv.kernel_size
-        return (tape_fmt(model) is not None and tuple(conv.stride) == (1, 1) and KH % 2 == 1 and KW % 2 == 1 and 3 <= KW <= 15 and KH >= 3
+        return (conv_fmt(model) is not None and tuple(conv.stride) == (1, 1) and KH % 2 == 1 and KW % 2 == 1 and 3 <= KW <= 15 and KH >= 3
                 and tuple(conv.padding) == (KH // 2, KW // 2) and F + TcConv.PF + 15 < 272 and conv.bias is not None)
 
     @classmethod
@@ -374,7 +386,7 @@ class TcConv:
 def _tc_s3_eligible(model, conv, F):
     """The head's 3x3 / stride (1,3) / pad (1,0) convolution (basic_cnns.py:391) = the stride-1 'same' 3x3 convolution sampled at
     columns 1, 4, 7, ... ; its backward is the stride-1 backward of the zero-inserted output gradient."""
-    return (tape_fmt(model) is not None and tuple(conv.kernel_size) == (3, 3) and tuple(conv.stride) == (1, 3)
+    return (conv_fmt(model) is not None and tuple(conv.kernel_size) == (3, 3) and tuple(conv.stride) == (1, 3)
             and tuple(conv.padding) == (1, 0) and F % 3 == 0 and F + TcConv.PF + 15 < 272 and conv.bias is not None)
 
 
@@ -475,7 +487,8 @@ LN_PIXEL = True
 def _cp8_resident(model, blocks, F):
     """bf16 / fp16 mode, no residual path: activations and gradients stay in the CP8 planes between the convolutions of the blocks
     (pool + dropout forward / backward and the bias gradients run on the planes, train_cp8.cu)."""
-    return (CP8_RESIDENT and not getattr(model, 'residual', False) and F % 4 == 0 and all(TcConv.eligible(model, c, F) for _, c in blocks)
+    return (CP8_RESIDENT and tape_fmt(model) is not None and not getattr(model, 'residual', False) and F % 4 == 0
+            and all(TcConv.eligible(model, c, F) for _, c in blocks)
             and _tc_s3_eligible(model, model.conv2[0], F))
 
 
@@ -532,7 +545,7 @@ class Tape:
         do full-height ones with more than 10 output channels unless rows_tc is False (_rows_tc_eligible)."""
         fmt = tape_fmt(self.model)
         if TcConv.eligible(self.model, conv, x.d.shape[3]) and x.d.shape[2] >= 2:
-            y, xc = TcConv.forward(name, conv, x.d, act, a, fmt)
+            y, xc = TcConv.forward(name, conv, x.d, act, a, conv_fmt(self.model))
             out = Node(y)
 
             def bwd_tc():
@@ -599,7 +612,7 @@ class Tape:
         """CNN block on fp32 NCHW: Conv2d (tensor cores behind the nchw<->CP8 converters when TcConv is eligible) -> LeakyReLU ->
         MaxPool((3,1)) -> dropout (+ x when `residual`)."""
         if TcConv.eligible(self.model, conv, x.d.shape[3]):
-            act, xc = TcConv.forward(name, conv, x.d, ops.ACT_LRELU, a, tape_fmt(self.model))
+            act, xc = TcConv.forward(name, conv, x.d, ops.ACT_LRELU, a, conv_fmt(self.model))
         else:
             act, xc = _conv_fwd(conv, x.d, ops.ACT_LRELU, a), None
         off = self._take_site()
@@ -649,7 +662,7 @@ class Tape:
         if split:
             y, xc = _tc_s3_forward_split(name, conv, x.d, ops.ACT_LRELU, a)
         elif planes or _tc_s3_eligible(self.model, conv, x.d.shape[3]):
-            y, xc = _tc_s3_forward(name, conv, x.d, ops.ACT_LRELU, a, tape_fmt(self.model))
+            y, xc = _tc_s3_forward(name, conv, x.d, ops.ACT_LRELU, a, conv_fmt(self.model))
         else:
             y, xc = _conv_fwd(conv, x.d, ops.ACT_LRELU, a), None
         off = self._take_site()
@@ -683,7 +696,7 @@ class Tape:
 def note_fp32_tape(model):
     """An eval-mode backward of a tensor-core model that runs on the fp32 NCHW tape says so, once per model class."""
     prec = getattr(model, 'precision', 'fp32')
-    if tape_fmt(model) is not None:
+    if conv_fmt(model) is not None:
         _exec.note_path(model, 'eval-mode backward runs on the fp32 NCHW training tape (tensor-core convolutions behind nchw<->CP8 converters), '
                                'not on the CP8-resident tape')
     elif prec in _exec.TC_PRECISIONS:
@@ -810,7 +823,8 @@ class FusedTrainStep:
         self.comm_events = None                        # bench.py: a list that receives CUDA events around the all-reduce
         self._state = StepState(dev, self.sites_per_step)
         self._tape = None
-        self.scaler = LossScaler(dev) if getattr(model, 'precision', 'fp32') == 'fp16' else None
+        # fp16x3 too: its split planes carry no scale, so an unscaled gradient below ~1e-3 would hit the lo half's 3e-8 absolute floor
+        self.scaler = LossScaler(dev) if getattr(model, 'precision', 'fp32') in ('fp16', 'fp16x3') else None
 
     @property
     def loss_scale(self):
