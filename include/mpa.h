@@ -98,6 +98,11 @@ int mpa_layernorm_frames(const float* frames, const float* ln_w, const float* ln
  * in [C][NT][F] (already zero-padded by the caller as exp126a:420 does), out [n][C][T][F]; gamma_log <= 0 -> no compression. */
 int mpa_gather_patches_f32(const float* in, float* out, int C, int NT, int F, int i0, int n, int T, int stride,
                            float gamma_log, void* stream);
+/* Its adjoint: g_in[c][r][f] = sum over the patches p covering frame r of g_out[p][c][r - (i0+p)*stride][f], times gamma_log / (1 +
+ * gamma_log * in[c][r][f]) (1 when gamma_log <= 0; `in` is the forward input and may then be NULL).  g_in [C][NT][F] overwritten (rows no
+ * patch covers are 0); one thread per element, deterministic. */
+int mpa_gather_patches_bwd_f32(const float* g_out, const float* in, float* g_in, int C, int NT, int F, int i0, int n, int T, int stride,
+                               float gamma_log, void* stream);
 
 /* Training-time augmentation fused with the patch cut (hcqt_datasets.py:67-141; SURVEY.md 8f row 1): for each of n patches starting at
  * frame start[b] of in [C][NT][F]:  random EQ  w_c(f) = 1 - 2e-6*eq_alpha[b]*(f - (eq_beta[b] - eq_offset[c]))^2  (:80-97; eq_alpha NULL or 0 = off)
@@ -391,6 +396,27 @@ typedef struct mpa_cqt_level {
 } mpa_cqt_level;
 int mpa_cqt_levels_f32(const mpa_cqt_level* levels, int n_levels, int n_frames, int band, const int* tuning_idx, float* out,
                        int out_frames, int out_bins, void* stream);
+/* Backward of mpa_cqt_levels_f32 (autograd from the HCQT to the audio): given g_out = dL/d out [H][out_frames][out_bins], writes
+ * dL/d y of every level's signal.  Per (frame, level) the spectrum is recomputed from y, w_r = row_scale * (sum of g_out over the row's
+ * destinations) * conj(C_r) / |C_r| (0 where |C_r| = 0), V = the transposed banded contraction of w (over the bin -> rows table),
+ * frame gradient = Re(FFT(V zero-extended to n_fft)) -> workspace; then the adjoint of the reflect-padded framing (overlap-add, with every
+ * reflection of signals shorter than n_fft) sums the frame gradients into g_y.  Levels that read the same signal pass the same g_y and are
+ * summed together; g_y is overwritten, or added to when `accumulate` is non-zero.  Deterministic (fixed summation order, no atomics).
+ * Workspace: mpa_cqt_levels_bwd_workspace bytes = n_frames * sum(n_fft) floats. */
+typedef struct mpa_cqt_level_grad {
+  float* g_y;                /* [n] gradient of the level's signal */
+  const int* bin_off;        /* [n_tunings][n_fft/2 + 2]: rows covering bin k are bin_rows[tuning][bin_off[tuning][k] .. bin_off[tuning][k+1]) */
+  const int* bin_rows;       /* [n_tunings][n_rows * band]: row indices, grouped by bin (bins < n_fft/2 + 1 only), ascending within a bin */
+} mpa_cqt_level_grad;
+size_t mpa_cqt_levels_bwd_workspace(const mpa_cqt_level* levels, int n_levels, int n_frames);
+int mpa_cqt_levels_bwd_f32(const mpa_cqt_level* levels, const mpa_cqt_level_grad* grads, int n_levels, int n_frames, int band,
+                           const int* tuning_idx, const float* g_out, int out_frames, int out_bins, int accumulate, void* workspace,
+                           size_t ws_bytes, void* stream);
+/* Transpose of mpa_decimate_gain_f32 for the same (half_taps, factor, gain, n_in): g_in[i] (+)= gain * sum_{t < floor(n_in/factor)}
+ * h[|i - factor*t|] * g_out[t] over the taps the forward reads (taps outside the signal are skipped there, so they carry nothing back).
+ * g_out: ceil(n_in/factor) floats, g_in: n_in floats, overwritten or added to (`accumulate`).  float64 accumulation. */
+int mpa_decimate_adjoint_f32(const float* g_out, float* g_in, const float* half_taps, int n_half, int factor, double gain, long long n_in,
+                             int accumulate, void* stream);
 /* librosa.estimate_tuning(y, sr, bins_per_octave) with n_fft=2048, hop=512, fmin=150, fmax=4000, threshold=0.1,
  * resolution=0.01: writes tuning_idx[0] in [0,100), tuning = -0.5 + 0.01*idx.  hann2048: periodic hann window. */
 size_t mpa_tuning_workspace(int n_frames);

@@ -35,7 +35,7 @@ def lib():
         _lib = ctypes.CDLL(LIB_PATH)
         _lib.mpa_last_error.restype = ctypes.c_char_p
         _lib.mpa_launch_count.restype = ctypes.c_longlong
-        for name in ('mpa_encoder_layer_workspace', 'mpa_conv_tc_packed_bytes', 'mpa_conv_tc_packed_bytes_fmt', 'mpa_conv_tc_pool_workspace_fmt', 'mpa_tuning_workspace', 'mpa_conv_tc_pool_workspace', 'mpa_conv_tc_ring_packed_bytes', 'mpa_gemm_tc_chunked_bytes', 'mpa_eval_workspace', 'mpa_lstm_layer_workspace', 'mpa_lstm_layer_bwd_workspace', 'mpa_conv_rows_fwd_workspace'):
+        for name in ('mpa_encoder_layer_workspace', 'mpa_conv_tc_packed_bytes', 'mpa_conv_tc_packed_bytes_fmt', 'mpa_conv_tc_pool_workspace_fmt', 'mpa_tuning_workspace', 'mpa_cqt_levels_bwd_workspace', 'mpa_conv_tc_pool_workspace', 'mpa_conv_tc_ring_packed_bytes', 'mpa_gemm_tc_chunked_bytes', 'mpa_eval_workspace', 'mpa_lstm_layer_workspace', 'mpa_lstm_layer_bwd_workspace', 'mpa_conv_rows_fwd_workspace'):
             if hasattr(_lib, name):
                 getattr(_lib, name).restype = ctypes.c_size_t
     return _lib

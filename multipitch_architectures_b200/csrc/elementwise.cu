@@ -378,6 +378,24 @@ __global__ void gather_patches_kernel(const float* __restrict__ in, float* __res
   }
 }
 
+// adjoint of gather_patches_kernel: one thread per input element sums the patches that read it (patch order), then applies
+// d log(1 + gamma*x) / dx = gamma / (1 + gamma*x)
+__global__ void gather_patches_bwd_kernel(const float* __restrict__ g_out, const float* __restrict__ in, float* __restrict__ g_in, long long total,
+                                          int C, int NT, int F, int i0, int n, int T, int stride, float gamma) {
+  for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
+    const int f = (int)(i % F);
+    const int r = (int)((i / F) % NT);
+    const int c = (int)(i / ((long long)F * NT));
+    // patch p covers frames [(i0+p)*stride, (i0+p)*stride + T)
+    const int p0 = max(0, (r - T + 1 <= 0 ? 0 : (r - T + stride) / stride) - i0);
+    const int p1 = min(n - 1, r / stride - i0);
+    float acc = 0.f;
+    for (int p = p0; p <= p1; ++p) acc += g_out[(((size_t)p * C + c) * T + (r - (i0 + p) * stride)) * F + f];
+    if (gamma > 0.f && acc != 0.f) acc *= gamma / __fadd_rn(1.f, __fmul_rn(gamma, in[i]));
+    g_in[i] = acc;
+  }
+}
+
 static inline int grid_for(long long total, int block) {
   long long g = (total + block - 1) / block;
   long long cap = 148LL * 16;
@@ -438,6 +456,19 @@ int mpa_gather_patches_f32(const float* in, float* out, int C, int NT, int F, in
   long long total = (long long)n * C * T * F;
   gather_patches_kernel<<<grid_for(total, 256), 256, 0, (cudaStream_t)stream>>>(in, out, total, C, NT, F, i0, T, stride, gamma_log);
   MPA_CHECK_LAUNCH("gather_patches");
+  return MPA_OK;
+}
+
+int mpa_gather_patches_bwd_f32(const float* g_out, const float* in, float* g_in, int C, int NT, int F, int i0, int n, int T, int stride,
+                               float gamma_log, void* stream) {
+  MPA_CHECK_ARCH();
+  MPA_REQUIRE(g_out && g_in && (in || gamma_log <= 0.f) && C > 0 && F > 0 && n > 0 && T > 0 && stride > 0 && i0 >= 0,
+              "gather_patches_bwd: bad argument");
+  MPA_REQUIRE((long long)(i0 + n - 1) * stride + T <= NT, "gather_patches_bwd: patch range exceeds the %d input frames", NT);
+  long long total = (long long)C * NT * F;
+  gather_patches_bwd_kernel<<<grid_for(total, 256), 256, 0, (cudaStream_t)stream>>>(g_out, in, g_in, total, C, NT, F, i0, n, T, stride,
+                                                                                    gamma_log);
+  MPA_CHECK_LAUNCH("gather_patches_bwd");
   return MPA_OK;
 }
 

@@ -167,6 +167,157 @@ __global__ void __launch_bounds__(256) cqt_levels_kernel(const __grid_constant__
   }
 }
 
+// ---- backward: the adjoint of cqt_levels_kernel, of the reflect-padded framing and of decimate_kernel --------------------------------
+// Every stage before the magnitude is linear, so with G_r = dL/d(re, im) of row r's complex response C_r,
+//   dL/dx_k = Re( sum_bin V[bin] e^{-2 pi i bin k / n_fft} ),  V[bin] = sum_r w_r b_{r, bin - s0_r},  w_r = scale_r * g_r * conj(C_r) / |C_r|
+// (g_r = sum of the upstream gradient over the row's destinations; w_r = 0 where |C_r| = 0, the convention of torch.abs): a transposed
+// banded contraction followed by one forward FFT.  The spectrum is recomputed from the signal (the forward keeps nothing).  Each thread
+// owns one output element and sums in a fixed order: two runs give the same bits, no atomics.
+struct CqtLevelsBwdParams {
+  mpa_cqt_level lv[kMaxCqtLevels];
+  mpa_cqt_level_grad gr[kMaxCqtLevels];
+  int log2n[kMaxCqtLevels];
+  size_t ws_off[kMaxCqtLevels];      // floats: level l's [n_frames][n_fft] frame gradients
+  int n_frames, band, out_frames, out_bins;
+  const int* tuning_idx;
+  const float* g_out;
+  float* ws;
+};
+// one CTA per (frame, level): the frame's gradient wrt its n_fft (reflect-padded) samples -> ws
+__global__ void __launch_bounds__(256) cqt_levels_bwd_kernel(const __grid_constant__ CqtLevelsBwdParams p) {
+  extern __shared__ float2 sm2[];
+  const mpa_cqt_level& L = p.lv[blockIdx.y];
+  const int n_fft = L.n_fft, log2n = p.log2n[blockIdx.y];
+  float2* a = sm2;              // [n_fft]
+  float2* tw = sm2 + n_fft;     // [n_fft/2]
+  float2* w = tw + n_fft / 2;   // [n_rows]
+  const int t = blockIdx.x;
+  load_frame_bitrev(a, tw, L.y, L.n, nullptr, (long long)t * L.hop - n_fft / 2, n_fft, log2n);
+  fft_smem(a, tw, n_fft, log2n);
+  const int tune = p.tuning_idx ? p.tuning_idx[0] : 0;
+  const int n_rows = L.n_rows, band = p.band;
+  const float2* bs = reinterpret_cast<const float2*>(L.basis) + (size_t)tune * n_rows * band;
+  const int* st = L.band_start + (size_t)tune * n_rows;
+  const float* sc = L.row_scale + (size_t)tune * n_rows;
+  const int nb = n_fft / 2 + 1;
+  for (int r = threadIdx.x; r < n_rows; r += blockDim.x) {
+    const int s0 = st[r];
+    const float2* br = bs + (size_t)r * band;
+    float re = 0.f, im = 0.f;
+    for (int f = 0; f < band; ++f) {            // the forward's contraction, same order
+      const int bin = s0 + f;
+      if (bin < nb) {
+        const float2 b = br[f], x = a[bin];
+        re = fmaf(b.x, x.x, re);
+        re = fmaf(-b.y, x.y, re);
+        im = fmaf(b.x, x.y, im);
+        im = fmaf(b.y, x.x, im);
+      }
+    }
+    float g = 0.f;
+    for (int d = 0; d < L.n_dest; ++d) {
+      const int code = L.dest[r * L.n_dest + d];
+      if (code >= 0) g += p.g_out[((size_t)(code >> 16) * p.out_frames + t) * p.out_bins + (code & 0xffff)];
+    }
+    const float m = sqrtf(re * re + im * im);
+    const float k = (m > 0.f) ? g * sc[r] / m : 0.f;
+    w[r] = make_float2(k * re, -k * im);
+  }
+  __syncthreads();                              // the spectrum in `a` is dead from here on
+  // transposed contraction over the bin -> rows table (rows whose band covers the bin), written bit-reversed for the FFT
+  const int* off = p.gr[blockIdx.y].bin_off + (size_t)tune * (nb + 1);
+  const int* rows = p.gr[blockIdx.y].bin_rows + (size_t)tune * n_rows * band;
+  for (int k = threadIdx.x; k < n_fft; k += blockDim.x) {
+    float vr = 0.f, vi = 0.f;
+    if (k < nb) {
+      for (int e = off[k]; e < off[k + 1]; ++e) {
+        const int r = rows[e];
+        const float2 b = bs[(size_t)r * band + (k - st[r])], wr = w[r];
+        vr = fmaf(b.x, wr.x, vr);
+        vr = fmaf(-b.y, wr.y, vr);
+        vi = fmaf(b.x, wr.y, vi);
+        vi = fmaf(b.y, wr.x, vi);
+      }
+    }
+    a[__brev((unsigned)k) >> (32 - log2n)] = make_float2(vr, vi);
+  }
+  __syncthreads();
+  fft_smem(a, tw, n_fft, log2n);
+  float* out = p.ws + p.ws_off[blockIdx.y] + (size_t)t * n_fft;
+  for (int k = threadIdx.x; k < n_fft; k += blockDim.x) out[k] = a[k].x;
+}
+
+__device__ __forceinline__ long long floor_div(long long a, long long b) {      // b > 0
+  const long long q = a / b;
+  return (a % b != 0 && a < 0) ? q - 1 : q;
+}
+
+// adjoint of the reflect-padded framing for one sample i of an n-sample signal: padded position q (frame t covers q = t*hop - n_fft/2 + k,
+// k < n_fft) reads sample i exactly when q = +-i (mod 2(n-1)), so every preimage q of i is enumerated (a signal shorter than n_fft has
+// several) and the frames covering it are summed, frame-major
+__device__ double ola_sample(const float* __restrict__ ws, long long i, long long n, int n_fft, int hop, int n_frames) {
+  const long long P = 2 * (n - 1);
+  const long long lo = -(long long)(n_fft / 2), hi = (long long)(n_frames - 1) * hop + n_fft / 2;      // padded positions [lo, hi)
+  double acc = 0.0;
+  const int nsets = (i == 0 || i == n - 1) ? 1 : 2;     // at the two end samples +i and -i name the same residue class
+  for (int s = 0; s < nsets; ++s) {
+    const long long base = s == 0 ? i : -i;
+    const long long m1 = floor_div(hi - 1 - base, P);
+    for (long long m = floor_div(lo - base + P - 1, P); m <= m1; ++m) {
+      const long long u = base + m * P + n_fft / 2;     // = t*hop + k
+      const long long t1 = min((long long)n_frames - 1, u / hop);
+      const long long t0 = max(0LL, floor_div(u - n_fft, hop) + 1);
+      for (long long t = t0; t <= t1; ++t) acc += (double)ws[t * n_fft + (u - t * hop)];
+    }
+  }
+  return acc;
+}
+
+// overlap-add of the frame gradients into the level signals' gradients; blockIdx.y = one signal, summing every level that reads it
+struct CqtOlaParams {
+  int grp_first[kMaxCqtLevels + 1];    // levels of signal g: order[grp_first[g] .. grp_first[g+1])
+  int order[kMaxCqtLevels];
+  int n_fft[kMaxCqtLevels], hop[kMaxCqtLevels];
+  size_t ws_off[kMaxCqtLevels];
+  float* g_y[kMaxCqtLevels];
+  long long n[kMaxCqtLevels];          // per signal
+  int n_frames, accumulate;
+  const float* ws;
+};
+__global__ void __launch_bounds__(256) cqt_ola_bwd_kernel(const __grid_constant__ CqtOlaParams p) {
+  const int g = blockIdx.y;
+  const long long n = p.n[g];
+  float* gy = p.g_y[g];
+  for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
+    double acc = p.accumulate ? (double)gy[i] : 0.0;
+    for (int q = p.grp_first[g]; q < p.grp_first[g + 1]; ++q) {
+      const int l = p.order[q];
+      acc += ola_sample(p.ws + p.ws_off[l], i, n, p.n_fft[l], p.hop[l], p.n_frames);
+    }
+    gy[i] = (float)acc;
+  }
+}
+
+// transpose of decimate_kernel: g_in[i] (+)= gain * sum_{t < n_out_real, |i - D*t| < n_half} h[|i - D*t|] * g_out[t]; float64 accumulation
+__global__ void decimate_adjoint_kernel(const float* __restrict__ g_out, float* __restrict__ g_in, const float* __restrict__ half, int n_half,
+                                        int factor, double gain, long long n_in, long long n_out_real, int accumulate) {
+  extern __shared__ float h[];
+  for (int i = threadIdx.x; i < n_half; i += blockDim.x) h[i] = half[i];
+  __syncthreads();
+  for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n_in; i += (long long)gridDim.x * blockDim.x) {
+    const long long t0 = max(0LL, -floor_div(-(i - (n_half - 1)), factor));
+    const long long t1 = min(n_out_real - 1, (i + n_half - 1) / factor);
+    double acc = 0.0;
+#pragma unroll 1
+    for (long long t = t0; t <= t1; ++t) {
+      const long long j = i - (long long)factor * t;
+      acc += (double)h[j < 0 ? -j : j] * (double)g_out[t];
+    }
+    acc *= gain;
+    g_in[i] = accumulate ? (float)((double)g_in[i] + acc) : (float)acc;
+  }
+}
+
 // STFT-2048 (hann) + piptrack peak picking; peaks appended to ws: [0]=count, then pitch[max], mag[max]
 __global__ void __launch_bounds__(256) tuning_peaks_kernel(const float* __restrict__ y, long long n, const float* __restrict__ window, float sr,
                                                            int* __restrict__ counter, float* __restrict__ pitch, float* __restrict__ mag, int max_peaks) {
@@ -434,6 +585,98 @@ int mpa_cqt_levels_f32(const mpa_cqt_level* levels, int n_levels, int n_frames, 
   p.tuning_idx = tuning_idx; p.out = out;
   cqt_levels_kernel<<<dim3(n_frames, n_levels), 256, (size_t)max_fft * 12, (cudaStream_t)stream>>>(p);
   MPA_CHECK_LAUNCH("cqt_levels");
+  return MPA_OK;
+}
+
+size_t mpa_cqt_levels_bwd_workspace(const mpa_cqt_level* levels, int n_levels, int n_frames) {
+  size_t floats = 0;
+  for (int i = 0; levels && i < n_levels; ++i) floats += (size_t)(n_frames < 1 ? 1 : n_frames) * levels[i].n_fft;
+  return floats * sizeof(float);
+}
+
+int mpa_cqt_levels_bwd_f32(const mpa_cqt_level* levels, const mpa_cqt_level_grad* grads, int n_levels, int n_frames, int band,
+                           const int* tuning_idx, const float* g_out, int out_frames, int out_bins, int accumulate, void* workspace,
+                           size_t ws_bytes, void* stream) {
+  MPA_CHECK_ARCH();
+  MPA_REQUIRE(levels && grads && g_out && workspace && n_levels >= 1 && n_levels <= kMaxCqtLevels, "cqt_levels_bwd: 1..%d levels", kMaxCqtLevels);
+  MPA_REQUIRE(n_frames >= 1 && n_frames <= out_frames && band >= 1 && out_bins < 65536, "cqt_levels_bwd: bad shape");
+  if (ws_bytes < mpa_cqt_levels_bwd_workspace(levels, n_levels, n_frames)) {
+    set_error("cqt_levels_bwd: workspace %zu < %zu bytes", ws_bytes, mpa_cqt_levels_bwd_workspace(levels, n_levels, n_frames));
+    return MPA_ERR_WORKSPACE;
+  }
+  CqtLevelsBwdParams p;
+  CqtOlaParams q;
+  memset(&p, 0, sizeof(p));
+  memset(&q, 0, sizeof(q));
+  int max_fft = 0, max_rows = 0, n_groups = 0;
+  size_t off = 0;
+  for (int i = 0; i < n_levels; ++i) {
+    const mpa_cqt_level& L = levels[i];
+    const mpa_cqt_level_grad& G = grads[i];
+    MPA_REQUIRE(L.y && L.basis && L.band_start && L.row_scale && L.dest && G.g_y && G.bin_off && G.bin_rows,
+                "cqt_levels_bwd: null argument in level %d", i);
+    MPA_REQUIRE(L.n_fft >= 64 && L.n_fft <= 4096 && (L.n_fft & (L.n_fft - 1)) == 0, "cqt_levels_bwd: n_fft must be a power of two in 64..4096");
+    MPA_REQUIRE(L.n >= 2 && L.hop >= 1 && L.n_rows >= 1 && L.n_rows <= 2048 && L.n_dest >= 1, "cqt_levels_bwd: bad level %d", i);
+    MPA_REQUIRE((long long)(n_frames - 1) * L.hop <= L.n, "cqt_levels_bwd: %d frames at hop %d exceed the signal (%lld samples)", n_frames, L.hop,
+                L.n);
+    p.lv[i] = L;
+    p.gr[i] = G;
+    p.log2n[i] = ilog2(L.n_fft);
+    p.ws_off[i] = q.ws_off[i] = off;
+    off += (size_t)n_frames * L.n_fft;
+    q.n_fft[i] = L.n_fft;
+    q.hop[i] = L.hop;
+    if (L.n_fft > max_fft) max_fft = L.n_fft;
+    if (L.n_rows > max_rows) max_rows = L.n_rows;
+  }
+  // group the levels by the signal gradient they write (first-occurrence order), so that one thread owns each signal sample
+  for (int i = 0, k = 0; i < n_levels; ++i) {
+    bool seen = false;
+    for (int j = 0; j < i; ++j) seen |= grads[j].g_y == grads[i].g_y;
+    if (seen) continue;
+    q.grp_first[n_groups] = k;
+    q.g_y[n_groups] = grads[i].g_y;
+    q.n[n_groups] = levels[i].n;
+    for (int j = i; j < n_levels; ++j) {
+      if (grads[j].g_y != grads[i].g_y) continue;
+      MPA_REQUIRE(levels[j].n == levels[i].n, "cqt_levels_bwd: levels %d and %d share a gradient buffer but not a length", i, j);
+      q.order[k++] = j;
+    }
+    q.grp_first[++n_groups] = k;
+  }
+  p.n_frames = n_frames; p.band = band; p.out_frames = out_frames; p.out_bins = out_bins;
+  p.tuning_idx = tuning_idx; p.g_out = g_out; p.ws = (float*)workspace;
+  q.n_frames = n_frames; q.accumulate = accumulate ? 1 : 0; q.ws = (const float*)workspace;
+  cudaStream_t st = (cudaStream_t)stream;
+  const size_t smem = (size_t)max_fft * 12 + (size_t)max_rows * 8;
+  if (smem > 48 * 1024) {
+    cudaError_t e = cudaFuncSetAttribute(cqt_levels_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) {
+      set_error("cqt_levels_bwd: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
+      return MPA_ERR_CUDA;
+    }
+  }
+  cqt_levels_bwd_kernel<<<dim3(n_frames, n_levels), 256, smem, st>>>(p);
+  MPA_CHECK_LAUNCH("cqt_levels_bwd");
+  long long n_max = 0;
+  for (int g = 0; g < n_groups; ++g) n_max = q.n[g] > n_max ? q.n[g] : n_max;
+  long long gx = (n_max + 255) / 256;
+  if (gx > 148 * 8) gx = 148 * 8;
+  cqt_ola_bwd_kernel<<<dim3((unsigned)gx, n_groups), 256, 0, st>>>(q);
+  MPA_CHECK_LAUNCH("cqt_ola_bwd");
+  return MPA_OK;
+}
+
+int mpa_decimate_adjoint_f32(const float* g_out, float* g_in, const float* half_taps, int n_half, int factor, double gain, long long n_in,
+                             int accumulate, void* stream) {
+  MPA_CHECK_ARCH();
+  MPA_REQUIRE(g_out && g_in && half_taps && factor >= 2 && (factor & (factor - 1)) == 0 && n_half >= 1 && n_half <= 4096 && n_in >= factor,
+              "decimate_adjoint: bad argument");
+  long long g = (n_in + 255) / 256;
+  if (g > 148 * 16) g = 148 * 16;
+  decimate_adjoint_kernel<<<(unsigned)g, 256, (size_t)n_half * sizeof(float), (cudaStream_t)stream>>>(g_out, g_in, half_taps, n_half, factor, gain,
+                                                                                                        n_in, n_in / factor, accumulate);
+  MPA_CHECK_LAUNCH("decimate_adjoint");
   return MPA_OK;
 }
 

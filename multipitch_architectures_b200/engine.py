@@ -239,8 +239,7 @@ def predict_patchwise(model, hcqt, batch=50, lo=0, hi=None):
     outs, npreds = [], []
     for i0 in range(lo, hi, batch):
         n = min(batch, hi - i0)
-        x = torch.empty(n, C, CONTEXT, F, dtype=torch.float32, device=dev)
-        _lib.call('gather_patches_f32', padded, x, C, N + CONTEXT, F, i0, n, CONTEXT, 1, 10.0, _lib.stream_ptr())
+        x = ops.gather_patches(padded, i0, n, CONTEXT, 1, 10.0)
         with torch.no_grad():
             y = model(x)
         if isinstance(y, tuple):
@@ -283,3 +282,43 @@ def _predict_patchwise_frames(model, hcqt, batch, lo, hi):
         return torch.empty(0, 0, dtype=torch.float32, device=dev)
     out = torch.cat(outs, 0) if len(outs) > 1 else outs[0]
     return (out, torch.cat(npreds, 0)) if npreds else out
+
+
+def audio_vjp(model, y, plan, g_act, lo=0, hi=None, batch=50, tuning_idx=None):
+    """Vector-Jacobian product of the audio -> activations map of the reference's test loop: y [n] fp32 CUDA audio, plan an HCQTPlan,
+    g_act [N, n_out] the upstream gradient of the activations of every HCQT frame (rows outside lo..hi-1 are not used) -> dL/dy [n] fp32
+    for L = sum(g_act[lo:hi] * activations[lo:hi]), the activations being predict_patchwise(model, hcqt, batch, lo, hi) of the HCQT of y
+    (37 / 38 zero frames of padding, stride-1 patches of 75 frames, log(1 + 10x)).
+
+    The HCQT runs once with grad and is detached to a leaf; the model (eval mode) runs on the same batches of `batch` consecutive patches
+    as predict_patchwise (the SAUnet's attention spans the batch axis), each batch's gradient flows back through ops.gather_patches into
+    the leaf, and one HCQT backward maps the sum to the audio.  Memory is one batch's tape, not the recording's.  Model parameters' .grad
+    and y.grad are left alone.  For a model with two outputs (PUnet: activations, note predictions) g_act applies to the first and the
+    second gets a zero gradient.  The tuning index (estimated when None) is a constant of the map (see HCQTPlan.run)."""
+    if model.training:
+        raise ValueError('audio_vjp differentiates the inference map: put the model in eval mode')
+    y = y.detach().contiguous().requires_grad_(True)
+    with torch.enable_grad():
+        hcqt, _ = plan.run(y, tuning_idx)
+    C, N, F = hcqt.shape
+    hi = N if hi is None else hi
+    if not (0 <= lo <= hi <= N):
+        raise ValueError('bad frame range')
+    if g_act.dim() != 2 or g_act.shape[0] != N:
+        raise ValueError(f'g_act must be [{N}, n_out] (one row per HCQT frame), got {tuple(g_act.shape)}')
+    g_act = g_act.to(device=hcqt.device, dtype=torch.float32)
+    padded = torch.zeros(C, N + CONTEXT, F, dtype=torch.float32, device=hcqt.device)
+    padded[:, HALF:HALF + N] = hcqt.detach()
+    padded.requires_grad_(True)
+    g_pad = torch.zeros_like(padded)
+    with torch.enable_grad():
+        for i0 in range(lo, hi, batch):
+            n = min(batch, hi - i0)
+            out = model(ops.gather_patches(padded, i0, n, CONTEXT, 1, 10.0))
+            outs = list(out) if isinstance(out, tuple) else [out]
+            grads = [g_act[i0:i0 + n].reshape(outs[0].shape)] + [torch.zeros_like(o) for o in outs[1:]]
+            keep = [k for k, o in enumerate(outs) if o.requires_grad]
+            (g,) = torch.autograd.grad([outs[k] for k in keep], [padded], [grads[k] for k in keep])
+            g_pad += g
+        (y_grad,) = torch.autograd.grad(hcqt, y, g_pad[:, HALF:HALF + N].contiguous())
+    return y_grad

@@ -184,6 +184,25 @@ def build_tables(sr, hop, fmin, bpo, num_octaves, list_harmonics, base_harmonics
     return tables
 
 
+def bin_rows(start, n_fft, band=BAND):
+    """Inverse of the banded layout for the HCQT backward (mpa_cqt_levels_bwd_f32): start [n_tunings, R] -> (off [n_tunings, nb+1],
+    rows [n_tunings, R*band]) int32, nb = n_fft/2 + 1; per tuning, the rows whose band [start, start+band) covers bin k are
+    rows[off[k]:off[k+1]] in ascending order (bins >= nb, which the forward skips, are left out)."""
+    n_tun, R = start.shape
+    nb = n_fft // 2 + 1
+    off = np.zeros((n_tun, nb + 1), dtype=np.int32)
+    rows = np.zeros((n_tun, R * band), dtype=np.int32)
+    r_all = np.repeat(np.arange(R), band)
+    for ti in range(n_tun):
+        b = (start[ti][:, None] + np.arange(band)[None, :]).ravel()
+        keep = b < nb
+        b, r = b[keep], r_all[keep]
+        order = np.lexsort((r, b))
+        rows[ti, :len(order)] = r[order]
+        off[ti, 1:] = np.cumsum(np.bincount(b, minlength=nb))
+    return off, rows
+
+
 def kaiser_fast_half_taps(factor=2):
     """|j| = 0 .. 16*factor-1 taps of resampy's kaiser_fast interpolation window walked at a factor:1 ratio
     (x 1/factor sample ratio)."""

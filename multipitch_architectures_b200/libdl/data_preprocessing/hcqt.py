@@ -3,9 +3,11 @@
 libmpa CUDA kernels (decimator chain, fused FFT + constant-Q contraction, tuning estimate)."""
 import ctypes
 import functools
+import math
 
 import numpy as np
 import torch
+from torch.autograd.function import once_differentiable
 
 from ... import _lib
 from . import _filterbank as FB
@@ -67,7 +69,7 @@ class HCQTPlan:
                 signal=sg, n_fft=n_fft, n_rows=t['dest'].shape[0], n_dest=t['dest'].shape[1],
                 basis=torch.from_numpy(np.ascontiguousarray(t['basis']).view(np.float32)).to(self.device),
                 start=torch.from_numpy(t['start']).to(self.device), scale=torch.from_numpy(t['scale']).to(self.device),
-                dest=torch.from_numpy(t['dest']).to(self.device)))
+                dest=torch.from_numpy(t['dest']).to(self.device), start_host=t['start']))
         self.signals = sorted({l['signal'] for l in self.levels} |
                               {(c, j) for (c, i) in {l['signal'] for l in self.levels} for j in range(i)})
         self.taps = {f: torch.from_numpy(FB.kaiser_fast_half_taps(f)).to(self.device)
@@ -77,6 +79,7 @@ class HCQTPlan:
         self.tunings = FB.tuning_values()
         self._frames = {}
         self._side = None
+        self._bin_rows = None       # backward only: per level (bin_off, bin_rows) device tables, built on first use
         self._graphs, self.graph_replays, self.graph_launches = {}, 0, 0     # run_graph: captured launch sequences per input length
 
     def n_frames(self, n):
@@ -96,7 +99,8 @@ class HCQTPlan:
         """plan.run(y) replayed from a CUDA graph captured once per input length: the ~25 small dependent launches of one clip (tuning
         estimate, decimator chain, one CQT launch per octave / rate) become ONE graph launch (the launch-bound 0.56 ms of a 30 s clip is
         mostly host launch latency).  The result lives in buffers OWNED BY THE PLAN and is overwritten by the next call of the same
-        length: for consumers that use it at once on the same stream (the inference engines); plan.run returns fresh tensors."""
+        length: for consumers that use it at once on the same stream (the inference engines); plan.run returns fresh tensors.
+        Inference only: the result never carries a grad_fn (use plan.run for gradients wrt y)."""
         if y.dim() != 1 or not y.is_cuda or y.dtype != torch.float32:
             raise _lib.MpaError('HCQTPlan.run_graph expects a 1-D float32 CUDA tensor')
         n = y.numel()
@@ -105,12 +109,12 @@ class HCQTPlan:
             if len(self._graphs) >= 4:
                 self._graphs.pop(next(iter(self._graphs)))
             y_static = y.contiguous().clone()
-            self.run(y_static)                                  # warm-up outside the capture (lazy module loading, workspace sizes)
+            self._forward(y_static, None)                       # warm-up outside the capture (lazy module loading, workspace sizes)
             torch.cuda.current_stream().synchronize()
             graph = torch.cuda.CUDAGraph()
             n0 = _lib.launch_count()
             with torch.cuda.graph(graph):
-                out, tun = self.run(y_static)
+                out, tun, _ = self._forward(y_static, None)
             g = self._graphs[n] = (graph, y_static, out, tun, _lib.launch_count() - n0)
         graph, y_static, out, tun, n_launches = g
         y_static.copy_(y)
@@ -120,9 +124,21 @@ class HCQTPlan:
         return out, tun
 
     def run(self, y, tuning_idx=None):
-        """y: 1-D float32 CUDA tensor -> (hcqt [H, n_frames, n_bins] fp32 CUDA, tuning_idx int32[1] CUDA)."""
+        """y: 1-D float32 CUDA tensor -> (hcqt [H, n_frames, n_bins] fp32 CUDA, tuning_idx int32[1] CUDA).
+
+        Differentiable in y: when grad mode is on and y.requires_grad, hcqt carries a grad_fn whose backward (mpa_cqt_levels_bwd_f32,
+        then mpa_decimate_adjoint_f32 back down the decimator chain) fills y.grad.  The tuning index is piecewise constant in y, so it is
+        treated as a constant: the backward uses the filter bank the forward selected, and tuning_idx is returned without grad.  There is
+        no double backward.  Without requires_grad the call launches exactly what it always did."""
         if y.dim() != 1 or not y.is_cuda or y.dtype != torch.float32:
             raise _lib.MpaError('HCQTPlan.run expects a 1-D float32 CUDA tensor')
+        if torch.is_grad_enabled() and y.requires_grad:
+            return _HcqtFunction.apply(y.contiguous(), self, tuning_idx)
+        out, tuning_idx, _ = self._forward(y, tuning_idx)
+        return out, tuning_idx
+
+    def _forward(self, y, tuning_idx):
+        """-> (hcqt, tuning_idx, {signal: decimated signal}) of y (no autograd)."""
         y = y.contiguous()
         n = y.numel()
         st = _lib.stream_ptr()
@@ -164,12 +180,74 @@ class HCQTPlan:
                 d.basis, d.band_start, d.row_scale = L['basis'].data_ptr(), L['start'].data_ptr(), L['scale'].data_ptr()
                 d.n_rows, d.dest, d.n_dest = L['n_rows'], L['dest'].data_ptr(), L['n_dest']
             _lib.call('cqt_levels_f32', arr, len(self.levels), n_frames, FB.BAND, tuning_idx, out, n_frames, self.n_bins, st)
-            return out, tuning_idx
+            return out, tuning_idx, sig
         for L in self.levels:
             s = sig[L['signal']]
             _lib.call('cqt_level_f32', s, _lib.i64(s.numel()), L['n_fft'], self.hop >> sum(L['signal']), n_frames, L['basis'], L['start'],
                       L['scale'], L['n_rows'], FB.BAND, tuning_idx, L['dest'], L['n_dest'], out, n_frames, self.n_bins, st)
-        return out, tuning_idx
+        return out, tuning_idx, sig
+
+    def _grad_tables(self):
+        if self._bin_rows is None:
+            self._bin_rows = [tuple(torch.from_numpy(a).to(self.device) for a in FB.bin_rows(L['start_host'], L['n_fft']))
+                              for L in self.levels]
+        return self._bin_rows
+
+    def _backward(self, g_out, sig, tuning_idx):
+        """dL/d hcqt [H, n_frames, n_bins] -> dL/dy, given the forward's decimated signals and tuning index."""
+        g_out = g_out.contiguous()
+        n_frames = g_out.shape[1]
+        st = _lib.stream_ptr()
+        grad = {k: torch.zeros_like(s) for k, s in sig.items()}
+        tabs = self._grad_tables()
+        # the filterbank adjoint, 16 levels per launch (the forward's one-launch limit); every call adds into the signal gradients
+        for lo in range(0, len(self.levels), 16):
+            idx = range(lo, min(lo + 16, len(self.levels)))
+            arr, garr = (CqtLevel * len(idx))(), (CqtLevelGrad * len(idx))()
+            for d, gd, li in zip(arr, garr, idx):
+                L = self.levels[li]
+                s = sig[L['signal']]
+                d.y, d.n, d.n_fft, d.hop = s.data_ptr(), s.numel(), L['n_fft'], self.hop >> sum(L['signal'])
+                d.basis, d.band_start, d.row_scale = L['basis'].data_ptr(), L['start'].data_ptr(), L['scale'].data_ptr()
+                d.n_rows, d.dest, d.n_dest = L['n_rows'], L['dest'].data_ptr(), L['n_dest']
+                gd.g_y, gd.bin_off, gd.bin_rows = grad[L['signal']].data_ptr(), tabs[li][0].data_ptr(), tabs[li][1].data_ptr()
+            ws_bytes = _lib.lib().mpa_cqt_levels_bwd_workspace(arr, len(idx), n_frames)
+            ws = torch.empty(ws_bytes, dtype=torch.uint8, device=g_out.device)
+            _lib.call('cqt_levels_bwd_f32', arr, garr, len(idx), n_frames, FB.BAND, tuning_idx, g_out, n_frames, self.n_bins, 1, ws,
+                      _lib.usize(ws_bytes), st)
+        # then back down the decimator chain: (c, i) feeds (c, i-1), (c, 0) feeds the input; descending order finishes every signal's
+        # gradient before it is propagated
+        for (c, i) in reversed(self.signals):
+            if (c, i) == (0, 0):
+                continue
+            prev, factor = ((0, 0), 2 ** c) if i == 0 else ((c, i - 1), 2)
+            taps = self.taps[factor]
+            _lib.call('decimate_adjoint_f32', grad[(c, i)], grad[prev], taps, taps.numel(), factor, ctypes.c_double(math.sqrt(factor)),
+                      _lib.i64(sig[prev].numel()), 1, st)
+        return grad[(0, 0)]
+
+
+class CqtLevelGrad(ctypes.Structure):
+    """mpa_cqt_level_grad (include/mpa.h)"""
+    _fields_ = [('g_y', ctypes.c_void_p), ('bin_off', ctypes.c_void_p), ('bin_rows', ctypes.c_void_p)]
+
+
+class _HcqtFunction(torch.autograd.Function):
+    """HCQTPlan.run with a backward to the audio; saves y, the decimated signals and the tuning index (no spectrum)."""
+
+    @staticmethod
+    def forward(ctx, y, plan, tuning_idx):
+        out, tun, sig = plan._forward(y, tuning_idx)
+        ctx.plan, ctx.keys = plan, list(sig)
+        ctx.save_for_backward(tun, *sig.values())
+        ctx.mark_non_differentiable(tun)
+        return out, tun
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, g_out, _g_tun):
+        tun, *sigs = ctx.saved_tensors
+        return ctx.plan._backward(g_out, dict(zip(ctx.keys, sigs)), tun), None, None
 
 
 @functools.lru_cache(maxsize=8)
@@ -186,7 +264,8 @@ def _hcqt_host(plan, f_audio):
 def compute_hcqt(f_audio, fs=22050, fmin=C1_HZ, fs_hcqt_target=91, bins_per_octave=60, num_octaves=6, num_harmonics=5,
                  num_subharmonics=1, center_bins=True, device='cuda'):
     """Drop-in for the reference's standard HCQT (hcqt.py:34-85): one individual CQT per (sub)harmonic, hop size derived from
-    num_octaves alone.  Returns (f_hcqt float64 ndarray [n_bins, n_frames, H], fs_hcqt, hopsize_cqt)."""
+    num_octaves alone.  Returns (f_hcqt float64 ndarray [n_bins, n_frames, H], fs_hcqt, hopsize_cqt).  NumPy in and out, so not
+    differentiable: for gradients wrt the audio use HCQTPlan.run on a tensor with requires_grad."""
     hopsize_cqt, _ = compute_hopsize_cqt(fs_hcqt_target, fs=fs, num_octaves=num_octaves)
     fs_hcqt = fs / hopsize_cqt
     assert np.mod(bins_per_octave, 12) == 0, 'Error: bins_per_octave no multiple of 12'
@@ -202,7 +281,8 @@ def compute_efficient_hcqt(f_audio, fs=22050, fmin=C1_HZ, fs_hcqt_target=91, bin
     """Drop-in for the reference function of the same name (hcqt.py:89-164).
 
     Returns (f_hcqt float64 ndarray [n_bins, n_frames, H], fs_hcqt, hopsize_cqt).  Harmonics related by powers of two
-    share one CQT, exactly like the reference; channel order: sub-harmonics (lowest first), then h = 1..num_harmonics."""
+    share one CQT, exactly like the reference; channel order: sub-harmonics (lowest first), then h = 1..num_harmonics.  NumPy in and
+    out, so not differentiable: for gradients wrt the audio use HCQTPlan.run on a tensor with requires_grad."""
     num_octaves_eff = num_octaves + int(np.ceil(np.log2(num_subharmonics + 1) + np.log2(num_harmonics)))
     hopsize_cqt, _ = compute_hopsize_cqt(fs_hcqt_target, fs=fs, num_octaves=num_octaves_eff)
     fs_hcqt = fs / hopsize_cqt
@@ -215,7 +295,8 @@ def compute_efficient_hcqt(f_audio, fs=22050, fmin=C1_HZ, fs_hcqt_target=91, bin
 
 
 def estimate_tuning(f_audio, fs=22050, bins_per_octave=36, device='cuda'):
-    """The whole-file tuning scalar the reference obtains from librosa.estimate_tuning (hcqt.py:122)."""
+    """The whole-file tuning scalar the reference obtains from librosa.estimate_tuning (hcqt.py:122).  Inference only: the estimate is
+    piecewise constant in the audio and has no gradient."""
     y = torch.from_numpy(np.ascontiguousarray(f_audio, dtype=np.float32)).to(device)
     n = y.numel()
     idx = torch.empty(1, dtype=torch.int32, device=y.device)

@@ -76,6 +76,44 @@ def layernorm_cf_input_grad(x, g, w, gw, gb, eps, gamma_log=0.0, stats=None):
     return dx
 
 
+def _gather_patches_fwd(frames, i0, n, T, stride, gamma):
+    C, NT, F = frames.shape
+    out = torch.empty(n, C, T, F, dtype=torch.float32, device=frames.device)
+    call('gather_patches_f32', frames, out, C, NT, F, i0, n, T, stride, gamma, stream_ptr())
+    return out
+
+
+class _GatherPatches(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, frames, i0, n, T, stride, gamma):
+        ctx.save_for_backward(frames)
+        ctx.args = (i0, n, T, stride, gamma)
+        return _gather_patches_fwd(frames, i0, n, T, stride, gamma)
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable
+    def backward(ctx, g):
+        (frames,) = ctx.saved_tensors
+        i0, n, T, stride, gamma = ctx.args
+        C, NT, F = frames.shape
+        g_in = torch.empty_like(frames)
+        call('gather_patches_bwd_f32', _f32(g).contiguous(), frames, g_in, C, NT, F, i0, n, T, stride, gamma, stream_ptr())
+        return g_in, None, None, None, None, None
+
+
+def gather_patches(frames, i0, n, T=75, stride=1, gamma=10.0):
+    """frames [C, NT, F] fp32 CUDA (zero-padded as the caller wants) -> [n, C, T, F]: patch b = log(1 + gamma * frames[:, (i0+b)*stride :
+    (i0+b)*stride + T, :]) (no compression when gamma <= 0), the reference dataset's patch cut.  Differentiable in frames
+    (mpa_gather_patches_bwd_f32) when grad mode is on and frames.requires_grad; no double backward."""
+    if frames.dim() != 3:
+        raise ValueError(f'expected frames [C, NT, F], got {tuple(frames.shape)}')
+    frames = _f32(frames).contiguous()
+    args = (int(i0), int(n), int(T), int(stride), float(gamma))
+    if torch.is_grad_enabled() and frames.requires_grad:
+        return _GatherPatches.apply(frames, *args)
+    return _gather_patches_fwd(frames, *args)
+
+
 def conv2d(x, wp, bias, Cout, ksize, stride=(1, 1), padding=(0, 0), act=ACT_NONE, act_param=0.0,
            scale=None, shift=None, x2=None):
     B, C1, H, W = x.shape
